@@ -11,7 +11,13 @@ the reference's `num_deductions`, include/statistics.hpp:151,354) over the devic
 kernel with the network already resident in HBM; `e2e` runs the same step from host buffers
 through tb_create + tb_solve + result read-back + tb_destroy.
 
-  python bench.py [--gpus N] [--steps K] [--warmup W] [--impl ours|reference] [--workload NAME]
+  python bench.py [--gpus N] [--steps K] [--warmup W] [--impl ours|reference] [--workload NAME] [--dump-outputs DIR]
+
+`--dump-outputs DIR` writes what the last timed step returned (best store lb / ub, has_solution, exhaustive,
+objective) as DIR/<name>.npy in float64, so that two builds can be compared output for output on the same inputs.
+When several solutions reach the best objective, which one lb / ub hold depends on which of the concurrent blocks
+found it first (two runs of the default workload on one B200: objective 286 both times, stores differing in 48 of
+13501 variables), so stores are compared by objective and by checking them against the network.
 
 N > 1 is launched under torchrun (one rank per GPU): subproblems are sharded idx = k*N + rank, the
 incumbent is exchanged through CUDA-IPC peer-mapped cells, torch.distributed only carries the
@@ -31,6 +37,9 @@ import numpy as np
 
 ROOT = os.path.dirname(os.path.abspath(__file__))
 sys.path.insert(0, ROOT)
+# The benchmark writes nothing into the tree it runs from: without this, importing tests/, tools/, oracle/ and
+# turbo_b200/ would leave __pycache__/ directories in a writable checkout.
+sys.dont_write_bytecode = True
 
 from tests import golden_io  # noqa: E402  (fixture loader only; no oracle code)
 from turbo_b200 import abi  # noqa: E402
@@ -180,6 +189,25 @@ def problem_bytes(pb):
     return int(pb.lb.nbytes + pb.ub.nbytes + pb.props.nbytes + sum(v.nbytes for _, _, v in pb.strategies))
 
 
+DUMP_BUDGET_BYTES = 64 << 20
+
+
+def dump_outputs(out_dir, pb, result):
+    """What tb_solve returned in the last timed step, as float64 .npy files (every int32 is exact in float64). A store
+    too large for the budget is written as a fixed, seeded sample of its variables, their indices in var_index.npy."""
+    os.makedirs(out_dir, exist_ok=True)
+    lb, ub = np.asarray(result["lb"]), np.asarray(result["ub"])
+    room = DUMP_BUDGET_BYTES - 4096                  # the three scalars and the .npy headers
+    if 2 * 8 * lb.size > room:
+        keep = np.sort(np.random.default_rng(0).choice(lb.size, room // (3 * 8), replace=False))
+        np.save(os.path.join(out_dir, "var_index.npy"), keep.astype(np.float64))
+        lb, ub = lb[keep], ub[keep]
+    has = result["has_solution"]
+    objective = result["lb"][pb.obj_var] if has and pb.obj_var >= 0 else np.nan      # as Solver.solve() reports it
+    for name, a in (("lb", lb), ("ub", ub), ("has_solution", has), ("exhaustive", result["exhaustive"]), ("objective", objective)):
+        np.save(os.path.join(out_dir, name + ".npy"), np.asarray(a, dtype=np.float64))
+
+
 def run_ours(args):
     import torch
     from turbo_b200 import engine
@@ -272,10 +300,12 @@ def run_ours(args):
     wall_s = time.perf_counter() - t0
     clocks = sampler.stop()
     merged = gather_results(solver)          # of the last timed step: the global best and the summed statistics
+    if args.dump_outputs and rank == 0:
+        dump_outputs(args.dump_outputs, pb, merged)
 
     # ---- e2e: host buffers -> tb_create (H2D) -> tb_solve -> results (D2H) -> tb_destroy -------------------
     # the drop-in call pattern (one solver per model); the split says where the time outside the kernel goes
-    e2e_steps = max(args.steps, 10) if args.e2e_steps is None else args.e2e_steps
+    e2e_steps = args.steps if args.e2e_steps is None else args.e2e_steps
     solver.close()                           # its device memory goes back to the pool the e2e solvers allocate from
     barrier()
     split = dict(create=0.0, link=0.0, solve=0.0, destroy=0.0)
@@ -448,6 +478,8 @@ def run_reference(args):
         secs += time.perf_counter() - t
         ded += r["stats"]["num_deductions"]
         nodes += r["stats"]["nodes"]
+    if args.dump_outputs:
+        dump_outputs(args.dump_outputs, pb, r)
     value = ded / secs
     line = {"impl": "reference", "metric": "propagations/sec", "value": value, "unit": "propagations/s", "n_gpus": args.gpus,
             "steps": args.steps, "warmup": args.warmup, "ms_per_step": secs * 1e3 / args.steps, "higher_is_better": True,
@@ -544,7 +576,9 @@ def run_report(args):
 def main():
     ap = argparse.ArgumentParser()
     ap.add_argument("--gpus", type=int, default=1)
-    ap.add_argument("--steps", type=int, default=5)
+    ap.add_argument("--steps", type=int, default=5,
+                    help="timed steps of the headline and of the e2e leg; the unsimplified_network and active_set side legs "
+                         "run min(steps, 3), which keeps the whole run short")
     ap.add_argument("--warmup", type=int, default=3)
     ap.add_argument("--impl", default="ours", choices=["ours", "reference"])
     ap.add_argument("--workload", default="simplified:trains15",
@@ -552,7 +586,7 @@ def main():
                          "solves by default, as the reference does unless -disable_simplify), or synthetic[:V:P]")
     ap.add_argument("--cutnodes", type=int, default=2000, help="node budget per search worker and step (thread block / host thread)")
     ap.add_argument("--sub", type=int, default=None, help="EPS depth; default: 17 for the default workload (both arms), else auto")
-    ap.add_argument("--e2e-steps", type=int, default=None, help="timed steps of the e2e leg (default: max(steps, 10))")
+    ap.add_argument("--e2e-steps", type=int, default=None, help="timed steps of the e2e leg (default: --steps)")
     ap.add_argument("--strong-ms", type=int, default=3000, help="wall budget of the strong-scaling leg (0 = skip)")
     ap.add_argument("--strong-sub", type=int, default=20, help="EPS depth of the strong-scaling leg: the same at every GPU count")
     ap.add_argument("--fp", default="wac1", choices=["ac1", "wac1", "ac1_active", "wac1_active"])
@@ -564,7 +598,11 @@ def main():
     ap.add_argument("--report", default=None, help="BASELINE.md §3 table instead of the bench line: comma list of configs (1 = wordpress7_500, 2 = trains15, 3 = accap_a3, or a workload name)")
     ap.add_argument("--report-ms", type=int, default=20000, help="wall budget of every leg of --report (the reference's -t 20000)")
     ap.add_argument("--report-no-cpu", action="store_true")
+    ap.add_argument("--dump-outputs", metavar="DIR", default=None,
+                    help="write what the last timed step returned as DIR/<name>.npy (float64, at most 64 MB in all)")
     args = ap.parse_args()
+    if args.steps < 1:
+        ap.error("--steps must be at least 1")
     if args.report:
         run_report(args)
     elif args.impl == "reference":

@@ -1,21 +1,10 @@
 import os
 import sys
 
-import pytest
-
 ROOT = os.path.dirname(os.path.dirname(os.path.abspath(__file__)))
 if ROOT not in sys.path:
     sys.path.insert(0, ROOT)
 
-REFERENCE = "/root/reference"
-
 
 def pytest_configure(config):
     config.addinivalue_line("markers", "gpu: needs a CUDA device (run on the B200 box)")
-
-
-@pytest.fixture(scope="session")
-def reference_dir():
-    if not os.path.isdir(os.path.join(REFERENCE, "benchmarks")):
-        pytest.skip("/root/reference is not present on this machine")
-    return REFERENCE

@@ -1,9 +1,12 @@
 """Regenerates tests/golden/*.npz from the reference's FlatZinc inputs.
 
-Run here (the container that has /root/reference); the GPU box only ever sees the committed
-fixtures. For every instance: the TNF produced by our C++ front-end (lb, ub, props, strategies,
-objective), the reference's expected optimum (benchmarks/test_list.csv) where one exists, and the
-sha256 of the oracle's root fixpoint (a regression pin for front-end + oracle).
+  python tests/golden/make_golden.py [--check] REFERENCE_CHECKOUT      (ptal/turbo @ 683f23c)
+
+The tests only ever read the committed fixtures. For every instance: the TNF produced by our C++
+front-end (lb, ub, props, strategies, objective), the reference's expected optimum
+(benchmarks/test_list.csv) where one exists, and the sha256 of the oracle's root fixpoint (a
+regression pin for front-end + oracle). With --check nothing is written: the arrays are rebuilt and
+compared with the committed ones, the names that differ are reported and the exit status is 1 if any do.
 """
 import csv
 import hashlib
@@ -18,8 +21,6 @@ sys.path.insert(0, ROOT)
 from oracle import oracle_py as orc  # noqa: E402
 from turbo_b200.model import Model  # noqa: E402
 
-REF = "/root/reference/benchmarks"
-
 
 def root_sha(pb):
     r = orc.fixpoint(pb)
@@ -31,7 +32,7 @@ def root_sha(pb):
     return h.hexdigest(), r["failed"]
 
 
-def dump(name, path, expected):
+def dump(name, path, expected, check=False):
     m = Model.from_fzn(path)
     pb = m.problem
     sha, failed = root_sha(pb)
@@ -40,22 +41,38 @@ def dump(name, path, expected):
     strat_vars = np.concatenate([vs for _, _, vs in pb.strategies] + [np.zeros(0, np.int32)]).astype(np.int32)
     meta = np.array([pb.obj_var, pb.c.has_eps_strategy, m.objective_kind, m.user_objective_var,
                      0 if expected is None else expected, 0 if expected is None else 1, int(failed)], dtype=np.int64)
-    np.savez_compressed(os.path.join(HERE, name + ".npz"), lb=pb.lb, ub=pb.ub, props=props, strat_meta=strat_meta,
-                        strat_vars=strat_vars, meta=meta, root_sha=np.array(sha))
+    arrays = dict(lb=pb.lb, ub=pb.ub, props=props, strat_meta=strat_meta, strat_vars=strat_vars, meta=meta,
+                  root_sha=np.array(sha))
+    out = os.path.join(HERE, name + ".npz")
+    if check:
+        old = np.load(out)
+        same = set(old.files) == set(arrays) and all(np.array_equal(old[k], v) for k, v in arrays.items())
+        print(f"{name:28s} {'same' if same else 'DIFFERS'}")
+        return same
+    np.savez_compressed(out, **arrays)
     print(f"{name:28s} V={pb.nvars:6d} P={pb.nprops:6d} expected={expected} root={sha[:12]}")
+    return True
 
 
-def main():
-    for path, exp in csv.reader(open(os.path.join(REF, "test_list.csv"))):
+def main(reference, check=False):
+    benchmarks = os.path.join(reference, "benchmarks")
+    same = []
+    for path, exp in csv.reader(open(os.path.join(benchmarks, "test_list.csv"))):
         if path.endswith(".xml"):
             continue            # XCSP3: out of scope (SURVEY.md §2.2)
         name = os.path.basename(path)[:-4]
-        dump(name, os.path.join("/root/reference", path), int(exp))
+        same.append(dump(name, os.path.join(reference, path), int(exp), check))
     for name in ("accap_a3", "trains15", "example_wordpress7_500"):
-        dump(name, os.path.join(REF, name + ".fzn"), None)
+        same.append(dump(name, os.path.join(benchmarks, name + ".fzn"), None, check))
     for name in ("bigdom", "valve6"):            # unsolved_bugs_data: no expected answer; valve6 has set variables
-        dump(name, os.path.join(REF, "unsolved_bugs_data", name + ".fzn"), None)
+        same.append(dump(name, os.path.join(benchmarks, "unsolved_bugs_data", name + ".fzn"), None, check))
+    return all(same)
 
 
 if __name__ == "__main__":
-    main()
+    args = sys.argv[1:]
+    check = "--check" in args
+    args = [a for a in args if a != "--check"]
+    if len(args) != 1:
+        raise SystemExit(__doc__)
+    sys.exit(0 if main(args[0], check) else 1)

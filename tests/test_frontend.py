@@ -5,7 +5,10 @@ force over the FlatZinc semantics written here in Python and (b) by the oracle o
 by the C++ front-end; status and optimum must agree, and the C++ FlatZinc checker must accept the
 oracle's solution.
 """
+import hashlib
 import itertools
+import json
+import os
 
 import numpy as np
 import pytest
@@ -150,8 +153,7 @@ def test_checker_rejects_wrong_points():
     assert m.check_solution(bad) > 0
 
 
-def test_output_format_and_syntax_subset():
-    text = """% a comment
+SYNTAX_SUBSET = """% a comment
 predicate foo(var int: a);
 array [1..2] of int: w = [1,-1];
 int: k = 3;
@@ -166,7 +168,10 @@ constraint int_eq(p,int_le(2,a));
 constraint int_plus(a,k,t) :: defines_var(t);
 solve :: seq_search([int_search(g,first_fail,indomain_min,complete),bool_search([p],input_order,indomain_max,complete)]) maximize a;
 """
-    m = Model.from_fzn_text(text)
+
+
+def test_output_format_and_syntax_subset():
+    m = Model.from_fzn_text(SYNTAX_SUBSET)
     assert m.parsed_variables == 4 and m.parsed_constraints == 3
     assert len(m.problem.strategies) == 3          # two annotations + the default strategy
     r = orc.solve(m.problem)
@@ -295,10 +300,45 @@ def test_set_variable_checker_and_errors():
         Model.from_fzn_text("var set of int: S;\nsolve satisfy;\n")
 
 
-def test_unsolved_bugs_valve6_goes_through_the_front_end(reference_dir):
-    import os
-    m = Model.from_fzn(os.path.join(reference_dir, "benchmarks", "unsolved_bugs_data", "valve6.fzn"))
-    assert m.problem.nvars > 10000 and m.objective_kind == 1 and not m.root_failed
+# ---- stored models: the network the front-end builds is pinned (tests/golden/fzn, tests/golden/make_frontend_pins.py) ----
+
+FZN_DIR = os.path.join(os.path.dirname(os.path.abspath(__file__)), "golden", "fzn")
+PINS = json.load(open(os.path.join(FZN_DIR, "pins.json")))
+
+
+def network_sha(m):
+    """sha256 of everything the front-end hands the engine: bounds, propagators, strategies and objective."""
+    from tests import golden_io
+    h = hashlib.sha256()
+    for k, a in sorted(golden_io.problem_arrays(m.problem).items()):
+        h.update(k.encode())
+        h.update(np.ascontiguousarray(a, np.int32).tobytes())
+    h.update(np.array([m.objective_kind, m.user_objective_var, int(m.root_failed)], np.int32).tobytes())
+    return h.hexdigest()
+
+
+def test_stored_model_inventory():
+    assert len(PINS) == 23 and all(os.path.exists(os.path.join(FZN_DIR, n + ".fzn")) for n in PINS)
+
+
+@pytest.mark.parametrize("name", sorted(PINS))
+def test_stored_model_builds_the_pinned_network(name):
+    m = Model.from_fzn(os.path.join(FZN_DIR, name + ".fzn"))
+    assert network_sha(m) == PINS[name]["tnf_sha256"]
+
+
+@pytest.mark.parametrize("name", sorted(PINS))
+def test_stored_model_optimum_passes_the_flatzinc_checker(name):
+    m = Model.from_fzn(os.path.join(FZN_DIR, name + ".fzn"))
+    best = PINS[name]["optimum"]
+    if m.root_failed:
+        assert best is None
+        return
+    r = orc.solve(m.problem, depth=2)
+    assert r["exhaustive"] and r["has_solution"] == (best is not None)
+    if best is not None:
+        assert m.user_objective(r["lb"], r["ub"]) == best
+        assert m.check_solution(r["lb"]) == 0 and m.check_tnf(r["lb"]) == 0
 
 
 # ---- half reification (_imp), bool_lin_*, array_int_minimum / maximum ---------------------------------------------------

@@ -10,7 +10,7 @@
   all       the proven optima of the headline instances (tests/golden/optima.json) are reproduced when the
             search completes, and never contradicted when it does not.
 
-Nothing here reads /root/reference; the oracle is the checker.
+The oracle is the checker.
 """
 import json
 import os

@@ -1,6 +1,6 @@
 """GPU parity tests: the CUDA engine (through the C ABI) against the CPU oracle, bit for bit.
 
-Everything here needs a B200; nothing reads /root/reference.
+Everything here needs a B200.
 """
 import numpy as np
 import pytest

@@ -1,5 +1,5 @@
-import time, sys
-sys.path.insert(0,'/root/repo')
+import os, time, sys
+sys.path.insert(0, os.path.dirname(os.path.dirname(os.path.abspath(__file__))))
 from tests import golden_io
 from turbo_b200 import engine, abi
 pb,_=golden_io.load('trains15')
