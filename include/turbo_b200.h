@@ -166,6 +166,23 @@ tb_status tb_solve(tb_solver*, volatile int32_t* stop_flag,
                    int32_t* best_lb, int32_t* best_ub, int32_t* has_solution,
                    int32_t* exhaustive, tb_stats* stats);
 
+/* Solves nroots problems that share this solver's network and strategies and differ in their root domains
+ * (root_lb / root_ub laid out [nroots][nvars]), in one launch of the solve kernel. Each root is searched as if it
+ * were the root store of its own tb_solve: its own incumbent, its own first-solution stop for satisfaction, its own
+ * result. Outputs: best_lb / best_ub [nroots][nvars] (may be NULL; rows of roots without a solution are left as they
+ * are), has_solution / exhaustive [nroots], objective [nroots] (value of obj_var in the returned store; TB_POS_INF
+ * when there is none or the problem is a satisfaction problem), stats = the whole batch (counters summed,
+ * eps_num_subproblems = nroots * 2^d). stop_flag and the solver's timeout apply to the whole batch; a root whose
+ * search had ended before them stays exhaustive.
+ * Every root must narrow the solver's root (root_lb >= problem lb, root_ub <= problem ub) and nroots >= 1, else
+ * TB_ERR_INVALID; a root with an empty domain is legal (no solution, exhaustive). Subproblems: subproblems_power = -1
+ * picks the smallest d with nroots * 2^d >= subproblems_factor * min(blocks, 4 * SMs), an explicit d applies per
+ * root; d shrinks until nroots * 2^d fits 2^40. TB_ERR_UNSUPPORTED: linked or sharded solvers (gpu_world > 1), the
+ * STORE_CLUSTER placement, tb_stream_solutions enabled. */
+tb_status tb_solve_batch(tb_solver*, int32_t nroots, const int32_t* root_lb, const int32_t* root_ub,
+                         volatile int32_t* stop_flag, int32_t* best_lb, int32_t* best_ub,
+                         int32_t* has_solution, int32_t* exhaustive, int32_t* objective, tb_stats* stats);
+
 /* Intermediate solutions (-i / -a; the reference's consumer thread, gpu_dive_and_solve.hpp:100-132; its barebones
  * architecture cannot, barebones_dive_and_solve.hpp:465-467).  tb_stream_solutions (before tb_solve) makes every
  * improving solution also land in a ring of `slots` store images; tb_poll_solution, called from ANOTHER host thread

@@ -294,9 +294,15 @@ __device__ __forceinline__ void decode_word(unsigned long long w, int& a, int& b
   if (!tbd::cls_loads_z(CLS)) c = (c << (32 - TBC_FIELD_BITS)) >> (32 - TBC_FIELD_BITS);
 }
 
+// Per-CTA state of the BATCH kernels only (a function-scope __shared__ object: the other kernels never reference it).
+struct BatchCtl { int won; };
+__device__ __forceinline__ BatchCtl& batch_ctl() { __shared__ BatchCtl b; return b; }
+
 // TMALL: every visit of every warp finds its propagator word in tensor memory (the table fits): the sweep is compiled
 // without the L2 path and without the test that chooses between the two.
-template <int MEM, bool ACT = false, bool TMALL = false>
+// BATCH: tb_solve_batch - subproblem g of depth D belongs to root g >> D, which has its own image, incumbent, stop word,
+// best store and closed-weight counter (BatchRoot); every batch-only branch is `if constexpr`.
+template <int MEM, bool ACT = false, bool TMALL = false, bool BATCH = false>
 struct Ctx {
   const DevParams& P;
   Ctl& c;
@@ -336,15 +342,23 @@ struct Ctx {
   __device__ __forceinline__ unsigned long long bound_word(int b) const {
     return ((unsigned long long)(~P.epoch) << 32) | (unsigned long long)((unsigned)b ^ 0x80000000u);
   }
+  // ---- tb_solve_batch: the root of the current task and its cells (thread 0) ----------------------------------------
+  __device__ __forceinline__ BatchRoot& batch_root() const { return P.batch_state[c.task_idx >> c.task_depth]; }
+  __device__ __forceinline__ bool batch_root_over() const { return *(volatile int*)&batch_root().stop != 0; }
+  __device__ __forceinline__ void batch_cut() const { *(volatile int*)&batch_root().cut = 1; }
+  __device__ __forceinline__ unsigned long long* bound_cell() const {
+    if constexpr (BATCH) return &batch_root().bound;
+    else return P.cells + TB_CELL_BOUND;
+  }
   // GridData::appx_best_bound (:426): this GPU's copy; a word left by another run reads as "no incumbent"
   __device__ __forceinline__ int read_bound() const {
-    const unsigned long long v = *(volatile unsigned long long*)(P.cells + TB_CELL_BOUND);
+    const unsigned long long v = *(volatile unsigned long long*)bound_cell();
     return (unsigned)(v >> 32) == ~P.epoch ? (int)((unsigned)v ^ 0x80000000u) : TBD_PINF;
   }
   // an improving solution goes to this GPU's cell and to every peer's over NVLink (:997 + SURVEY 8e)
   __device__ __forceinline__ void publish_bound(int l) const {
     const unsigned long long w = bound_word(l);
-    atomicMin(P.cells + TB_CELL_BOUND, w);
+    atomicMin(bound_cell(), w);
     for (int g = 0; g < P.npeers; ++g) atomicMin_system(P.peer_cells[g] + TB_CELL_BOUND, w);
   }
   __device__ __forceinline__ bool stop_raised() const {
@@ -1094,6 +1108,36 @@ struct Ctx {
     }
   }
 
+  // ---- tb_solve_batch: the best store of the task's root --------------------------------------------------------
+  // Optimisation: the block takes the root's lock and writes the image only if its bound still beats the image's; the
+  // copy has landed before the lock is released, so two writers never interleave. Satisfaction: only the block that won
+  // the root's stop word gets here, and writes without the lock.
+  __device__ __forceinline__ void batch_save_best(int bound) {
+    BatchCtl& b = batch_ctl();
+    if (tid == 0) {
+      BatchRoot& r = batch_root();
+      if (P.obj_var >= 0) {
+        while (atomicCAS(&r.lock, 0, 1) != 0) __nanosleep(64);
+        __threadfence();
+        b.won = bound < *(volatile int*)&r.img_bound;
+      } else b.won = 1;
+    }
+    sync();
+    const bool won = b.won != 0;
+    if (won) {
+      save_store(P.batch_best + (size_t)(c.task_idx >> c.task_depth) * 2 * P.vpad, true);
+      if (threadIdx.x == 0) bulk_wait_all();
+      __threadfence();
+      sync();
+    }
+    if (tid == 0) {
+      BatchRoot& r = batch_root();
+      if (won) { *(volatile int*)&r.img_bound = bound; *(volatile int*)&r.has = 1; }
+      __threadfence();
+      if (P.obj_var >= 0) atomicExch(&r.lock, 0);
+    }
+  }
+
   // ---- propagate() (barebones :903-1031) -----------------------------------------------------------
   // Runs the fixpoint, classifies the node, records solutions, updates counters and the stop flag.
   // Sets c.leaf / c.failed / c.stop uniformly (valid after return).
@@ -1123,14 +1167,21 @@ struct Ctx {
           st->best_bound = l;
         }
       } else {
-        improved = st->solutions == 0;          // satisfaction: first solution wins
-        sync();
+        if constexpr (BATCH) {                  // satisfaction: the first solution of the ROOT wins
+          if (tid == 0) batch_ctl().won = atomicCAS(&batch_root().stop, 0, 1) == 0;
+          sync();
+          improved = batch_ctl().won != 0;
+        } else {
+          improved = st->solutions == 0;          // satisfaction: first solution wins
+          sync();
+        }
         if (tid == 0) st->t_best = (long long)(globaltimer_ns() - P.t_start);
       }
       if (improved) {
-        save_store(g_best);
+        if constexpr (BATCH) batch_save_best(P.obj_var >= 0 ? c.best_bound : 0);
+        else save_store(g_best);
         if (tid == 0) { st->solutions++; st->has_best = 1; }
-        if (P.stream_slots) stream_solution(P.obj_var >= 0 ? c.best_bound : 0);
+        if constexpr (!BATCH) { if (P.stream_slots) stream_solution(P.obj_var >= 0 ? c.best_bound : 0); }
       }
     }
     if (tid == 0) {
@@ -1143,12 +1194,18 @@ struct Ctx {
       st->t_fixpoint += (long long)(t1 - t0);
       if (solution && P.obj_var < 0) {       // satisfaction: stop everybody after the first solution
         st->exhaustive = 0;
-        c.stop = 1;
-        raise_stop(true);
+        // (batch: the root's stop word is raised, its blocks move on; a root stopped by its first solution is never
+        // exhaustive, whatever weight the task that found it closes)
+        if constexpr (BATCH) batch_cut();
+        else {
+          c.stop = 1;
+          raise_stop(true);
+        }
       }
       if ((P.cutnodes && st->nodes >= P.cutnodes) || stop_raised()) {
         st->exhaustive = 0;
         c.stop = 1;
+        if constexpr (BATCH) batch_cut();
       }
     }
     sync();
@@ -1169,7 +1226,11 @@ struct Ctx {
 
   // thread 0 only
   __device__ __forceinline__ void push_decision(int val_order, int var) {
-    if (c.depth >= P.max_depth) { st->error = TB_ERR_DEPTH; st->exhaustive = 0; c.stop = 1; raise_stop(false); c.pushed = 0; return; }
+    if (c.depth >= P.max_depth) {
+      st->error = TB_ERR_DEPTH; st->exhaustive = 0; c.stop = 1; raise_stop(false); c.pushed = 0;
+      if constexpr (BATCH) batch_cut();
+      return;
+    }
     int l, u; store.ld(var, l, u);
     Decision d;
     d.var = var; d.cur = -1;
@@ -1253,7 +1314,7 @@ struct Ctx {
       if (!c.leaf) {
         bool pushed = split();
         if (tid == 0) {
-          if (!pushed) { c.leaf = 1; st->exhaustive = 0; }
+          if (!pushed) { c.leaf = 1; st->exhaustive = 0; if constexpr (BATCH) batch_cut(); }
           else {
             --c.remaining_depth;
             --c.depth;                        // decisions are not recorded while diving
@@ -1294,11 +1355,20 @@ struct Ctx {
           c.remaining_depth = c.task_depth; c.leaf = 0; c.failed = 0;
           c.task_nodes = 0; c.abandon = 0;
           c.t_mark = (long long)globaltimer_ns();
+          if constexpr (BATCH) {
+            c.best_bound = TBD_PINF;          // the incumbent of ANOTHER root must never prune this one
+            c.abandon = batch_root_over();    // (nothing left to do for a root that is over)
+          }
         }
-        for (int i = tid; i < P.nsnap; i += T) g_snap_tag[i] = -1;       // snapshots belong to one subproblem
-        load_store(P.root_store);
-        sync();
-        mode = M_DIVE;
+        if constexpr (BATCH) sync();
+        if (BATCH && c.abandon) mode = M_NEXT;
+        else {
+          for (int i = tid; i < P.nsnap; i += T) g_snap_tag[i] = -1;       // snapshots belong to one subproblem
+          if constexpr (BATCH) load_store(P.batch_roots + (size_t)(idx >> c.task_depth) * 2 * P.vpad);
+          else load_store(P.root_store);
+          sync();
+          mode = M_DIVE;
+        }
       }
       if (mode == M_DIVE && !(c.remaining_depth > 0 && !c.leaf && !c.stop)) {
         // the dive is over: at the subproblem (remaining depth 0), or at a leaf above it
@@ -1330,6 +1400,11 @@ struct Ctx {
             }
             if ((idx & ((1ull << remaining) - 1ull)) == 0ull) st->eps_skipped += next - idx;
           }
+          // the leaf closes the 2^remaining tasks of depth D below it: counted once, by the task aligned on them
+          if constexpr (BATCH) {
+            if (tid == 0 && (idx & ((1ull << remaining) - 1ull)) == 0ull)
+              atomicAdd(&batch_root().closed, 1ull << (TB_BATCH_WEIGHT_BITS - c.task_depth + remaining));
+          }
           mode = M_NEXT;
         } else if (!c.stop) {
           if (tid == 0 && P.has_eps_strategy) { c.cur_strategy = max(1, c.cur_strategy); c.next_unassigned = 0; }
@@ -1348,13 +1423,20 @@ struct Ctx {
               moved |= store.embed(P.obj_var, TBD_NINF, tbd::pred(c.best_bound));
               if (moved) mark_var(P.obj_var);
             }
-            if (appx == TBD_NINF) { c.stop = 1; raise_stop(true); }
+            if (appx == TBD_NINF) {
+              if constexpr (BATCH) { *(volatile int*)&batch_root().stop = 1; batch_cut(); }   // this root only
+              else { c.stop = 1; raise_stop(true); }
+            }
           }
+          // batch: a root that is over (see propagate) is left at the next node, by every block working on it
+          bool over = false;
+          if constexpr (BATCH) { if (tid == 0) over = batch_root_over(); }
           // tail splitting: somebody is waiting for work and this subproblem has been going on for a while
-          if (tid == 0 && P.split_bits && ++c.task_nodes >= (unsigned)P.split_min_nodes && (c.task_nodes & 255u) == 0u &&
-              somebody_waits() && c.task_depth + P.split_bits <= 56 &&
+          if (tid == 0 && !over && P.split_bits && ++c.task_nodes >= (unsigned)P.split_min_nodes && (c.task_nodes & 255u) == 0u &&
+              somebody_waits() && c.task_depth + P.split_bits <= (BATCH ? P.batch_max_depth : 56) &&
               *(volatile unsigned*)(P.split_ctl + TB_SPLIT_N) < (unsigned)TB_SPLIT_CAP)
             c.abandon = push_split() ? 1 : 0;
+          if constexpr (BATCH) { if (over) c.abandon = 1; }
           sync();
           if (c.stop) mode = M_SOLVE_END;
           else if (c.abandon) mode = M_NEXT;          // its children are in the pool now; this block takes one of them
@@ -1363,6 +1445,10 @@ struct Ctx {
       if (mode == M_SOLVE_END) {
         sync();
         if (tid == 0 && !(P.cutnodes && st->nodes >= P.cutnodes) && !stop_raised()) { if (c.task_entry < 0) st->eps_solved += 1; else st->eps_parts += 1; }
+        // (a block that was cut marked the root in propagate / push_decision)
+        if constexpr (BATCH) {
+          if (tid == 0 && !c.stop) atomicAdd(&batch_root().closed, 1ull << (TB_BATCH_WEIGHT_BITS - c.task_depth));
+        }
         mode = M_NEXT;
       }
       if (mode == M_NEXT) {
@@ -1381,7 +1467,7 @@ struct Ctx {
         if (!c.leaf) {
           bool pushed = split();
           if (tid == 0) {
-            if (!pushed) { c.leaf = 1; st->exhaustive = 0; }
+            if (!pushed) { c.leaf = 1; st->exhaustive = 0; if constexpr (BATCH) batch_cut(); }
             else {
               --c.remaining_depth;
               --c.depth;                        // decisions are not recorded while diving
@@ -1418,7 +1504,7 @@ struct Ctx {
             }
           }
           if (tid == 0) {
-            if (!pushed) { c.leaf = 1; st->exhaustive = 0; }
+            if (!pushed) { c.leaf = 1; st->exhaustive = 0; if constexpr (BATCH) batch_cut(); }
             else {
               Decision& d = dec[c.depth - 1];
               d.cur = 0;
@@ -1485,8 +1571,8 @@ __device__ __forceinline__ Ctl* shared_ctl(Ctl* local) {
   return (Ctl*)r;
 }
 
-template <int MEM, bool ACT, bool TMALL>
-__device__ __forceinline__ void ctx_init(Ctx<MEM, ACT, TMALL>& k, Ctl* local, unsigned char* dyn) {
+template <int MEM, bool ACT, bool TMALL, bool BATCH>
+__device__ __forceinline__ void ctx_init(Ctx<MEM, ACT, TMALL, BATCH>& k, Ctl* local, unsigned char* dyn) {
   const DevParams& P = k.P;
   k.lc = local;
   if (MEM == TB_MEM_STORE_CLUSTER) {
@@ -1554,7 +1640,7 @@ __device__ __forceinline__ void ctx_init(Ctx<MEM, ACT, TMALL>& k, Ctl* local, un
       const int ch = warp + v * nwarps;
       // (the table is padded behind its end: a chunk index past nchunks reads zeros that are never evaluated)
       unsigned long long wd = __ldg(P.words + (size_t)ch * 32 + lane);
-      if (Ctx<MEM, ACT, TMALL>::kAbs && ch < P.nchunks) {
+      if (Ctx<MEM, ACT, TMALL, BATCH>::kAbs && ch < P.nchunks) {
         int cls = 0;
 #pragma unroll
         for (int step = 16; step > 0; step >>= 1)
@@ -1577,7 +1663,7 @@ __device__ __forceinline__ void ctx_init(Ctx<MEM, ACT, TMALL>& k, Ctl* local, un
     }
     if (bytes) { while (!mbar_try_wait(&local->mbar, k.mbar_phase)) {} k.mbar_phase ^= 1; }
     k.words = (const unsigned long long*)sprops;
-    if (Ctx<MEM, ACT, TMALL>::kAbs) {
+    if (Ctx<MEM, ACT, TMALL, BATCH>::kAbs) {
       // the staged copy is this CTA's own: rewrite its slot fields to absolute shared addresses (see StoreAbs)
       unsigned long long* tw = (unsigned long long*)sprops;
       for (int i = threadIdx.x; i < P.nchunks * 32; i += blockDim.x) {
@@ -1593,8 +1679,8 @@ __device__ __forceinline__ void ctx_init(Ctx<MEM, ACT, TMALL>& k, Ctl* local, un
   }
 }
 
-template <int MEM, bool ACT, bool TMALL>
-__device__ __forceinline__ void ctx_finish(Ctx<MEM, ACT, TMALL>& k) {
+template <int MEM, bool ACT, bool TMALL, bool BATCH>
+__device__ __forceinline__ void ctx_finish(Ctx<MEM, ACT, TMALL, BATCH>& k) {
   // fold the per-thread / per-warp counters into the block statistics
   unsigned n = k.narrowed;
   for (int o = 16; o > 0; o >>= 1) n += __shfl_xor_sync(0xffffffffu, n, o);
@@ -1612,13 +1698,13 @@ __device__ __forceinline__ void ctx_finish(Ctx<MEM, ACT, TMALL>& k) {
 // kernels
 // ================================================================================================
 
-// The persistent dive-and-solve kernel (gpu_barebones_solve, barebones :620-901).
-template <int MEM, bool ACT = false, bool TMALL = false>
+// The persistent dive-and-solve kernel (gpu_barebones_solve, barebones :620-901). BATCH: tb_solve_batch.
+template <int MEM, bool ACT = false, bool TMALL = false, bool BATCH = false>
 __global__ void __launch_bounds__(TB_MAX_THREADS) solve_kernel(const __grid_constant__ DevParams P) {
   extern __shared__ __align__(128) unsigned char dyn[];
   __shared__ Ctl c_local;
   Ctl& c = *shared_ctl<MEM>(&c_local);
-  Ctx<MEM, ACT, TMALL> k(P, c);
+  Ctx<MEM, ACT, TMALL, BATCH> k(P, c);
   ctx_init(k, &c_local, dyn);
   const int tid = k.tid;
   BlockStats* st = k.st;
@@ -1809,6 +1895,10 @@ struct tb_solver {
   // batch buffers (grown on demand)
   int *d_in_lb = nullptr, *d_in_ub = nullptr, *d_out_lb = nullptr, *d_out_ub = nullptr, *d_out_i0 = nullptr, *d_out_i1 = nullptr;
   size_t batch_cap = 0;
+  // tb_solve_batch buffers (grown on demand): root images, best images, BatchRoot cells
+  int *d_batch_roots = nullptr, *d_batch_best = nullptr;
+  BatchRoot* d_batch_state = nullptr;
+  size_t batch_roots_cap = 0;
   int32_t* h_pinned_one = nullptr;
 };
 
@@ -2591,12 +2681,16 @@ static double now_ms() {
   return t.tv_sec * 1e3 + t.tv_nsec * 1e-6;
 }
 
-extern "C" tb_status tb_solve(tb_solver* s, volatile int32_t* stop_flag, int32_t* best_lb, int32_t* best_ub,
-                              int32_t* has_solution, int32_t* exhaustive, tb_stats* stats) {
-  if (!s) { set_error("null solver"); return TB_ERR_INVALID; }
-  CU(cudaSetDevice(s->device));
-  DevParams& P = s->P;
-  const double t_begin = now_ms();
+// What tb_solve and tb_solve_batch share: a new epoch, the grid cells and the split pool reset, the launch (`launch`
+// starts the solve kernel on P), the poll loop on *stop_flag / the timeout (wait_solving_ends, memory_gpu.hpp:174-196)
+// and the block statistics.
+struct SearchRun {
+  bool interrupted = false;          // the host raised the stop word (stop_flag or timeout)
+  float kernel_ms = 0.f;
+  std::vector<BlockStats> blocks;
+};
+template <class Launch>
+static tb_status run_search(tb_solver* s, DevParams& P, double t_begin, volatile int32_t* stop_flag, Launch&& launch, SearchRun& run) {
   tb_status rc;
   if ((rc = reset_stats(s, s->num_blocks))) return rc;
   P.t_start = host_globaltimer_probe(s);
@@ -2623,40 +2717,51 @@ extern "C" tb_status tb_solve(tb_solver* s, volatile int32_t* stop_flag, int32_t
   }
   CU(cudaMemcpyAsync(s->d_cells + TB_CELL_NEXT, &first_free, sizeof(first_free), cudaMemcpyHostToDevice, s->stream));
   CU(cudaEventRecord(s->ev_start, s->stream));
-  rc = dispatch(s, [&](auto M, auto A, auto TM) -> tb_status {
-    CU(launch_workers(s, solve_kernel<decltype(M)::value, decltype(A)::value, decltype(TM)::value>, s->num_blocks, P));
-    CU(cudaGetLastError());
-    return TB_OK;
-  });
-  if (rc) return rc;
+  if ((rc = launch(P))) return rc;
   CU(cudaEventRecord(s->ev_stop, s->stream));
-  // wait_solving_ends (memory_gpu.hpp:174-196): poll stop / timeout, raise the device flag asynchronously
-  bool interrupted = false;
   while (true) {
     cudaError_t q = cudaEventQuery(s->ev_stop);
     if (q == cudaSuccess) break;
     if (q != cudaErrorNotReady) { set_error(std::string("kernel failed: ") + cudaGetErrorString(q)); return TB_ERR_CUDA; }
     bool must = (stop_flag && *stop_flag) || (s->opt.timeout_ms && now_ms() - t_begin >= (double)s->opt.timeout_ms);
-    if (must && !interrupted) {
-      interrupted = true;
+    if (must && !run.interrupted) {
+      run.interrupted = true;
       CU(cudaMemcpyAsync((int*)(s->d_cells + TB_CELL_STOP) + 1, s->h_pinned_one, sizeof(int), cudaMemcpyHostToDevice, s->copy_stream));
     }
     struct timespec ts = {0, 200000};
     nanosleep(&ts, nullptr);
   }
   CU(cudaStreamSynchronize(s->stream));
-  float kms = 0.f;
-  CU(cudaEventElapsedTime(&kms, s->ev_start, s->ev_stop));
-  std::vector<BlockStats> bs((size_t)s->num_blocks);
-  CU(cudaMemcpy(bs.data(), P.stats, bs.size() * sizeof(BlockStats), cudaMemcpyDeviceToHost));
+  CU(cudaEventElapsedTime(&run.kernel_ms, s->ev_start, s->ev_stop));
+  run.blocks.resize((size_t)s->num_blocks);
+  CU(cudaMemcpy(run.blocks.data(), P.stats, run.blocks.size() * sizeof(BlockStats), cudaMemcpyDeviceToHost));
+  return TB_OK;
+}
+
+extern "C" tb_status tb_solve(tb_solver* s, volatile int32_t* stop_flag, int32_t* best_lb, int32_t* best_ub,
+                              int32_t* has_solution, int32_t* exhaustive, tb_stats* stats) {
+  if (!s) { set_error("null solver"); return TB_ERR_INVALID; }
+  CU(cudaSetDevice(s->device));
+  DevParams& P = s->P;
+  const double t_begin = now_ms();
+  SearchRun run;
+  tb_status rc = run_search(s, P, t_begin, stop_flag, [&](const DevParams& Pl) {
+    return dispatch(s, [&](auto M, auto A, auto TM) -> tb_status {
+      CU(launch_workers(s, solve_kernel<decltype(M)::value, decltype(A)::value, decltype(TM)::value>, s->num_blocks, Pl));
+      CU(cudaGetLastError());
+      return TB_OK;
+    });
+  }, run);
+  if (rc) return rc;
+  const std::vector<BlockStats>& bs = run.blocks;
   tb_stats st; memset(&st, 0, sizeof(st));
   st.exhaustive = 1;
   fill_config(s, &st);
   int best_block = -1;
   reduce_stats(bs, &st, &best_block);
   for (auto& b : bs) if (b.error) { set_error("decision stack overflow (raise max_depth)"); rc = (tb_status)b.error; }
-  if (interrupted) st.exhaustive = 0;
-  st.kernel_ms = kms;
+  if (run.interrupted) st.exhaustive = 0;
+  st.kernel_ms = run.kernel_ms;
   st.timers_ns[TB_TIMER_OVERALL] = (int64_t)((now_ms() - t_begin) * 1e6);
   if (has_solution) *has_solution = best_block >= 0;
   s->last_lb.assign((size_t)std::max(1, s->nvars), 0); s->last_ub.assign((size_t)std::max(1, s->nvars), 0);
@@ -2669,6 +2774,136 @@ extern "C" tb_status tb_solve(tb_solver* s, volatile int32_t* stop_flag, int32_t
   if (exhaustive) *exhaustive = st.exhaustive;
   if (stats) *stats = st;
   s->last_stats = st; s->last_has = best_block >= 0; s->last_exhaustive = st.exhaustive; s->last_valid = 1;
+  return rc;
+}
+
+static tb_status ensure_batch_roots(tb_solver* s, size_t n) {
+  if (n <= s->batch_roots_cap) return TB_OK;
+  tb_status rc;
+  const size_t img = (size_t)2 * s->P.vpad;
+  if ((rc = dev_alloc(s, &s->d_batch_roots, n * img))) return rc;
+  if ((rc = dev_alloc(s, &s->d_batch_best, n * img))) return rc;
+  if ((rc = dev_alloc(s, &s->d_batch_state, n))) return rc;
+  s->batch_roots_cap = n;
+  return TB_OK;
+}
+
+extern "C" tb_status tb_solve_batch(tb_solver* s, int32_t nroots, const int32_t* root_lb, const int32_t* root_ub,
+                                    volatile int32_t* stop_flag, int32_t* best_lb, int32_t* best_ub,
+                                    int32_t* has_solution, int32_t* exhaustive, int32_t* objective, tb_stats* stats) {
+  if (!s || nroots < 1 || (s->nvars && (!root_lb || !root_ub))) {
+    set_error("tb_solve_batch: needs nroots >= 1 and root_lb / root_ub"); return TB_ERR_INVALID;
+  }
+  if (!s->peer_cells.empty() || s->opt.gpu_world > 1) { set_error("tb_solve_batch: a batch runs on one GPU (linked or sharded solvers are not supported)"); return TB_ERR_UNSUPPORTED; }
+  if (s->mem_kind == TB_MEM_STORE_CLUSTER) { set_error("tb_solve_batch: the STORE_CLUSTER placement is not supported"); return TB_ERR_UNSUPPORTED; }
+  if (s->P.stream_slots) { set_error("tb_solve_batch: intermediate solutions (tb_stream_solutions) are not supported"); return TB_ERR_UNSUPPORTED; }
+  // Every root narrows the solver's root: the layout pass chose each propagator's device class (folded constants, exact
+  // 32-bit arithmetic) from the root bounds, which stays valid under narrowing only.
+  const size_t nv = (size_t)s->nvars;
+  for (size_t r = 0; r < (size_t)nroots; ++r)
+    for (size_t v = 0; v < nv; ++v)
+      if (root_lb[r * nv + v] < s->root_lb[v] || root_ub[r * nv + v] > s->root_ub[v]) {
+        set_error("tb_solve_batch: root " + std::to_string(r) + " widens the solver's domain of variable " + std::to_string(v));
+        return TB_ERR_INVALID;
+      }
+  CU(cudaSetDevice(s->device));
+  const double t_begin = now_ms();
+  // subproblems per root: -sub -1 is the tb_create rule with the roots folded in; the index (r << d) | local must fit
+  // the dispenser's TB_K_BITS
+  int d = s->opt.subproblems_power;
+  if (d < 0) {
+    d = 0;
+    const unsigned long long want = (unsigned long long)s->opt.subproblems_factor * (unsigned long long)std::min(s->num_blocks, 4 * s->num_sms);
+    while (((unsigned long long)nroots << d) < want && d < TB_K_BITS) ++d;
+  }
+  while (d > 0 && ((unsigned long long)nroots << d) > (1ull << TB_K_BITS)) --d;
+  int root_bits = 0;
+  while ((1ull << root_bits) < (unsigned long long)nroots) ++root_bits;
+  tb_status rc;
+  if ((rc = ensure_batch_roots(s, (size_t)nroots))) return rc;
+  DevParams P = s->P;
+  const size_t img = (size_t)2 * P.vpad;
+  // root images in the slot layout; a root with an empty referenced variable fails before any search, as tb_solve's
+  // does: it is over from the start, and its subproblems are skipped
+  std::vector<int> images((size_t)nroots * img, 0);
+  std::vector<BatchRoot> state((size_t)nroots);
+  std::vector<char> failed((size_t)nroots, 0);
+  for (size_t r = 0; r < (size_t)nroots; ++r) {
+    int* im = images.data() + r * img;
+    for (size_t v = 0; v < nv; ++v) {
+      const int l = root_lb[r * nv + v], u = root_ub[r * nv + v];
+      im[img_lb(s, (int)v)] = l; im[img_ub(s, (int)v)] = u;
+      if (l > u && s->layout.referenced[v]) failed[r] = 1;
+    }
+    BatchRoot& b = state[r];
+    memset(&b, 0, sizeof(b));
+    b.bound = ~0ull;                                   // epoch 0, no incumbent (as the cell at tb_create)
+    b.img_bound = TBD_PINF;
+    b.stop = failed[r];
+  }
+  CU(cudaMemcpyAsync(s->d_batch_roots, images.data(), images.size() * sizeof(int), cudaMemcpyHostToDevice, s->stream));
+  CU(cudaMemcpyAsync(s->d_batch_state, state.data(), state.size() * sizeof(BatchRoot), cudaMemcpyHostToDevice, s->stream));
+  P.batch_roots = s->d_batch_roots; P.batch_best = s->d_batch_best; P.batch_state = s->d_batch_state;
+  P.subproblems_power = d;
+  P.num_subproblems = (unsigned long long)nroots << d;
+  P.batch_max_depth = std::min(TB_BATCH_WEIGHT_BITS, 64 - root_bits);
+  // (the BATCH kernel has the registers of the others - __launch_bounds__ caps them all - and a few bytes more of
+  // static shared memory, which the 64 bytes configure() reserves beside Ctl cover: the grid of tb_create fits)
+  rc = dispatch(s, [&](auto M, auto A, auto TM) -> tb_status {
+    if constexpr (decltype(M)::value != TB_MEM_STORE_CLUSTER) {
+      if (s->shared_bytes)
+        CU(cudaFuncSetAttribute(solve_kernel<decltype(M)::value, decltype(A)::value, decltype(TM)::value, true>,
+                                cudaFuncAttributeMaxDynamicSharedMemorySize, (int)s->shared_bytes));
+    }
+    return TB_OK;
+  });
+  if (rc) return rc;
+  SearchRun run;
+  rc = run_search(s, P, t_begin, stop_flag, [&](const DevParams& Pl) {
+    return dispatch(s, [&](auto M, auto A, auto TM) -> tb_status {
+      if constexpr (decltype(M)::value == TB_MEM_STORE_CLUSTER) { set_error("tb_solve_batch: STORE_CLUSTER"); return TB_ERR_UNSUPPORTED; }
+      else {
+        CU(launch_workers(s, solve_kernel<decltype(M)::value, decltype(A)::value, decltype(TM)::value, true>, s->num_blocks, Pl));
+        CU(cudaGetLastError());
+        return TB_OK;
+      }
+    });
+  }, run);
+  if (rc) return rc;
+  CU(cudaMemcpy(state.data(), s->d_batch_state, state.size() * sizeof(BatchRoot), cudaMemcpyDeviceToHost));
+  bool any = false;
+  for (auto& b : state) any |= b.has != 0;
+  if (any) CU(cudaMemcpy(images.data(), s->d_batch_best, images.size() * sizeof(int), cudaMemcpyDeviceToHost));
+  tb_stats st; memset(&st, 0, sizeof(st));
+  st.exhaustive = 1;
+  fill_config(s, &st);
+  st.subproblems_power = d;
+  st.eps_num_subproblems = P.num_subproblems;
+  reduce_stats(run.blocks, &st, nullptr);
+  for (auto& b : run.blocks) if (b.error) { set_error("decision stack overflow (raise max_depth)"); rc = (tb_status)b.error; }
+  // per root: exhaustive iff all of its search space was closed and no block was cut while searching it (roots that
+  // finished before a stop or a timeout stay exhaustive); a failed root is exhaustive without a solution
+  const unsigned long long all = 1ull << TB_BATCH_WEIGHT_BITS;
+  int all_exhaustive = 1;
+  std::vector<int32_t> lb(std::max<size_t>(1, nv)), ub(std::max<size_t>(1, nv));
+  for (size_t r = 0; r < (size_t)nroots; ++r) {
+    const BatchRoot& b = state[r];
+    const bool has = !failed[r] && b.has;
+    const int exh = failed[r] ? 1 : (b.closed == all && !b.cut);
+    all_exhaustive &= exh;
+    if (has_solution) has_solution[r] = has;
+    if (exhaustive) exhaustive[r] = exh;
+    if (objective) objective[r] = TB_POS_INF;
+    if (!has) continue;
+    unpack_store(s, images.data() + r * img, lb.data(), ub.data());
+    if (objective && s->root_obj_var >= 0) objective[r] = lb[(size_t)s->root_obj_var];
+    if (best_lb && nv) memcpy(best_lb + r * nv, lb.data(), nv * 4);
+    if (best_ub && nv) memcpy(best_ub + r * nv, ub.data(), nv * 4);
+  }
+  st.exhaustive = all_exhaustive;
+  st.kernel_ms = run.kernel_ms;
+  st.timers_ns[TB_TIMER_OVERALL] = (int64_t)((now_ms() - t_begin) * 1e6);
+  if (stats) *stats = st;
   return rc;
 }
 

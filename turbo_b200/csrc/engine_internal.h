@@ -70,6 +70,23 @@ struct SplitEntry {
 };
 static_assert(sizeof(SplitEntry) == 32, "TB_CELL_BLOCK_BYTES counts 32 bytes per pool entry");
 #define TB_SPLIT_CAP 16384
+
+// tb_solve_batch: what the grid shares about one root of the batch (written by the host before each launch).
+// Subproblem index g = (r << d) | local; a task of depth D belongs to root g >> D.
+struct BatchRoot {
+  unsigned long long bound;     // the root's incumbent, the TB_CELL_BOUND word (epoch-tagged, unsigned atomicMin)
+  unsigned long long closed;    // weight of the root's search space closed: 2^(56 - D) per task of depth D searched to
+                                // the end, 2^(56 - D + rem) per dive leaf at remaining depth rem; 2^56 = everything
+  int stop;                     // the root is over (first solution of a satisfaction problem, unbounded objective)
+  int cut;                      // a block was cut (stop, cutnodes, depth) while searching it, or stop was raised
+  int lock;                     // one writer of the root's best image at a time
+  int has;                      // the best image holds a solution
+  int img_bound;                // objective of the best image (TBD_PINF = none)
+  int pad_;
+};
+static_assert(sizeof(BatchRoot) == 40, "host and device agree on BatchRoot");
+#define TB_BATCH_WEIGHT_BITS 56
+
 // words of the split control block (unsigned), which lives in the cell block (TB_CELL_SPLIT) so that the peers see it
 enum { TB_SPLIT_N = 0, TB_SPLIT_WAITING = 1, TB_SPLIT_GONE = 2, TB_SPLIT_HINT = 3, TB_SPLIT_STARTED = 4, TB_SPLIT_NSLOTS = 5, TB_SPLIT_EPOCH = 6 };
 
@@ -129,4 +146,10 @@ struct DevParams {
   int tmem_cols, tmem_visits;
   int act_off;                           // byte offset of the active-set area in dynamic shared memory
   int act_fpw;                           // chunk flags per warp (multiple of 32): chunk ch is flag (ch / nwarps) of warp (ch % nwarps)
+  // tb_solve_batch (read by the BATCH kernels only): num_subproblems = nroots << subproblems_power
+  const int* batch_roots;                // [nroots][2 * vpad] root images, layout of a block store
+  int* batch_best;                       // [nroots][2 * vpad] best store of each root
+  BatchRoot* batch_state;                // [nroots]
+  int batch_max_depth;                   // deepest task: root bits + depth fit the 64-bit index, at most 56
+  int pad6_;
 };

@@ -38,6 +38,7 @@ def lib():
         L.tb_dive.argtypes = [vp, C.c_uint64, C.c_int32, i32p, i32p, i32p, i32p]
         L.tb_dive_batch.argtypes = [vp, C.c_uint64, C.c_int32, C.c_int32, i32p, i32p, i32p, i32p]
         L.tb_solve.argtypes = [vp, i32p, i32p, i32p, i32p, i32p, C.POINTER(abi.TbStats)]
+        L.tb_solve_batch.argtypes = [vp, C.c_int32, i32p, i32p, i32p, i32p, i32p, i32p, i32p, i32p, C.POINTER(abi.TbStats)]
         L.tb_link_peers.argtypes = [C.POINTER(vp), C.c_int32]
         L.tb_export_bound_handle.argtypes = [vp, vp]
         L.tb_import_peer_bounds.argtypes = [vp, vp, C.c_int32]
@@ -52,7 +53,7 @@ def lib():
         L.tb_version.restype = C.c_char_p
         L.tb_device_count.restype = C.c_int32
         for name in ("tb_create", "tb_propagate", "tb_propagate_batch", "tb_dive", "tb_dive_batch", "tb_solve",
-                     "tb_link_peers", "tb_export_bound_handle", "tb_import_peer_bounds", "tb_read_bound",
+                     "tb_solve_batch", "tb_link_peers", "tb_export_bound_handle", "tb_import_peer_bounds", "tb_read_bound",
                      "tb_get_config"):
             getattr(L, name).restype = C.c_int
         _LIB = L
@@ -229,6 +230,27 @@ class Solver:
             obj = int(lb[self.problem.obj_var])
         return dict(lb=lb[:self.problem.nvars], ub=ub[:self.problem.nvars], has_solution=bool(has.value),
                     exhaustive=bool(exh.value), objective=obj, stats=st.as_dict())
+
+    def solve_batch(self, lb, ub, stop_flag=None):
+        """tb_solve_batch: K roots of this solver's network ([K, nvars] int32 domains, each a narrowing of the
+        problem's), searched in one launch as K independent solve() calls. `objective` holds abi.POS_INF where a
+        root has no solution or the problem is a satisfaction problem; rows of lb / ub without a solution are zero."""
+        n = self.problem.nvars
+        lb = np.ascontiguousarray(lb, dtype=np.int32).reshape(-1, n)
+        ub = np.ascontiguousarray(ub, dtype=np.int32).reshape(-1, n)
+        if lb.shape != ub.shape:
+            raise ValueError("lb and ub must have the same shape [K, nvars]")
+        k = lb.shape[0]
+        olb = np.zeros((k, max(1, n)), np.int32)
+        oub = np.zeros((k, max(1, n)), np.int32)
+        has = np.zeros(max(1, k), np.int32)
+        exh = np.zeros(max(1, k), np.int32)
+        obj = np.zeros(max(1, k), np.int32)
+        st = abi.TbStats()
+        _check(lib().tb_solve_batch(self._h, k, _p(lb), _p(ub), stop_flag, _p(olb), _p(oub), _p(has), _p(exh), _p(obj),
+                                    C.byref(st)))
+        return dict(lb=olb[:, :n], ub=oub[:, :n], has_solution=has[:k].astype(bool), exhaustive=exh[:k].astype(bool),
+                    objective=obj[:k].astype(np.int64), stats=st.as_dict())
 
     def export_bound_handle(self):
         buf = C.create_string_buffer(64)
