@@ -93,11 +93,6 @@ __device__ __forceinline__ void bulk_wait_all() {
 // ITS propagator word of visit k in columns 2k, 2k+1 of its own TMEM lane. tcgen05.st fills them once per launch,
 // one tcgen05.ld per visit reads them back with a latency of a dozen cycles instead of an L2 round trip, and the
 // table stream leaves the L2 -> SM path altogether.
-#ifdef TB_NO_TMEM
-#define TB_TMEM_CODE 0
-#else
-#define TB_TMEM_CODE 1
-#endif
 __device__ __forceinline__ void tmem_alloc(unsigned* smem_dst, unsigned ncols) {
   asm volatile("tcgen05.alloc.cta_group::1.sync.aligned.shared::cta.b32 [%0], %1;" ::"r"(smem_u32(smem_dst)), "r"(ncols) : "memory");
   asm volatile("tcgen05.relinquish_alloc_permit.cta_group::1.sync.aligned;" ::: "memory");
@@ -294,6 +289,16 @@ __device__ __forceinline__ void decode_word(unsigned long long w, int& a, int& b
   if (!tbd::cls_loads_z(CLS)) c = (c << (32 - TBC_FIELD_BITS)) >> (32 - TBC_FIELD_BITS);
 }
 
+// The class that owns chunk `ch`: the table is sorted by class, so it is the largest cls with cls_begin[cls] <= ch
+// (empty classes are skipped by the <=).
+__device__ __forceinline__ int chunk_class(const DevParams& P, int ch) {
+  int cls = 0;
+#pragma unroll
+  for (int step = 16; step > 0; step >>= 1)
+    if (cls + step < TBC_NUM && ch >= P.cls_begin[cls + step]) cls += step;
+  return cls;
+}
+
 // Per-CTA state of the BATCH kernels only (a function-scope __shared__ object: the other kernels never reference it).
 struct BatchCtl { int won; };
 __device__ __forceinline__ BatchCtl& batch_ctl() { __shared__ BatchCtl b; return b; }
@@ -312,7 +317,7 @@ struct Ctx {
   unsigned mbar_phase;
   unsigned tm_warp;        // tensor-memory address of this warp's table words (tm_visits of them; 0 = none)
   int tm_visits;
-  unsigned fp_rot;         // rotation of the three fixpoint flag words, kept across calls (fixpoint3)
+  unsigned fp_rot;         // rotation of the three fixpoint flag words, kept across calls (dense fixpoint)
   int sel_par;             // which selection cell the next split() uses
   unsigned narrowed;       // per-thread count of published bounds
   unsigned long long deductions;     // per-warp (lane-uniform) count of propagator evaluations
@@ -559,42 +564,20 @@ struct Ctx {
   }
 
   // ---- fixpoint (BlockAsynchronousFixpointGPU::fixpoint + warp_fixpoint, barebones :925-965) ---
-  // The part of one sweep that falls in class CLS. A warp walks the whole table ch = warp, warp + nwarps, ...
-  // (so the classes load-balance together and the next chunk's words are always prefetched, across class
-  // boundaries too); the table is sorted by class, so the walk is a chain of per-class loops in each of which
-  // the operator is a compile-time constant. A chunk is 32 propagators of one class. With WAC1
-  // (`warp_fixpoint`, :951-962) the warp iterates the chunk to a warp-local fixpoint before moving on.
-  // `changed` / `failed` are warp-uniform; `notent` is per lane: the fused `ask` (:972-982) evaluated on the
-  // last snapshot, which in the sweep where nothing changed is the final store.
-  // One lane's TBC_U words of a chunk (adjacent in the table: one vector load).
-  struct Words { unsigned long long w[TBC_U]; };
-
   // What the sweeps touch, copied out of the context into registers for the duration of one fixpoint: the
   // context itself lives in local memory whenever a kernel calls the fixpoint from more than one place, and the
   // volatile accesses of the loop would otherwise re-read its fields from there at every evaluation.
   // (TMALL: the words in tensor memory carry absolute shared addresses, see StoreAbs)
-#ifdef TB_FIXPOINT_V2
-  static constexpr bool kAbs = false;       // (round 1's loop works on slots)
-#else
-  static constexpr bool kAbs = !ACT && TBC_U == 1 && ((TB_TMEM_CODE && TMALL && MEM == TB_MEM_STORE_SHARED) || MEM == TB_MEM_TCN_SHARED);
-#endif
+  static constexpr bool kAbs = !ACT && TBC_U == 1 && ((TMALL && MEM == TB_MEM_STORE_SHARED) || MEM == TB_MEM_TCN_SHARED);
   struct HotSlots { StoreRef<MEM> store; const unsigned long long* words; unsigned narrowed; unsigned tm; int tm_visits; };
   struct HotAbs { StoreAbs store; const unsigned long long* words; unsigned narrowed; unsigned tm; int tm_visits; };
   struct Hot : std::conditional<kAbs, HotAbs, HotSlots>::type {};
 
-  struct Walk {
-    int ch;                 // current chunk of this warp
-    int widx;               // index of this lane's first word in the chunk the warp visits after the next one
-    Words cur, nxt;         // this lane's words of the current chunk and of the next one (in flight)
-    unsigned evals;         // warp evaluations (x 32 TBC_U propagators) of this sweep
-    unsigned pad_evals;     // propagator evaluations spent on padding lanes
-    int late_chg;           // a chunk visit ended on a change (AC1: some visit changed something)
-    int failed;             // warp-uniform
-    int notent;             // per lane: non-zero iff some propagator of this lane is not entailed
-  };
+  // One lane's TBC_U words of a chunk (adjacent in the table: one vector load).
+  struct Words { unsigned long long w[TBC_U]; };
 
-  // A chunk's words are requested at the end of the visit before the previous one. The global table is followed
-  // by 2 * nwarps + 1 chunks of padding (tb_create), so the prefetch needs no bound check; the shared copy (TCN_SHARED) is not, and clamps.
+  // A warp requests the words of its next chunk before it knows whether the sweep goes on: the global table is followed
+  // by padding chunks (tb_create), so the request needs no bound check; the shared copy (TCN_SHARED) is not, and clamps.
   __device__ __forceinline__ Words load_words(const unsigned long long* words, int i) const {
     Words r;
     if (MEM == TB_MEM_TCN_SHARED) i = min(i, (P.nchunks * 32 - 1) * TBC_U);
@@ -611,131 +594,29 @@ struct Ctx {
   // Orders this thread's published bounds before its re-reads (see tbd::emptied).
   // (Promptness, not correctness: a re-read that misses the thread's own update finds "work" again and republishes the
   // same bounds; an empty interval is found by the next evaluation that loads it; the sweep barrier publishes everything.
-  // TB_NO_PUBLISH_FENCE drops it - with a cluster the fence is MEMBAR + ERRBAR + CCTL.IVALL, 12 % of the stall samples.)
+  // With a cluster the fence is MEMBAR + ERRBAR + CCTL.IVALL, 12 % of the stall samples; dropping it gained 0.5 %.)
   __device__ __forceinline__ void publish_fence() const {
-#ifndef TB_NO_PUBLISH_FENCE
     if (MEM == TB_MEM_STORE_CLUSTER) asm volatile("fence.sc.cluster;" ::: "memory");
     else asm volatile("fence.sc.cta;" ::: "memory");
-#endif
   }
 
-  // The part of one sweep that falls in class CLS. A warp walks the whole table ch = warp, warp + nwarps, ...
-  // (so the classes load-balance together and the next chunk's words are always prefetched, across class
-  // boundaries too); the table is sorted by class, so the walk is a chain of per-class loops in each of which
-  // the operator is a compile-time constant. A chunk is 32 * TBC_U propagators of one class. With WAC1
-  // (`warp_fixpoint`, :951-962) the warp iterates the chunk to a warp-local fixpoint before moving on.
-  // Every branch below is warp-uniform (votes), so the hot path carries no reconvergence bookkeeping.
-  template <int CLS>
-  __device__ __forceinline__ void sweep_class(Hot& h, Walk& w, const bool wac1, const int nwarps) {
-    const StoreRef<MEM>& store = h.store;
-    unsigned& narrowed = h.narrowed;
-    const int ce = P.cls_begin[CLS + 1];
-    unsigned e0 = w.evals;
-    bool dead = false;
-    do {
-      int fa[TBC_U], fb[TBC_U], fc[TBC_U];
-#pragma unroll
-      for (int u = 0; u < TBC_U; ++u) decode_word<CLS>(w.cur.w[u], fa[u], fb[u], fc[u]);
-      tbd::Snap s[TBC_U];
-      e0 = w.evals;
-      for (;;) {
-        bool chg = false;
-#pragma unroll
-        for (int u = 0; u < TBC_U; ++u) tbd::load_snap<CLS>(store, fa[u], fb[u], fc[u], s[u]);
-#pragma unroll
-        for (int u = 0; u < TBC_U; ++u) chg |= tbd::has_work<CLS>(s[u]);
-        ++w.evals;
-        if (!__any_sync(0xffffffffu, chg)) break;          // the chunk is at its warp-local fixpoint
-        // somebody has work: compute the new bounds, publish the ones that moved (per bound, predicated),
-        // then re-read and look for empty intervals
-#pragma unroll
-        for (int u = 0; u < TBC_U; ++u) {
-          tbd::Snap n;
-          tbd::narrow<CLS>(s[u], n);
-          tbd::publish<CLS>(store, fa[u], fb[u], fc[u], s[u], n, narrowed);
-        }
-        bool fail = false;
-#pragma unroll
-        for (int u = 0; u < TBC_U; ++u) fail |= tbd::emptied<CLS>(store, fa[u], fb[u], fc[u]);
-        dead = __any_sync(0xffffffffu, fail);
-        if (dead | !wac1) { w.late_chg = 1; break; }
-      }
-#pragma unroll
-      for (int u = 0; u < TBC_U; ++u) w.notent |= tbd::not_entailed_bits<CLS>(s[u]);
-      w.ch += nwarps;
-      // Rotate the prefetch queue: `nxt` was requested a whole visit ago, and the new request lands directly in
-      // `nxt` (a register copy of data still in flight would wait for the whole L2 round trip). The guard is
-      // always true; it ties the copy to a value produced at the end of the visit, otherwise the scheduler
-      // moves the copy to the top of the visit, right behind the request it depends on.
-      if (w.evals != 0u) w.cur = w.nxt;
-      w.nxt = load_words(h.words, w.widx);
-      w.widx += nwarps * 32 * TBC_U;
-    } while (w.ch < ce && !dead);
-    if (dead) w.failed = 1;
-    // the class's last chunk is padded with copies of its last propagator: do not count those lanes
-    if (w.ch - nwarps == ce - 1) w.pad_evals += (w.evals - e0) * (unsigned)(32 * TBC_U - P.cls_last[CLS]);
-  }
-
-  // Returns the OR of the flag bits of the last sweep; `iters` = number of block sweeps.
-  __device__ __forceinline__ int fixpoint(int& iters) {
-    // (broadcast from lane 0: tells the compiler the warp index is warp-uniform, so the walk's loop control
-    // lives in uniform registers and its branches need no reconvergence bookkeeping)
-    const int lane = tid & 31, warp = __shfl_sync(0xffffffffu, tid >> 5, 0), nwarps = T >> 5;
-    const bool wac1 = P.fixpoint_kind == TB_FP_WAC1 && P.nprops > P.wac1_threshold;
-    Hot h;
-    h.store = store; h.words = words; h.narrowed = narrowed;
-    unsigned long long ded = 0;
-    int it = 0, f;
-    for (;; ++it) {
-      Walk w;
-      w.ch = warp; w.evals = w.pad_evals = 0; w.late_chg = 0; w.failed = 0; w.notent = 0;
-      w.widx = (warp * 32 + lane) * TBC_U;
-      w.cur = load_words(h.words, w.widx);
-      w.widx += nwarps * 32 * TBC_U;
-      w.nxt = load_words(h.words, w.widx);
-      w.widx += nwarps * 32 * TBC_U;
-#define TB_SWEEP(CLS) if (w.ch < P.cls_begin[CLS + 1] && !w.failed) sweep_class<CLS>(h, w, wac1, nwarps);
-      TB_SWEEP(TBC_ADD_S) TB_SWEEP(TBC_ADD_XK) TB_SWEEP(TBC_ADD_ZK) TB_SWEEP(TBC_ADD_G)
-      TB_SWEEP(TBC_MUL) TB_SWEEP(TBC_TDIV) TB_SWEEP(TBC_TMOD) TB_SWEEP(TBC_MIN) TB_SWEEP(TBC_MAX)
-      TB_SWEEP(TBC_EQ_S) TB_SWEEP(TBC_EQ_T) TB_SWEEP(TBC_EQ_F) TB_SWEEP(TBC_EQ_ZK) TB_SWEEP(TBC_EQ_G)
-      TB_SWEEP(TBC_LEQ_S) TB_SWEEP(TBC_LEQ_T) TB_SWEEP(TBC_LEQ_F) TB_SWEEP(TBC_LEQ_ZK) TB_SWEEP(TBC_LEQ_G)
-#undef TB_SWEEP
-      ded += (unsigned long long)w.evals * (unsigned long long)(32 * TBC_U) - (unsigned long long)w.pad_evals;
-      // a visit changed something iff it took more than one evaluation (WAC1) or ended on a change
-      const unsigned visits = (unsigned)(w.ch - warp) / (unsigned)nwarps;
-      const bool changed = w.evals > visits || w.late_chg;
-      int bits = (changed ? F_CHANGED : 0) | (w.failed ? F_FAILED : 0) | (w.notent ? F_NOT_ENTAILED : 0);
-      bits = __reduce_or_sync(0xffffffffu, bits);
-      const int slot = it % 3;
-      if (lane == 0 && bits) atomicOr(&c.flags[slot], bits);
-      if (tid == 0) c.flags[(it + 1) % 3] = 0;
-      sync();
-      f = c.flags[slot];
-      if (!(f & F_CHANGED) || (f & F_FAILED)) break;
-    }
-    iters = it + 1;
-    narrowed = h.narrowed;
-    deductions += ded;
-    // leave slot 0 clean for the next call (nobody reads flags until the next fixpoint's barrier)
-    sync();
-    if (tid < 3) c.flags[tid] = 0;
-    sync();
-    return f;
-  }
-
-  // ---- the dense fixpoint, third generation (default; -DTB_FIXPOINT_V2 keeps the loop above) -------------------
-  // Same sweeps, same warp-local WAC1 iteration, same flags; what changed is what a visit that finds nothing to do
-  // (nine out of ten) has to execute:
+  // ---- the dense fixpoint -----------------------------------------------------------------------------------------
+  // A sweep: a warp walks the whole table ch = warp, warp + nwarps, ... (so the classes load-balance together and the
+  // next chunk's words are always requested ahead, across class boundaries too); the table is sorted by class, so the
+  // walk is a chain of per-class loops in each of which the operator is a compile-time constant. A chunk is 32 * TBC_U
+  // propagators of one class, TBC_U per lane. With WAC1 (`warp_fixpoint`, :951-962) the warp iterates the chunk to a
+  // warp-local fixpoint before moving on. Every branch is warp-uniform (votes), so the hot path carries no reconvergence bookkeeping.
+  // Nine visits out of ten find nothing to do, and the loop is shaped for them:
   //   * the work path is one cold block: after publishing, ONE re-read of the operands is both the emptiness check
   //     (failure detection, tbd::emptied) and the snapshot of the next warp-local iteration; failure leaves the
   //     sweep from there, so the hot loop carries no `dead` / `late change` flags;
   //   * evaluations are counted as visits (derived from the walk) + re-evaluations (counted in the work path);
-  //   * the fused `ask` stops at the first non-entailed propagator the warp sees in a sweep: the node then cannot
-  //     be a solution, whatever the other chunks say (all-entailed sweeps still check every chunk);
+  //   * the `ask` (:972-982) is fused into the sweeps, evaluated on the last snapshot, which in the sweep where nothing
+  //     changed is the final store; it stops at the first non-entailed propagator the warp sees in a sweep: the node then
+  //     cannot be a solution, whatever the other chunks say (all-entailed sweeps still check every chunk);
   //   * every flag the warp reports is warp-uniform: no REDUX before the atomicOr;
-  //   * the three flag words keep rotating across calls, so a fixpoint ends on its last sweep's barrier (the loop
-  //     above spends two more barriers per call on clearing them).
-  struct Walk3 {
+  //   * the three flag words keep rotating across calls, so a fixpoint ends on its last sweep's barrier.
+  struct Walk {
     int ch;                       // current chunk of this warp (uniform)
     int widx;                     // index of this lane's first word of the chunk the warp visits next
     Words cur;                    // this lane's words of the current chunk (requested at the end of the previous visit)
@@ -746,18 +627,18 @@ struct Ctx {
     unsigned ta;                  // tensor-memory address of the next request's words (two columns per visit)
   };
 
-  // The words of the chunk a warp visits `tk` visits into its sweep: from tensor memory when they are there.
-  __device__ __forceinline__ Words next_words(const Hot& h, Walk3& w) const {
+  // The words of the chunk the warp visits next: from tensor memory when they are there.
+  __device__ __forceinline__ Words next_words(const Hot& h, Walk& w) const {
     Words r;
-    if (TB_TMEM_CODE && TBC_U == 1 && MEM == TB_MEM_STORE_SHARED && (TMALL || w.ta < h.tm + 2u * (unsigned)h.tm_visits)) r.w[0] = tmem_ld64(w.ta);
+    if (TBC_U == 1 && MEM == TB_MEM_STORE_SHARED && (TMALL || w.ta < h.tm + 2u * (unsigned)h.tm_visits)) r.w[0] = tmem_ld64(w.ta);
     else r = load_words(h.words, w.widx);
     w.ta += 2u;
     return r;
   }
 
-  // Returns true when the store failed (the sweep is over for this warp).
+  // The part of one sweep that falls in class CLS. Returns true when the store failed (the sweep is over for this warp).
   template <int CLS>
-  __device__ __forceinline__ bool sweep_class3(Hot& h, Walk3& w, const bool wac1, const int nwarps, const int stride) {
+  __device__ __forceinline__ bool sweep_class(Hot& h, Walk& w, const bool wac1, const int nwarps, const int stride) {
     const auto& store = h.store;
     const int ce = P.cls_begin[CLS + 1];
     unsigned last_extra = 0;      // re-evaluations of the latest visit that had work, and which chunk that was
@@ -814,7 +695,10 @@ struct Ctx {
     return false;
   }
 
-  __device__ __forceinline__ int fixpoint3(int& iters) {
+  // Returns the OR of the flag bits of the last sweep; `iters` = number of block sweeps.
+  __device__ __forceinline__ int fixpoint(int& iters) {
+    // (broadcast from lane 0: tells the compiler the warp index is warp-uniform, so the walk's loop control
+    // lives in uniform registers and its branches need no reconvergence bookkeeping)
     const int lane = tid & 31, warp = __shfl_sync(0xffffffffu, tid >> 5, 0), nwarps = T >> 5;
     const int stride = nwarps * 32 * TBC_U;
     const bool wac1 = P.fixpoint_kind == TB_FP_WAC1 && P.nprops > P.wac1_threshold;
@@ -827,14 +711,14 @@ struct Ctx {
     unsigned rot = fp_rot;
     int it = 0, f;
     for (;; ++it) {
-      Walk3 w;
+      Walk w;
       w.ch = warp; w.extra = w.pad_evals = 0; w.changed = 0; w.notent = 0;
       w.widx = (warp * 32 + lane) * TBC_U;
       w.ta = h.tm;
       w.cur = next_words(h, w);
       w.widx += stride;
       bool failed = false;
-#define TB_SWEEP(CLS) if (!failed && w.ch < P.cls_begin[CLS + 1]) failed = sweep_class3<CLS>(h, w, wac1, nwarps, stride);
+#define TB_SWEEP(CLS) if (!failed && w.ch < P.cls_begin[CLS + 1]) failed = sweep_class<CLS>(h, w, wac1, nwarps, stride);
       TB_SWEEP(TBC_ADD_S) TB_SWEEP(TBC_ADD_XK) TB_SWEEP(TBC_ADD_ZK) TB_SWEEP(TBC_ADD_G)
       TB_SWEEP(TBC_MUL) TB_SWEEP(TBC_TDIV) TB_SWEEP(TBC_TMOD) TB_SWEEP(TBC_MIN) TB_SWEEP(TBC_MAX)
       TB_SWEEP(TBC_EQ_S) TB_SWEEP(TBC_EQ_T) TB_SWEEP(TBC_EQ_F) TB_SWEEP(TBC_EQ_ZK) TB_SWEEP(TBC_EQ_G)
@@ -860,8 +744,8 @@ struct Ctx {
   }
 
   // ---- active-set fixpoint (TB_FP_*_ACTIVE; SURVEY 8f.2, the idea of FixpointSubsetGPU, barebones :636,984) ------
-  // Same sweeps, same warp-local WAC1 iteration, same flags as fixpoint(), but a warp only evaluates the chunks one
-  // of whose variables moved since the chunk was last evaluated.  State in dynamic shared memory (P.act_off):
+  // The same warp-local WAC1 iteration and the same flag bits as the dense fixpoint, but a warp only evaluates the chunks
+  // one of whose variables moved since the chunk was last evaluated.  State in dynamic shared memory (P.act_off):
   //   vbits  : one bit per slot, set (red.or) by whoever moves a bound of the slot;
   //   dirty  : one byte per chunk, grouped per owning warp (chunk ch = flag ch / nwarps of warp ch % nwarps), set in
   //            the marking phase between two sweeps from vbits and the slot -> chunks watch lists (global, L2), cleared
@@ -877,27 +761,27 @@ struct Ctx {
     if (ACT) atomicOr(act_vbits() + (slot >> 5), 1u << (slot & 31));
   }
 
-  // The chunks that load `slot` are due (direct marking: the publisher does it itself, into the flags of the NEXT sweep).
-  __device__ __forceinline__ void mark_watchers(int slot, unsigned char* dnext, int nwarps, int lw, int FPW) const {
+  // The chunks that load `slot` are due: set their flags in `dirty` (chunk ch is flag ch >> lw of warp ch & (nwarps - 1)).
+  // One 64-bit word names a slot's first three watchers, the few slots with more continue through the CSR list.
+  __device__ __forceinline__ void mark_watchers(int slot, unsigned char* dirty, int nwarps, int lw, int FPW) const {
     const unsigned long long wd = __ldg(P.watch_inline + slot);
 #pragma unroll
     for (int k = 0; k < 3; ++k) {
       const unsigned id = (unsigned)(wd >> (16 * k)) & 0xFFFFu;
-      if (id != 0xFFFFu) dnext[(id & (unsigned)(nwarps - 1)) * FPW + (id >> lw)] = 1;
+      if (id != 0xFFFFu) dirty[(id & (unsigned)(nwarps - 1)) * FPW + (id >> lw)] = 1;
     }
     if ((unsigned)(wd >> 48) == 0xFFFEu) {
       const int e = __ldg(P.watch_off + slot + 1);
       for (int k = __ldg(P.watch_off + slot) + 3; k < e; ++k) {
         const int ch = __ldg(P.watch_list + k);
-        dnext[(ch & (nwarps - 1)) * FPW + (ch >> lw)] = 1;
+        dirty[(ch & (nwarps - 1)) * FPW + (ch >> lw)] = 1;
       }
     }
   }
 
   template <int CLS>
   __device__ __forceinline__ void active_visit(Hot& h, const Words& cur, const bool wac1, const int ch, unsigned* vbits,
-                                               unsigned char* ne_slot, unsigned& evals, unsigned& pad_evals, int& late_chg, int& failed,
-                                               unsigned char* dnext = nullptr, int nwarps = 0, int lw = 0, int FPW = 0) {
+                                               unsigned char* ne_slot, unsigned& evals, unsigned& pad_evals, int& late_chg, int& failed) {
     const StoreRef<MEM>& store = h.store;
     int fa[TBC_U], fb[TBC_U], fc[TBC_U];
 #pragma unroll
@@ -918,15 +802,9 @@ struct Ctx {
         tbd::Snap n;
         tbd::narrow<CLS>(s[u], n);
         tbd::publish<CLS>(store, fa[u], fb[u], fc[u], s[u], n, h.narrowed);
-        if (dnext) {
-          if (tbd::cls_loads_x(CLS) && ((n.xl != s[u].xl) | (n.xu != s[u].xu))) mark_watchers(fa[u], dnext, nwarps, lw, FPW);
-          if ((n.yl != s[u].yl) | (n.yu != s[u].yu)) mark_watchers(fb[u], dnext, nwarps, lw, FPW);
-          if (tbd::cls_loads_z(CLS) && ((n.zl != s[u].zl) | (n.zu != s[u].zu))) mark_watchers(fc[u], dnext, nwarps, lw, FPW);
-        } else {
-          if (tbd::cls_loads_x(CLS) && ((n.xl != s[u].xl) | (n.xu != s[u].xu))) atomicOr(vbits + (fa[u] >> 5), 1u << (fa[u] & 31));
-          if ((n.yl != s[u].yl) | (n.yu != s[u].yu)) atomicOr(vbits + (fb[u] >> 5), 1u << (fb[u] & 31));
-          if (tbd::cls_loads_z(CLS) && ((n.zl != s[u].zl) | (n.zu != s[u].zu))) atomicOr(vbits + (fc[u] >> 5), 1u << (fc[u] & 31));
-        }
+        if (tbd::cls_loads_x(CLS) && ((n.xl != s[u].xl) | (n.xu != s[u].xu))) atomicOr(vbits + (fa[u] >> 5), 1u << (fa[u] & 31));
+        if ((n.yl != s[u].yl) | (n.yu != s[u].yu)) atomicOr(vbits + (fb[u] >> 5), 1u << (fb[u] & 31));
+        if (tbd::cls_loads_z(CLS) && ((n.zl != s[u].zl) | (n.zu != s[u].zu))) atomicOr(vbits + (fc[u] >> 5), 1u << (fc[u] & 31));
       }
       bool fail = false;
 #pragma unroll
@@ -952,18 +830,6 @@ struct Ctx {
     unsigned char* dirty = (unsigned char*)(vbits + nvw);
     unsigned char* mydirty = dirty + warp * FPW;
     unsigned char* mynotent = dirty + nwarps * FPW + warp * FPW;
-    // TB_ACTIVE_DIRECT: whoever publishes a bound marks its watchers itself, into a SECOND set of dirty flags that the
-    // next sweep reads: one barrier per sweep instead of two (the marking phase only runs once, at the start of the call,
-    // for what moved outside the fixpoint: the decision, the incumbent, a restored store), and the flag words rotate
-    // across calls as in fixpoint3.
-#ifdef TB_ACTIVE_DIRECT
-    constexpr bool DIRECT = true;
-#else
-    constexpr bool DIRECT = false;
-#endif
-    unsigned char* dirty1 = dirty + 2 * nwarps * FPW;
-    int par = 0;
-    unsigned rot = fp_rot;
     Hot h;
     h.store = store; h.words = words; h.narrowed = narrowed;
     h.tm = __shfl_sync(0xffffffffu, tm_warp, 0); h.tm_visits = tm_visits;
@@ -971,16 +837,12 @@ struct Ctx {
     int it = 0, f;
     for (;; ++it) {
       // ---- marking phase: moved slots -> dirty chunks
-      if (DIRECT && it == 0) for (int i = tid; i < nwarps * FPW / 4; i += T) ((unsigned*)dirty1)[i] = 0u;
-      if (DIRECT && it > 0) {
-        // (the publishers of the previous sweep have marked this sweep's chunks already)
-      } else if (c.dirty_all) {
+      if (c.dirty_all) {
         for (int i = tid; i < nwarps * FPW; i += T) { const int w = i / FPW, k = i - w * FPW; dirty[i] = (k * nwarps + w) < P.nchunks ? 1 : 0; }
         for (int i = tid; i < nvw; i += T) vbits[i] = 0;
       } else {
         // every thread follows the watchers of the moved slots of its own words (moved slots are spread thinly over the
-        // words, so the lanes of a warp work on different slots at the same time: one L2 round trip per round of bits);
-        // one 64-bit word names a slot's first three watchers, the few slots with more continue through the CSR list
+        // words, so the lanes of a warp work on different slots at the same time: one L2 round trip per round of bits)
         for (int i = tid; i < nvw; i += T) {
           unsigned m = vbits[i];
           if (m) {
@@ -988,36 +850,22 @@ struct Ctx {
             do {
               const int v = (i << 5) + __ffs((int)m) - 1;
               m &= m - 1;
-              const unsigned long long wd = __ldg(P.watch_inline + v);
-#pragma unroll
-              for (int k = 0; k < 3; ++k) {
-                const unsigned id = (unsigned)(wd >> (16 * k)) & 0xFFFFu;
-                if (id != 0xFFFFu) dirty[(id & (unsigned)(nwarps - 1)) * FPW + (id >> lw)] = 1;
-              }
-              if ((unsigned)(wd >> 48) == 0xFFFEu) {
-                const int e = __ldg(P.watch_off + v + 1);
-                for (int k = __ldg(P.watch_off + v) + 3; k < e; ++k) {
-                  const int ch = __ldg(P.watch_list + k);
-                  dirty[(ch & (nwarps - 1)) * FPW + (ch >> lw)] = 1;
-                }
-              }
+              mark_watchers(v, dirty, nwarps, lw, FPW);
             } while (m);
           }
         }
       }
-      if (!DIRECT || it == 0) sync();
+      sync();
       if (tid == 0) {
         c.dirty_all = 0;
-        if (DIRECT) c.flags[(rot + 1u) % 3u] = 0; else c.flags[(it + 1) % 3] = 0;
+        c.flags[(it + 1) % 3] = 0;
       }
       // ---- sweep: this warp's dirty chunks
       unsigned evals = 0, pad_evals = 0, visits = 0;
       int late_chg = 0, failed = 0;
-      unsigned char* const dcur = (DIRECT && par ? dirty1 : dirty) + warp * FPW;
-      unsigned char* const dnext = DIRECT ? (par ? dirty : dirty1) : nullptr;
       for (int g = 0; g < FPW && !failed; g += 32) {
-        unsigned mask = __ballot_sync(0xffffffffu, dcur[g + lane] != 0);
-        if (mask) dcur[g + lane] = 0;
+        unsigned mask = __ballot_sync(0xffffffffu, mydirty[g + lane] != 0);
+        if (mask) mydirty[g + lane] = 0;
         while (mask && !failed) {
           const int k = g + __ffs((int)mask) - 1;
           mask &= mask - 1;
@@ -1025,14 +873,10 @@ struct Ctx {
           Words cur;
           // (the k-th chunk of this warp: its words are in tensor memory when the table fits, a dozen cycles away
           // instead of an L2 round trip on the critical path of a sweep that visits one or two chunks)
-          if (TB_TMEM_CODE && TBC_U == 1 && MEM == TB_MEM_STORE_SHARED && k < h.tm_visits) cur.w[0] = tmem_ld64(h.tm + 2u * (unsigned)k);
+          if (TBC_U == 1 && MEM == TB_MEM_STORE_SHARED && k < h.tm_visits) cur.w[0] = tmem_ld64(h.tm + 2u * (unsigned)k);
           else cur = load_words(h.words, (ch * 32 + lane) * TBC_U);
-          int cls = 0;                                          // warp-uniform; the table is sorted by class:
-#pragma unroll
-          for (int step = 16; step > 0; step >>= 1)            // largest cls with cls_begin[cls] <= ch (empty classes skipped by <=)
-            if (cls + step < TBC_NUM && ch >= P.cls_begin[cls + step]) cls += step;
-          switch (cls) {
-#define TB_CASE(CLS) case CLS: active_visit<CLS>(h, cur, wac1, ch, vbits, mynotent + k, evals, pad_evals, late_chg, failed, dnext, nwarps, lw, FPW); break;
+          switch (chunk_class(P, ch)) {                         // warp-uniform
+#define TB_CASE(CLS) case CLS: active_visit<CLS>(h, cur, wac1, ch, vbits, mynotent + k, evals, pad_evals, late_chg, failed); break;
             TB_CASE(TBC_ADD_S) TB_CASE(TBC_ADD_XK) TB_CASE(TBC_ADD_ZK) TB_CASE(TBC_ADD_G)
             TB_CASE(TBC_MUL) TB_CASE(TBC_TDIV) TB_CASE(TBC_TMOD) TB_CASE(TBC_MIN) TB_CASE(TBC_MAX)
             TB_CASE(TBC_EQ_S) TB_CASE(TBC_EQ_T) TB_CASE(TBC_EQ_F) TB_CASE(TBC_EQ_ZK) TB_CASE(TBC_EQ_G)
@@ -1050,29 +894,20 @@ struct Ctx {
       const bool changed = evals > visits || late_chg;
       int bits = (changed ? F_CHANGED : 0) | (failed ? F_FAILED : 0) | (ne ? F_NOT_ENTAILED : 0);
       bits = __reduce_or_sync(0xffffffffu, bits);
-      const int slot = DIRECT ? (int)(rot % 3u) : it % 3;
+      const int slot = it % 3;
       if (lane == 0 && bits) atomicOr(&c.flags[slot], bits);
       sync();
       f = c.flags[slot];
-      ++rot; par ^= 1;
       if (!(f & F_CHANGED) || (f & F_FAILED)) break;
     }
     iters = it + 1;
     narrowed = h.narrowed;
     deductions += ded;
-    if (DIRECT) { fp_rot = rot; return f; }
+    // leave slot 0 clean for the next call (nobody reads flags until the next fixpoint's barrier)
     sync();
     if (tid < 3) c.flags[tid] = 0;
     sync();
     return f;
-  }
-
-  __device__ __forceinline__ int dense_fixpoint(int& iters) {
-#if defined(TB_FIXPOINT_V2)
-    return fixpoint(iters);
-#else
-    return fixpoint3(iters);
-#endif
   }
 
   // ---- intermediate solutions (-i / -a) --------------------------------------------------------------------------
@@ -1149,7 +984,7 @@ struct Ctx {
     if (P.obj_var >= 0) { int l, u; store.ld(P.obj_var, l, u); pre_failed |= l > u; }
     if (pre_failed) f = F_FAILED;
     else if constexpr (ACT) f = fixpoint_active(iters);
-    else f = dense_fixpoint(iters);
+    else f = fixpoint(iters);
     const bool failed = (f & F_FAILED) != 0;
     const bool solution = !failed && !(f & F_NOT_ENTAILED);
     unsigned long long t1 = 0;
@@ -1298,9 +1133,27 @@ struct Ctx {
   }
 
   // ---- EPS dive (barebones :663-741) ------------------------------------------------------------------
+  // One step of the dive below a node that propagate() left open: branch, and take the child that bit
+  // remaining_depth - 1 of `idx` names (decisions are not recorded while diving). A node with nothing left to
+  // branch on is a leaf.
+  __device__ __forceinline__ void dive_step(unsigned long long idx) {
+    if (c.leaf) return;
+    bool pushed = split();
+    if (tid == 0) {
+      if (!pushed) { c.leaf = 1; st->exhaustive = 0; if constexpr (BATCH) batch_cut(); }
+      else {
+        --c.remaining_depth;
+        --c.depth;
+        const Decision& d = dec[0];
+        int bit = (int)((idx >> c.remaining_depth) & 1ull);
+        store.embed(d.var, bit ? d.clb1 : d.clb0, bit ? d.cub1 : d.cub0);
+        mark_var(d.var);
+      }
+    }
+  }
+
   // Dives from the problem root following the bits of `idx`. Returns remaining depth (uniform).
   __device__ __forceinline__ int dive(unsigned long long idx, int depth_power) {
-    
     if (tid == 0) {
       c.cur_strategy = 0; c.next_unassigned = 0; c.depth = 0;
       c.remaining_depth = depth_power; c.leaf = 0; c.failed = 0;
@@ -1311,20 +1164,7 @@ struct Ctx {
     while (c.remaining_depth > 0 && !c.leaf && !c.stop) {
       sync();
       propagate();
-      if (!c.leaf) {
-        bool pushed = split();
-        if (tid == 0) {
-          if (!pushed) { c.leaf = 1; st->exhaustive = 0; if constexpr (BATCH) batch_cut(); }
-          else {
-            --c.remaining_depth;
-            --c.depth;                        // decisions are not recorded while diving
-            const Decision& d = dec[0];
-            int bit = (int)((idx >> c.remaining_depth) & 1ull);
-            store.embed(d.var, bit ? d.clb1 : d.clb0, bit ? d.cub1 : d.cub0);
-            mark_var(d.var);
-          }
-        }
-      }
+      dive_step(idx);
       sync();
     }
     if (tid == 0) st->t_dive += (long long)globaltimer_ns() - c.t_mark;
@@ -1464,20 +1304,7 @@ struct Ctx {
       propagate();
 
       if (mode == M_DIVE) {
-        if (!c.leaf) {
-          bool pushed = split();
-          if (tid == 0) {
-            if (!pushed) { c.leaf = 1; st->exhaustive = 0; if constexpr (BATCH) batch_cut(); }
-            else {
-              --c.remaining_depth;
-              --c.depth;                        // decisions are not recorded while diving
-              const Decision& d = dec[0];
-              int bit = (int)((idx >> c.remaining_depth) & 1ull);
-              store.embed(d.var, bit ? d.clb1 : d.clb0, bit ? d.cub1 : d.cub0);
-            mark_var(d.var);
-            }
-          }
-        }
+        dive_step(idx);
         sync();
       } else {
         // III. branch
@@ -1614,18 +1441,18 @@ __device__ __forceinline__ void ctx_init(Ctx<MEM, ACT, TMALL, BATCH>& k, Ctl* lo
   }
   if (ACT) {
     // vbits, dirty and notent flags start clear; the first fixpoint evaluates everything (dirty_all)
-    const int words_ = (P.vpad >> 5) + ((3 * (int)(blockDim.x >> 5) * P.act_fpw + 3) >> 2);
+    const int words_ = (P.vpad >> 5) + ((2 * (int)(blockDim.x >> 5) * P.act_fpw + 3) >> 2);
     unsigned* a = (unsigned*)(dyn + P.act_off);
     for (int i = threadIdx.x; i < words_; i += blockDim.x) a[i] = 0u;
   }
   k.sync();
   k.tm_warp = 0; k.tm_visits = 0;
-  if (TB_TMEM_CODE && MEM == TB_MEM_STORE_SHARED && TBC_U == 1 && !P.tmem_cols && threadIdx.x < 32) {
+  if (MEM == TB_MEM_STORE_SHARED && TBC_U == 1 && !P.tmem_cols && threadIdx.x < 32) {
     // A CTA of a kernel that carries tensor-memory code holds the SM's allocation permit until it gives it up, and no
     // second CTA starts on the SM meanwhile (measured: TB_TMEM=0 ran one CTA per SM): give it up at once.
     asm volatile("tcgen05.relinquish_alloc_permit.cta_group::1.sync.aligned;" ::: "memory");
   }
-  if (TB_TMEM_CODE && MEM == TB_MEM_STORE_SHARED && TBC_U == 1 && P.tmem_cols) {
+  if (MEM == TB_MEM_STORE_SHARED && TBC_U == 1 && P.tmem_cols) {
     // the table goes to tensor memory: one warp allocates the CTA's columns, every warp stores the words of its own
     // first tmem_visits visits into its quarter of the lanes (chunk ch = warp + k * nwarps at columns 2k, 2k + 1)
     const int warp = (int)(threadIdx.x >> 5), lane = (int)(threadIdx.x & 31), nwarps = (int)(blockDim.x >> 5);
@@ -1640,13 +1467,7 @@ __device__ __forceinline__ void ctx_init(Ctx<MEM, ACT, TMALL, BATCH>& k, Ctl* lo
       const int ch = warp + v * nwarps;
       // (the table is padded behind its end: a chunk index past nchunks reads zeros that are never evaluated)
       unsigned long long wd = __ldg(P.words + (size_t)ch * 32 + lane);
-      if (Ctx<MEM, ACT, TMALL, BATCH>::kAbs && ch < P.nchunks) {
-        int cls = 0;
-#pragma unroll
-        for (int step = 16; step > 0; step >>= 1)
-          if (cls + step < TBC_NUM && ch >= P.cls_begin[cls + step]) cls += step;
-        wd = word_to_abs(wd, cls, smem_u32(dyn));
-      }
+      if (Ctx<MEM, ACT, TMALL, BATCH>::kAbs && ch < P.nchunks) wd = word_to_abs(wd, chunk_class(P, ch), smem_u32(dyn));
       tmem_st64(k.tm_warp + 2u * (unsigned)v, wd);
     }
     asm volatile("tcgen05.wait::st.sync.aligned;" ::: "memory");
@@ -1667,11 +1488,7 @@ __device__ __forceinline__ void ctx_init(Ctx<MEM, ACT, TMALL, BATCH>& k, Ctl* lo
       // the staged copy is this CTA's own: rewrite its slot fields to absolute shared addresses (see StoreAbs)
       unsigned long long* tw = (unsigned long long*)sprops;
       for (int i = threadIdx.x; i < P.nchunks * 32; i += blockDim.x) {
-        const int ch = i >> 5;
-        int cls = 0;
-#pragma unroll
-        for (int step = 16; step > 0; step >>= 1)
-          if (cls + step < TBC_NUM && ch >= P.cls_begin[cls + step]) cls += step;
+        const int cls = chunk_class(P, i >> 5);
         tw[i] = word_to_abs(tw[i], cls, smem_u32(dyn));
       }
       k.sync();
@@ -1690,7 +1507,7 @@ __device__ __forceinline__ void ctx_finish(Ctx<MEM, ACT, TMALL, BATCH>& k) {
   }
   if (threadIdx.x == 0) bulk_wait_all();     // images still on their way to global memory (best store, snapshots)
   k.sync();        // with a cluster: nobody leaves while a peer may still touch its shared memory
-  if (TB_TMEM_CODE && MEM == TB_MEM_STORE_SHARED && TBC_U == 1 && k.P.tmem_cols && threadIdx.x < 32)
+  if (MEM == TB_MEM_STORE_SHARED && TBC_U == 1 && k.P.tmem_cols && threadIdx.x < 32)
     tmem_dealloc(k.lc->tmem_base, (unsigned)k.P.tmem_cols);
 }
 
@@ -1759,7 +1576,7 @@ __global__ void __launch_bounds__(TB_MAX_THREADS) propagate_kernel(const __grid_
       k.sync();
       if (c.leaf) { f = F_FAILED; iters = 0; k.sync(); }
       else if constexpr (ACT) f = k.fixpoint_active(iters);
-      else f = k.dense_fixpoint(iters);
+      else f = k.fixpoint(iters);
       if (tid == 0) {
         k.st->fixpoint_iterations += (unsigned long long)iters;
         k.st->nodes++;
@@ -1982,9 +1799,6 @@ static tb_status dispatch(const tb_solver* s, F&& f) {
   using Active = std::true_type;          // active-set fixpoint: shared-memory placements only
   using Mixed = std::false_type;          // table words from tensor memory where they fit, from L2 beyond
   using AllTm = std::true_type;           // the whole table is in tensor memory (s->tmall)
-#ifdef TB_SASS_PROBE      // (developer builds: one instantiation, to read its SASS quickly)
-  return f(std::integral_constant<int, TB_MEM_STORE_SHARED>{}, Dense{}, AllTm{});
-#else
   switch (s->mem_kind) {
     case TB_MEM_GLOBAL: return f(std::integral_constant<int, TB_MEM_GLOBAL>{}, Dense{}, Mixed{});
     case TB_MEM_STORE_SHARED:
@@ -1997,7 +1811,6 @@ static tb_status dispatch(const tb_solver* s, F&& f) {
   }
   set_error("unsupported memory kind");
   return TB_ERR_UNSUPPORTED;
-#endif
 }
 
 // Launch `workers` workers: one CTA each, or one cluster of s->cluster CTAs each (STORE_CLUSTER).
@@ -2055,7 +1868,7 @@ static tb_status configure(tb_solver* s) {
   const size_t reserved = dp.reservedSharedMemPerBlock + sizeof(Ctl) + 64;
   // the active-set fixpoint keeps one bit per slot and two bytes per chunk next to the store (upper bound here, the
   // exact figure needs the thread count: place_active)
-  const size_t act_b = s->want_active ? (s->store_bytes / 64 + 3 * ((size_t)s->P.nchunks + 1024) + 64) : 0;
+  const size_t act_b = s->want_active ? (s->store_bytes / 64 + 2 * ((size_t)s->P.nchunks + 1024) + 64) : 0;
   const size_t store_b = s->store_bytes + act_b, prop_b = s->prop_bytes;
   auto blocks_for = [&](size_t dyn) -> int {
     if (dyn + sizeof(Ctl) + 64 > max_block_smem) return 0;
@@ -2155,7 +1968,7 @@ static void place_active(tb_solver* s) {
   s->P.act_fpw = std::max(32, (per_warp + 31) / 32 * 32);
   const size_t table = s->mem_kind == TB_MEM_TCN_SHARED ? (size_t)s->P.nchunks * 32 * TBC_U * 8 : 0;
   s->P.act_off = (int)(s->store_bytes + table);
-  const size_t act = (size_t)s->P.vpad / 8 + (size_t)3 * nwarps * s->P.act_fpw;     // moved bits, dirty, cached ask, second dirty set
+  const size_t act = (size_t)s->P.vpad / 8 + (size_t)2 * nwarps * s->P.act_fpw;     // moved bits, dirty, cached ask
   s->shared_bytes = (size_t)s->P.act_off + (act + 15) / 16 * 16;
 }
 
@@ -2204,7 +2017,7 @@ static tb_status set_smem_attr(tb_solver* s) {
       // (measured). The policy above already keeps to 1024 resident threads per SM at 64 registers (__launch_bounds__)
       // and to the shared memory of the SM, and the CTAs split the 512 tensor-memory columns between them (tb_create):
       // for those kernels its own arithmetic stands.
-      if ((TB_TMEM_CODE && m == TB_MEM_STORE_SHARED && TBC_U == 1) || env_int("TB_IGNORE_OCCUPANCY_API", 0)) {
+      if ((m == TB_MEM_STORE_SHARED && TBC_U == 1) || env_int("TB_IGNORE_OCCUPANCY_API", 0)) {
         // (own arithmetic: shared memory was accounted for by configure(); registers and threads here. The grid MUST be
         // co-resident: blocks that find no work wait for the others - tail splitting - and a CTA that cannot start
         // because its SM is full of waiting CTAs would never let them finish.)
@@ -2367,7 +2180,7 @@ extern "C" tb_status tb_create(tb_solver** out, const tb_problem* pb, const tb_o
   // Tensor memory as the table cache (STORE_SHARED, dense kinds): the resident CTAs of an SM share its 512 columns, a
   // CTA's warps share the CTA's columns by quarter (warp index mod 4), a visit takes two columns. TB_TMEM=0: off.
   P.tmem_cols = 0; P.tmem_visits = 0;
-  if (TB_TMEM_CODE && TBC_U == 1 && s->mem_kind == TB_MEM_STORE_SHARED && env_int("TB_TMEM", 1) != 0 && P.nchunks > 0) {
+  if (TBC_U == 1 && s->mem_kind == TB_MEM_STORE_SHARED && env_int("TB_TMEM", 1) != 0 && P.nchunks > 0) {
     int cols = 32;
     while (cols * 2 * s->blocks_per_sm <= 512) cols *= 2;
     const int nwarps = s->threads / 32, per_quarter = (nwarps + 3) / 4;
@@ -2391,9 +2204,9 @@ extern "C" tb_status tb_create(tb_solver** out, const tb_problem* pb, const tb_o
   {
     const TnfLayout& L = s->layout;
     unsigned long long* d = nullptr;
-    // Padding behind the table: a warp requests the words of the chunks two visits ahead (ch + 2 * nwarps) without a bound
-    // check, so 2 * nwarps + 1 chunks past the end are read (never used). nwarps is the warp count of a whole worker:
-    // threads * cluster / 32, up to 512 with a cluster of 16.
+    // Padding behind the table: a warp requests the words of its next chunk (ch + nwarps) before it knows whether the sweep
+    // goes on, without a bound check, so up to nwarps chunks past the end are read (never used); 2 * nwarps + 1 chunks of
+    // padding cover that. nwarps is the warp count of a whole worker: threads * cluster / 32, up to 512 with a cluster of 16.
     const size_t pad_words = (size_t)(2 * (s->threads * std::max(1, s->cluster) / 32) + 1) * 32 * TBC_U;
     if ((rc = dev_alloc(s, &d, L.words.size() + pad_words))) return fail(rc);
     if (cudaMemset(d, 0, (L.words.size() + pad_words) * 8) != cudaSuccess ||

@@ -108,7 +108,7 @@ struct DevParams {
   int rank, world, max_depth, npeers;
   int observe_stop, pad3_;      // 0 for the parity hooks (tb_propagate / tb_dive): the stop cells are neither read nor raised
   unsigned epoch, steal;        // tb_solve call number of this solver (tags the grid cells); stealing from peers enabled
-  int cluster_size, cluster_log2, vc, zero;    // (zero: always 0, opaque to the compiler; see TB_PIN_PREFETCH)  // STORE_CLUSTER: CTAs per cluster, its log2, variables per CTA slice
+  int cluster_size, cluster_log2, vc, pad7_;   // STORE_CLUSTER: CTAs per cluster, its log2, variables per CTA slice
   // per-block scratch in global memory, [slot] major
   int* block_root;              // snapshot of the subproblem root (root_store, barebones :89)
   int* block_best;              // best solution of the block (best_store, :92)
