@@ -183,6 +183,26 @@ tb_status tb_solve_batch(tb_solver*, int32_t nroots, const int32_t* root_lb, con
                          volatile int32_t* stop_flag, int32_t* best_lb, int32_t* best_ub,
                          int32_t* has_solution, int32_t* exhaustive, int32_t* objective, tb_stats* stats);
 
+/* Solves ngroups problems in one launch, each the network over a UNION of boxes: root r (root_lb / root_ub laid out
+ * [nroots][nvars], each a narrowing of the solver's root) is one box of group group_of[r]. A group's answer is what
+ * tb_solve would return if its root store could be that union (a domain with holes, x != v as {x <= v-1} u {x >= v+1},
+ * or one problem split into cubes): has_solution = some box has a solution; for optimisation objective = the minimum
+ * over the boxes and the store a solution of one box at that objective; for satisfaction the first solution found,
+ * which ends every box of its group (the group is then not exhaustive, as in tb_solve); exhaustive = every box of the
+ * group was searched to its end and no block was cut while searching it. The boxes of a group share its incumbent: a
+ * solution found in one prunes all of them from then on. Groups never affect each other. Boxes may overlap (only the
+ * union counts). A box with an empty referenced domain is decided on the host (no solution, searched) and does not end
+ * its group. Outputs per group: best_lb / best_ub [ngroups][nvars] (may be NULL; rows of groups without a solution are
+ * left as they are), has_solution / exhaustive / objective [ngroups] (objective = TB_POS_INF when there is no solution
+ * or the problem is a satisfaction problem); stats = the whole launch. Subproblems per root, stop_flag and the timeout
+ * apply as in tb_solve_batch (nroots roots). TB_ERR_INVALID: nroots < 1, ngroups < 1, a group_of[r] outside
+ * [0, ngroups), a group without a root, a root that widens the solver's root. TB_ERR_UNSUPPORTED: as tb_solve_batch.
+ * tb_solve_batch is tb_solve_groups with group_of[r] = r. */
+tb_status tb_solve_groups(tb_solver*, int32_t nroots, const int32_t* root_lb, const int32_t* root_ub,
+                          const int32_t* group_of, int32_t ngroups, volatile int32_t* stop_flag,
+                          int32_t* best_lb, int32_t* best_ub, int32_t* has_solution, int32_t* exhaustive,
+                          int32_t* objective, tb_stats* stats);
+
 /* Intermediate solutions (-i / -a; the reference's consumer thread, gpu_dive_and_solve.hpp:100-132; its barebones
  * architecture cannot, barebones_dive_and_solve.hpp:465-467).  tb_stream_solutions (before tb_solve) makes every
  * improving solution also land in a ring of `slots` store images; tb_poll_solution, called from ANOTHER host thread

@@ -300,13 +300,15 @@ __device__ __forceinline__ int chunk_class(const DevParams& P, int ch) {
 }
 
 // Per-CTA state of the BATCH kernels only (a function-scope __shared__ object: the other kernels never reference it).
-struct BatchCtl { int won; };
+// `group`: the group of the current task's root, set by thread 0 when the task starts.
+struct BatchCtl { int won; int group; };
 __device__ __forceinline__ BatchCtl& batch_ctl() { __shared__ BatchCtl b; return b; }
 
 // TMALL: every visit of every warp finds its propagator word in tensor memory (the table fits): the sweep is compiled
 // without the L2 path and without the test that chooses between the two.
-// BATCH: tb_solve_batch - subproblem g of depth D belongs to root g >> D, which has its own image, incumbent, stop word,
-// best store and closed-weight counter (BatchRoot); every batch-only branch is `if constexpr`.
+// BATCH: tb_solve_groups - subproblem g of depth D belongs to root g >> D, which has its own image and closed-weight
+// counter (BatchRoot); its group has the incumbent, the stop word and the best store (BatchGroup); every batch-only
+// branch is `if constexpr`.
 template <int MEM, bool ACT = false, bool TMALL = false, bool BATCH = false>
 struct Ctx {
   const DevParams& P;
@@ -347,12 +349,13 @@ struct Ctx {
   __device__ __forceinline__ unsigned long long bound_word(int b) const {
     return ((unsigned long long)(~P.epoch) << 32) | (unsigned long long)((unsigned)b ^ 0x80000000u);
   }
-  // ---- tb_solve_batch: the root of the current task and its cells (thread 0) ----------------------------------------
+  // ---- tb_solve_groups: the root of the current task, its group and their cells (thread 0) --------------------------
   __device__ __forceinline__ BatchRoot& batch_root() const { return P.batch_state[c.task_idx >> c.task_depth]; }
-  __device__ __forceinline__ bool batch_root_over() const { return *(volatile int*)&batch_root().stop != 0; }
+  __device__ __forceinline__ BatchGroup& batch_group() const { return P.batch_groups[batch_ctl().group]; }
+  __device__ __forceinline__ bool batch_group_over() const { return *(volatile int*)&batch_group().stop != 0; }
   __device__ __forceinline__ void batch_cut() const { *(volatile int*)&batch_root().cut = 1; }
   __device__ __forceinline__ unsigned long long* bound_cell() const {
-    if constexpr (BATCH) return &batch_root().bound;
+    if constexpr (BATCH) return &batch_group().bound;
     else return P.cells + TB_CELL_BOUND;
   }
   // GridData::appx_best_bound (:426): this GPU's copy; a word left by another run reads as "no incumbent"
@@ -943,33 +946,33 @@ struct Ctx {
     }
   }
 
-  // ---- tb_solve_batch: the best store of the task's root --------------------------------------------------------
-  // Optimisation: the block takes the root's lock and writes the image only if its bound still beats the image's; the
+  // ---- tb_solve_groups: the best store of the task's group ------------------------------------------------------
+  // Optimisation: the block takes the group's lock and writes the image only if its bound still beats the image's; the
   // copy has landed before the lock is released, so two writers never interleave. Satisfaction: only the block that won
-  // the root's stop word gets here, and writes without the lock.
+  // the group's stop word gets here, and writes without the lock.
   __device__ __forceinline__ void batch_save_best(int bound) {
     BatchCtl& b = batch_ctl();
     if (tid == 0) {
-      BatchRoot& r = batch_root();
+      BatchGroup& g = batch_group();
       if (P.obj_var >= 0) {
-        while (atomicCAS(&r.lock, 0, 1) != 0) __nanosleep(64);
+        while (atomicCAS(&g.lock, 0, 1) != 0) __nanosleep(64);
         __threadfence();
-        b.won = bound < *(volatile int*)&r.img_bound;
+        b.won = bound < *(volatile int*)&g.img_bound;
       } else b.won = 1;
     }
     sync();
     const bool won = b.won != 0;
     if (won) {
-      save_store(P.batch_best + (size_t)(c.task_idx >> c.task_depth) * 2 * P.vpad, true);
+      save_store(P.batch_best + (size_t)b.group * 2 * P.vpad, true);
       if (threadIdx.x == 0) bulk_wait_all();
       __threadfence();
       sync();
     }
     if (tid == 0) {
-      BatchRoot& r = batch_root();
-      if (won) { *(volatile int*)&r.img_bound = bound; *(volatile int*)&r.has = 1; }
+      BatchGroup& g = batch_group();
+      if (won) { *(volatile int*)&g.img_bound = bound; *(volatile int*)&g.has = 1; }
       __threadfence();
-      if (P.obj_var >= 0) atomicExch(&r.lock, 0);
+      if (P.obj_var >= 0) atomicExch(&g.lock, 0);
     }
   }
 
@@ -1002,8 +1005,8 @@ struct Ctx {
           st->best_bound = l;
         }
       } else {
-        if constexpr (BATCH) {                  // satisfaction: the first solution of the ROOT wins
-          if (tid == 0) batch_ctl().won = atomicCAS(&batch_root().stop, 0, 1) == 0;
+        if constexpr (BATCH) {                  // satisfaction: the first solution of the GROUP wins
+          if (tid == 0) batch_ctl().won = atomicCAS(&batch_group().stop, 0, 1) == 0;
           sync();
           improved = batch_ctl().won != 0;
         } else {
@@ -1029,8 +1032,8 @@ struct Ctx {
       st->t_fixpoint += (long long)(t1 - t0);
       if (solution && P.obj_var < 0) {       // satisfaction: stop everybody after the first solution
         st->exhaustive = 0;
-        // (batch: the root's stop word is raised, its blocks move on; a root stopped by its first solution is never
-        // exhaustive, whatever weight the task that found it closes)
+        // (batch: the group's stop word is raised, the blocks of its roots move on; the root that found the group's
+        // first solution is never exhaustive, whatever weight the task that found it closes, so neither is the group)
         if constexpr (BATCH) batch_cut();
         else {
           c.stop = 1;
@@ -1196,8 +1199,10 @@ struct Ctx {
           c.task_nodes = 0; c.abandon = 0;
           c.t_mark = (long long)globaltimer_ns();
           if constexpr (BATCH) {
-            c.best_bound = TBD_PINF;          // the incumbent of ANOTHER root must never prune this one
-            c.abandon = batch_root_over();    // (nothing left to do for a root that is over)
+            c.best_bound = TBD_PINF;          // the incumbent of ANOTHER group must never prune this one
+            const BatchRoot& r = batch_root();
+            batch_ctl().group = r.group;
+            c.abandon = r.skip || batch_group_over();   // (nothing left to do for a root that is over)
           }
         }
         if constexpr (BATCH) sync();
@@ -1264,13 +1269,13 @@ struct Ctx {
               if (moved) mark_var(P.obj_var);
             }
             if (appx == TBD_NINF) {
-              if constexpr (BATCH) { *(volatile int*)&batch_root().stop = 1; batch_cut(); }   // this root only
+              if constexpr (BATCH) { *(volatile int*)&batch_group().stop = 1; batch_cut(); }   // this group only
               else { c.stop = 1; raise_stop(true); }
             }
           }
-          // batch: a root that is over (see propagate) is left at the next node, by every block working on it
+          // batch: a group that is over (see propagate) is left at the next node, by every block working on it
           bool over = false;
-          if constexpr (BATCH) { if (tid == 0) over = batch_root_over(); }
+          if constexpr (BATCH) { if (tid == 0) over = batch_group_over(); }
           // tail splitting: somebody is waiting for work and this subproblem has been going on for a while
           if (tid == 0 && !over && P.split_bits && ++c.task_nodes >= (unsigned)P.split_min_nodes && (c.task_nodes & 255u) == 0u &&
               somebody_waits() && c.task_depth + P.split_bits <= (BATCH ? P.batch_max_depth : 56) &&
@@ -1515,7 +1520,7 @@ __device__ __forceinline__ void ctx_finish(Ctx<MEM, ACT, TMALL, BATCH>& k) {
 // kernels
 // ================================================================================================
 
-// The persistent dive-and-solve kernel (gpu_barebones_solve, barebones :620-901). BATCH: tb_solve_batch.
+// The persistent dive-and-solve kernel (gpu_barebones_solve, barebones :620-901). BATCH: tb_solve_groups.
 template <int MEM, bool ACT = false, bool TMALL = false, bool BATCH = false>
 __global__ void __launch_bounds__(TB_MAX_THREADS) solve_kernel(const __grid_constant__ DevParams P) {
   extern __shared__ __align__(128) unsigned char dyn[];
@@ -1712,10 +1717,11 @@ struct tb_solver {
   // batch buffers (grown on demand)
   int *d_in_lb = nullptr, *d_in_ub = nullptr, *d_out_lb = nullptr, *d_out_ub = nullptr, *d_out_i0 = nullptr, *d_out_i1 = nullptr;
   size_t batch_cap = 0;
-  // tb_solve_batch buffers (grown on demand): root images, best images, BatchRoot cells
+  // tb_solve_groups buffers (grown on demand): root images and BatchRoot cells, best images and BatchGroup cells
   int *d_batch_roots = nullptr, *d_batch_best = nullptr;
   BatchRoot* d_batch_state = nullptr;
-  size_t batch_roots_cap = 0;
+  BatchGroup* d_batch_groups = nullptr;
+  size_t batch_roots_cap = 0, batch_groups_cap = 0;
   int32_t* h_pinned_one = nullptr;
 };
 
@@ -2590,33 +2596,51 @@ extern "C" tb_status tb_solve(tb_solver* s, volatile int32_t* stop_flag, int32_t
   return rc;
 }
 
-static tb_status ensure_batch_roots(tb_solver* s, size_t n) {
-  if (n <= s->batch_roots_cap) return TB_OK;
+static tb_status ensure_batch_buffers(tb_solver* s, size_t nroots, size_t ngroups) {
   tb_status rc;
   const size_t img = (size_t)2 * s->P.vpad;
-  if ((rc = dev_alloc(s, &s->d_batch_roots, n * img))) return rc;
-  if ((rc = dev_alloc(s, &s->d_batch_best, n * img))) return rc;
-  if ((rc = dev_alloc(s, &s->d_batch_state, n))) return rc;
-  s->batch_roots_cap = n;
+  if (nroots > s->batch_roots_cap) {
+    if ((rc = dev_alloc(s, &s->d_batch_roots, nroots * img))) return rc;
+    if ((rc = dev_alloc(s, &s->d_batch_state, nroots))) return rc;
+    s->batch_roots_cap = nroots;
+  }
+  if (ngroups > s->batch_groups_cap) {
+    if ((rc = dev_alloc(s, &s->d_batch_best, ngroups * img))) return rc;
+    if ((rc = dev_alloc(s, &s->d_batch_groups, ngroups))) return rc;
+    s->batch_groups_cap = ngroups;
+  }
   return TB_OK;
 }
 
-extern "C" tb_status tb_solve_batch(tb_solver* s, int32_t nroots, const int32_t* root_lb, const int32_t* root_ub,
-                                    volatile int32_t* stop_flag, int32_t* best_lb, int32_t* best_ub,
-                                    int32_t* has_solution, int32_t* exhaustive, int32_t* objective, tb_stats* stats) {
-  if (!s || nroots < 1 || (s->nvars && (!root_lb || !root_ub))) {
-    set_error("tb_solve_batch: needs nroots >= 1 and root_lb / root_ub"); return TB_ERR_INVALID;
+// tb_solve_groups, and tb_solve_batch with group_of[r] = r; `fn` names the entry point in error messages.
+static tb_status solve_groups(tb_solver* s, const char* fn, int32_t nroots, const int32_t* root_lb, const int32_t* root_ub,
+                              const int32_t* group_of, int32_t ngroups, volatile int32_t* stop_flag, int32_t* best_lb,
+                              int32_t* best_ub, int32_t* has_solution, int32_t* exhaustive, int32_t* objective,
+                              tb_stats* stats) {
+  const std::string name(fn);
+  if (!s || nroots < 1 || ngroups < 1 || !group_of || (s->nvars && (!root_lb || !root_ub))) {
+    set_error(name + ": needs nroots >= 1, ngroups >= 1, root_lb / root_ub and group_of"); return TB_ERR_INVALID;
   }
-  if (!s->peer_cells.empty() || s->opt.gpu_world > 1) { set_error("tb_solve_batch: a batch runs on one GPU (linked or sharded solvers are not supported)"); return TB_ERR_UNSUPPORTED; }
-  if (s->mem_kind == TB_MEM_STORE_CLUSTER) { set_error("tb_solve_batch: the STORE_CLUSTER placement is not supported"); return TB_ERR_UNSUPPORTED; }
-  if (s->P.stream_slots) { set_error("tb_solve_batch: intermediate solutions (tb_stream_solutions) are not supported"); return TB_ERR_UNSUPPORTED; }
+  if (!s->peer_cells.empty() || s->opt.gpu_world > 1) { set_error(name + ": a batch runs on one GPU (linked or sharded solvers are not supported)"); return TB_ERR_UNSUPPORTED; }
+  if (s->mem_kind == TB_MEM_STORE_CLUSTER) { set_error(name + ": the STORE_CLUSTER placement is not supported"); return TB_ERR_UNSUPPORTED; }
+  if (s->P.stream_slots) { set_error(name + ": intermediate solutions (tb_stream_solutions) are not supported"); return TB_ERR_UNSUPPORTED; }
+  std::vector<int> members((size_t)ngroups, 0);
+  for (int32_t r = 0; r < nroots; ++r) {
+    if (group_of[r] < 0 || group_of[r] >= ngroups) {
+      set_error(name + ": root " + std::to_string(r) + " names group " + std::to_string(group_of[r]) + ", outside [0, ngroups)");
+      return TB_ERR_INVALID;
+    }
+    ++members[(size_t)group_of[r]];
+  }
+  for (int32_t g = 0; g < ngroups; ++g)
+    if (!members[(size_t)g]) { set_error(name + ": group " + std::to_string(g) + " has no root"); return TB_ERR_INVALID; }
   // Every root narrows the solver's root: the layout pass chose each propagator's device class (folded constants, exact
   // 32-bit arithmetic) from the root bounds, which stays valid under narrowing only.
   const size_t nv = (size_t)s->nvars;
   for (size_t r = 0; r < (size_t)nroots; ++r)
     for (size_t v = 0; v < nv; ++v)
       if (root_lb[r * nv + v] < s->root_lb[v] || root_ub[r * nv + v] > s->root_ub[v]) {
-        set_error("tb_solve_batch: root " + std::to_string(r) + " widens the solver's domain of variable " + std::to_string(v));
+        set_error(name + ": root " + std::to_string(r) + " widens the solver's domain of variable " + std::to_string(v));
         return TB_ERR_INVALID;
       }
   CU(cudaSetDevice(s->device));
@@ -2633,30 +2657,35 @@ extern "C" tb_status tb_solve_batch(tb_solver* s, int32_t nroots, const int32_t*
   int root_bits = 0;
   while ((1ull << root_bits) < (unsigned long long)nroots) ++root_bits;
   tb_status rc;
-  if ((rc = ensure_batch_roots(s, (size_t)nroots))) return rc;
+  if ((rc = ensure_batch_buffers(s, (size_t)nroots, (size_t)ngroups))) return rc;
   DevParams P = s->P;
   const size_t img = (size_t)2 * P.vpad;
   // root images in the slot layout; a root with an empty referenced variable fails before any search, as tb_solve's
-  // does: it is over from the start, and its subproblems are skipped
+  // does: its subproblems are skipped, and its group goes on with its other roots
   std::vector<int> images((size_t)nroots * img, 0);
   std::vector<BatchRoot> state((size_t)nroots);
-  std::vector<char> failed((size_t)nroots, 0);
   for (size_t r = 0; r < (size_t)nroots; ++r) {
     int* im = images.data() + r * img;
+    BatchRoot& b = state[r];
+    memset(&b, 0, sizeof(b));
+    b.group = group_of[r];
     for (size_t v = 0; v < nv; ++v) {
       const int l = root_lb[r * nv + v], u = root_ub[r * nv + v];
       im[img_lb(s, (int)v)] = l; im[img_ub(s, (int)v)] = u;
-      if (l > u && s->layout.referenced[v]) failed[r] = 1;
+      if (l > u && s->layout.referenced[v]) b.skip = 1;
     }
-    BatchRoot& b = state[r];
-    memset(&b, 0, sizeof(b));
-    b.bound = ~0ull;                                   // epoch 0, no incumbent (as the cell at tb_create)
-    b.img_bound = TBD_PINF;
-    b.stop = failed[r];
+  }
+  std::vector<BatchGroup> groups((size_t)ngroups);
+  for (BatchGroup& g : groups) {
+    memset(&g, 0, sizeof(g));
+    g.bound = ~0ull;                                   // epoch 0, no incumbent (as the cell at tb_create)
+    g.img_bound = TBD_PINF;
   }
   CU(cudaMemcpyAsync(s->d_batch_roots, images.data(), images.size() * sizeof(int), cudaMemcpyHostToDevice, s->stream));
   CU(cudaMemcpyAsync(s->d_batch_state, state.data(), state.size() * sizeof(BatchRoot), cudaMemcpyHostToDevice, s->stream));
+  CU(cudaMemcpyAsync(s->d_batch_groups, groups.data(), groups.size() * sizeof(BatchGroup), cudaMemcpyHostToDevice, s->stream));
   P.batch_roots = s->d_batch_roots; P.batch_best = s->d_batch_best; P.batch_state = s->d_batch_state;
+  P.batch_groups = s->d_batch_groups;
   P.subproblems_power = d;
   P.num_subproblems = (unsigned long long)nroots << d;
   P.batch_max_depth = std::min(TB_BATCH_WEIGHT_BITS, 64 - root_bits);
@@ -2674,7 +2703,7 @@ extern "C" tb_status tb_solve_batch(tb_solver* s, int32_t nroots, const int32_t*
   SearchRun run;
   rc = run_search(s, P, t_begin, stop_flag, [&](const DevParams& Pl) {
     return dispatch(s, [&](auto M, auto A, auto TM) -> tb_status {
-      if constexpr (decltype(M)::value == TB_MEM_STORE_CLUSTER) { set_error("tb_solve_batch: STORE_CLUSTER"); return TB_ERR_UNSUPPORTED; }
+      if constexpr (decltype(M)::value == TB_MEM_STORE_CLUSTER) { set_error(name + ": STORE_CLUSTER"); return TB_ERR_UNSUPPORTED; }
       else {
         CU(launch_workers(s, solve_kernel<decltype(M)::value, decltype(A)::value, decltype(TM)::value, true>, s->num_blocks, Pl));
         CU(cudaGetLastError());
@@ -2684,9 +2713,11 @@ extern "C" tb_status tb_solve_batch(tb_solver* s, int32_t nroots, const int32_t*
   }, run);
   if (rc) return rc;
   CU(cudaMemcpy(state.data(), s->d_batch_state, state.size() * sizeof(BatchRoot), cudaMemcpyDeviceToHost));
+  CU(cudaMemcpy(groups.data(), s->d_batch_groups, groups.size() * sizeof(BatchGroup), cudaMemcpyDeviceToHost));
   bool any = false;
-  for (auto& b : state) any |= b.has != 0;
-  if (any) CU(cudaMemcpy(images.data(), s->d_batch_best, images.size() * sizeof(int), cudaMemcpyDeviceToHost));
+  for (auto& g : groups) any |= g.has != 0;
+  std::vector<int> best(any ? (size_t)ngroups * img : 0);
+  if (any) CU(cudaMemcpy(best.data(), s->d_batch_best, best.size() * sizeof(int), cudaMemcpyDeviceToHost));
   tb_stats st; memset(&st, 0, sizeof(st));
   st.exhaustive = 1;
   fill_config(s, &st);
@@ -2694,30 +2725,48 @@ extern "C" tb_status tb_solve_batch(tb_solver* s, int32_t nroots, const int32_t*
   st.eps_num_subproblems = P.num_subproblems;
   reduce_stats(run.blocks, &st, nullptr);
   for (auto& b : run.blocks) if (b.error) { set_error("decision stack overflow (raise max_depth)"); rc = (tb_status)b.error; }
-  // per root: exhaustive iff all of its search space was closed and no block was cut while searching it (roots that
-  // finished before a stop or a timeout stay exhaustive); a failed root is exhaustive without a solution
+  // per root: exhausted iff all of its search space was closed and no block was cut while searching it (roots that
+  // finished before a stop or a timeout stay exhausted); a skipped root is exhausted without a solution. A group is
+  // exhaustive iff all of its roots are.
   const unsigned long long all = 1ull << TB_BATCH_WEIGHT_BITS;
+  std::vector<int> exh((size_t)ngroups, 1);
+  for (const BatchRoot& b : state) exh[(size_t)b.group] &= b.skip ? 1 : (b.closed == all && !b.cut);
   int all_exhaustive = 1;
   std::vector<int32_t> lb(std::max<size_t>(1, nv)), ub(std::max<size_t>(1, nv));
-  for (size_t r = 0; r < (size_t)nroots; ++r) {
-    const BatchRoot& b = state[r];
-    const bool has = !failed[r] && b.has;
-    const int exh = failed[r] ? 1 : (b.closed == all && !b.cut);
-    all_exhaustive &= exh;
-    if (has_solution) has_solution[r] = has;
-    if (exhaustive) exhaustive[r] = exh;
-    if (objective) objective[r] = TB_POS_INF;
+  for (size_t g = 0; g < (size_t)ngroups; ++g) {
+    const bool has = groups[g].has != 0;
+    all_exhaustive &= exh[g];
+    if (has_solution) has_solution[g] = has;
+    if (exhaustive) exhaustive[g] = exh[g];
+    if (objective) objective[g] = TB_POS_INF;
     if (!has) continue;
-    unpack_store(s, images.data() + r * img, lb.data(), ub.data());
-    if (objective && s->root_obj_var >= 0) objective[r] = lb[(size_t)s->root_obj_var];
-    if (best_lb && nv) memcpy(best_lb + r * nv, lb.data(), nv * 4);
-    if (best_ub && nv) memcpy(best_ub + r * nv, ub.data(), nv * 4);
+    unpack_store(s, best.data() + g * img, lb.data(), ub.data());
+    if (objective && s->root_obj_var >= 0) objective[g] = lb[(size_t)s->root_obj_var];
+    if (best_lb && nv) memcpy(best_lb + g * nv, lb.data(), nv * 4);
+    if (best_ub && nv) memcpy(best_ub + g * nv, ub.data(), nv * 4);
   }
   st.exhaustive = all_exhaustive;
   st.kernel_ms = run.kernel_ms;
   st.timers_ns[TB_TIMER_OVERALL] = (int64_t)((now_ms() - t_begin) * 1e6);
   if (stats) *stats = st;
   return rc;
+}
+
+extern "C" tb_status tb_solve_groups(tb_solver* s, int32_t nroots, const int32_t* root_lb, const int32_t* root_ub,
+                                     const int32_t* group_of, int32_t ngroups, volatile int32_t* stop_flag,
+                                     int32_t* best_lb, int32_t* best_ub, int32_t* has_solution, int32_t* exhaustive,
+                                     int32_t* objective, tb_stats* stats) {
+  return solve_groups(s, "tb_solve_groups", nroots, root_lb, root_ub, group_of, ngroups, stop_flag, best_lb, best_ub,
+                      has_solution, exhaustive, objective, stats);
+}
+
+extern "C" tb_status tb_solve_batch(tb_solver* s, int32_t nroots, const int32_t* root_lb, const int32_t* root_ub,
+                                    volatile int32_t* stop_flag, int32_t* best_lb, int32_t* best_ub,
+                                    int32_t* has_solution, int32_t* exhaustive, int32_t* objective, tb_stats* stats) {
+  std::vector<int32_t> own((size_t)std::max(0, nroots));
+  for (size_t r = 0; r < own.size(); ++r) own[r] = (int32_t)r;
+  return solve_groups(s, "tb_solve_batch", nroots, root_lb, root_ub, own.data(), nroots, stop_flag, best_lb, best_ub,
+                      has_solution, exhaustive, objective, stats);
 }
 
 // ---- final gather across processes (SURVEY §8e; reduce_blocks, barebones :1033-1067, across GPUs) -------------------

@@ -71,20 +71,27 @@ struct SplitEntry {
 static_assert(sizeof(SplitEntry) == 32, "TB_CELL_BLOCK_BYTES counts 32 bytes per pool entry");
 #define TB_SPLIT_CAP 16384
 
-// tb_solve_batch: what the grid shares about one root of the batch (written by the host before each launch).
-// Subproblem index g = (r << d) | local; a task of depth D belongs to root g >> D.
+// tb_solve_groups / tb_solve_batch: what the grid shares about one root of the batch and about one group of roots
+// (both written by the host before each launch). Subproblem index g = (r << d) | local; a task of depth D belongs to
+// root g >> D, and root r to group BatchRoot::group. A group is solved over the union of its roots' boxes: the roots
+// share its incumbent, its stop word and its best store. tb_solve_batch puts every root in a group of its own.
 struct BatchRoot {
-  unsigned long long bound;     // the root's incumbent, the TB_CELL_BOUND word (epoch-tagged, unsigned atomicMin)
   unsigned long long closed;    // weight of the root's search space closed: 2^(56 - D) per task of depth D searched to
                                 // the end, 2^(56 - D + rem) per dive leaf at remaining depth rem; 2^56 = everything
-  int stop;                     // the root is over (first solution of a satisfaction problem, unbounded objective)
   int cut;                      // a block was cut (stop, cutnodes, depth) while searching it, or stop was raised
-  int lock;                     // one writer of the root's best image at a time
-  int has;                      // the best image holds a solution
-  int img_bound;                // objective of the best image (TBD_PINF = none)
+  int skip;                     // a referenced domain is empty at the root: decided on the host, its subproblems skipped
+  int group;                    // the group the root belongs to
   int pad_;
 };
-static_assert(sizeof(BatchRoot) == 40, "host and device agree on BatchRoot");
+static_assert(sizeof(BatchRoot) == 24, "host and device agree on BatchRoot");
+struct BatchGroup {
+  unsigned long long bound;     // the group's incumbent, the TB_CELL_BOUND word (epoch-tagged, unsigned atomicMin)
+  int stop;                     // the group is over (first solution of a satisfaction problem, unbounded objective)
+  int lock;                     // one writer of the group's best image at a time
+  int has;                      // the best image holds a solution
+  int img_bound;                // objective of the best image (TBD_PINF = none)
+};
+static_assert(sizeof(BatchGroup) == 24, "host and device agree on BatchGroup");
 #define TB_BATCH_WEIGHT_BITS 56
 
 // words of the split control block (unsigned), which lives in the cell block (TB_CELL_SPLIT) so that the peers see it
@@ -146,10 +153,13 @@ struct DevParams {
   int tmem_cols, tmem_visits;
   int act_off;                           // byte offset of the active-set area in dynamic shared memory
   int act_fpw;                           // chunk flags per warp (multiple of 32): chunk ch is flag (ch / nwarps) of warp (ch % nwarps)
-  // tb_solve_batch (read by the BATCH kernels only): num_subproblems = nroots << subproblems_power
+  // tb_solve_groups (read by the BATCH kernels only): num_subproblems = nroots << subproblems_power
   const int* batch_roots;                // [nroots][2 * vpad] root images, layout of a block store
-  int* batch_best;                       // [nroots][2 * vpad] best store of each root
+  int* batch_best;                       // [ngroups][2 * vpad] best store of each group
   BatchRoot* batch_state;                // [nroots]
   int batch_max_depth;                   // deepest task: root bits + depth fit the 64-bit index, at most 56
   int pad6_;
+  BatchGroup* batch_groups;              // [ngroups]
+  unsigned long long pad8_;              // the size stays a multiple of 16: the kernel arguments behind DevParams keep
+                                         // their alignment, so their loads keep their width
 };

@@ -39,6 +39,8 @@ def lib():
         L.tb_dive_batch.argtypes = [vp, C.c_uint64, C.c_int32, C.c_int32, i32p, i32p, i32p, i32p]
         L.tb_solve.argtypes = [vp, i32p, i32p, i32p, i32p, i32p, C.POINTER(abi.TbStats)]
         L.tb_solve_batch.argtypes = [vp, C.c_int32, i32p, i32p, i32p, i32p, i32p, i32p, i32p, i32p, C.POINTER(abi.TbStats)]
+        L.tb_solve_groups.argtypes = [vp, C.c_int32, i32p, i32p, i32p, C.c_int32, i32p, i32p, i32p, i32p, i32p, i32p,
+                                      C.POINTER(abi.TbStats)]
         L.tb_link_peers.argtypes = [C.POINTER(vp), C.c_int32]
         L.tb_export_bound_handle.argtypes = [vp, vp]
         L.tb_import_peer_bounds.argtypes = [vp, vp, C.c_int32]
@@ -53,7 +55,7 @@ def lib():
         L.tb_version.restype = C.c_char_p
         L.tb_device_count.restype = C.c_int32
         for name in ("tb_create", "tb_propagate", "tb_propagate_batch", "tb_dive", "tb_dive_batch", "tb_solve",
-                     "tb_solve_batch", "tb_link_peers", "tb_export_bound_handle", "tb_import_peer_bounds", "tb_read_bound",
+                     "tb_solve_batch", "tb_solve_groups", "tb_link_peers", "tb_export_bound_handle", "tb_import_peer_bounds", "tb_read_bound",
                      "tb_get_config"):
             getattr(L, name).restype = C.c_int
         _LIB = L
@@ -251,6 +253,35 @@ class Solver:
                                     C.byref(st)))
         return dict(lb=olb[:, :n], ub=oub[:, :n], has_solution=has[:k].astype(bool), exhaustive=exh[:k].astype(bool),
                     objective=obj[:k].astype(np.int64), stats=st.as_dict())
+
+    def solve_groups(self, lb, ub, groups, ngroups=None, stop_flag=None):
+        """tb_solve_groups: K roots of this solver's network ([K, nvars] int32 boxes, each a narrowing of the
+        problem's), root r a box of group groups[r]; each group is solved over the union of its boxes, with one
+        incumbent shared by its boxes. `ngroups` defaults to max(groups) + 1. Returns arrays of length ngroups, shaped
+        as solve_batch's."""
+        n = self.problem.nvars
+        lb = np.ascontiguousarray(lb, dtype=np.int32).reshape(-1, n)
+        ub = np.ascontiguousarray(ub, dtype=np.int32).reshape(-1, n)
+        if lb.shape != ub.shape:
+            raise ValueError("lb and ub must have the same shape [K, nvars]")
+        k = lb.shape[0]
+        groups = np.ascontiguousarray(groups, dtype=np.int32).reshape(-1)
+        if groups.shape[0] != k:
+            raise ValueError("groups must have one entry per root")
+        if ngroups is None:
+            ngroups = int(groups.max()) + 1 if k else 0
+        m = max(1, ngroups)
+        olb = np.zeros((m, max(1, n)), np.int32)
+        oub = np.zeros((m, max(1, n)), np.int32)
+        has = np.zeros(m, np.int32)
+        exh = np.zeros(m, np.int32)
+        obj = np.zeros(m, np.int32)
+        st = abi.TbStats()
+        _check(lib().tb_solve_groups(self._h, k, _p(lb), _p(ub), _p(groups), ngroups, stop_flag, _p(olb), _p(oub),
+                                     _p(has), _p(exh), _p(obj), C.byref(st)))
+        g = max(0, ngroups)
+        return dict(lb=olb[:g, :n], ub=oub[:g, :n], has_solution=has[:g].astype(bool), exhaustive=exh[:g].astype(bool),
+                    objective=obj[:g].astype(np.int64), stats=st.as_dict())
 
     def export_bound_handle(self):
         buf = C.create_string_buffer(64)
