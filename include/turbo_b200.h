@@ -203,6 +203,31 @@ tb_status tb_solve_groups(tb_solver*, int32_t nroots, const int32_t* root_lb, co
                           int32_t* best_lb, int32_t* best_ub, int32_t* has_solution, int32_t* exhaustive,
                           int32_t* objective, tb_stats* stats);
 
+/* Optimises nobj objectives of one network over one union of boxes, in one launch: objective m minimises
+ * (maximize[m] == 0) or maximises (maximize[m] == 1) variable obj_var[m] over the union of nboxes boxes (box_lb /
+ * box_ub laid out [nboxes][nvars], each a narrowing of the solver's root, as in tb_solve_groups). The solution hull of
+ * a model - the smallest and largest value of each variable in any solution - is 2n such objectives. The problem's own
+ * obj_var plays no part: to keep to optimal or near-optimal solutions, narrow its upper bound in the boxes. All the
+ * objectives share the union, so every solution any of them finds is a witness for all of them: it gives every
+ * objective it improves an incumbent and, where it beats that objective's best, its store. Outputs per objective
+ * [nobj]: has_solution; objective = the optimum in the objective's own sense (TB_POS_INF without a solution; an
+ * unbounded maximisation reports TB_POS_INF and an unbounded minimisation TB_NEG_INF, with has_solution = 1, and that
+ * objective ends there, not exhaustive); exhaustive = every box was searched to its end for this objective and no block
+ * was cut while doing so (a non-exhaustive objective holds a witnessed value: an inner bound of the hull); best_lb /
+ * best_ub [nobj][nvars] (may be NULL) = a solution store with obj_var[m] FIXED to the objective's value, so that the
+ * row's lower bounds are a point with that value (rows of objectives without a solution are left as they are).
+ * Repeated objectives are legal; a box with an empty referenced domain is decided on the host, as in tb_solve_groups.
+ * A box in which an objective's variable is empty but read by no propagator gives that objective no solution (its
+ * search fails at every node of the box), while the other objectives search the box as usual.
+ * stop_flag, the timeout and the subproblems per root apply as in tb_solve_groups, with nobj * nboxes roots.
+ * TB_ERR_INVALID: nboxes < 1, nobj < 1, an obj_var outside [0, nvars), a maximize other than 0 / 1, a widening box,
+ * nobj * nboxes above 2^40 (the subproblem index). TB_ERR_NOMEM: no host memory for the nobj * nboxes roots.
+ * TB_ERR_UNSUPPORTED: as tb_solve_batch. */
+tb_status tb_solve_objectives(tb_solver*, int32_t nboxes, const int32_t* box_lb, const int32_t* box_ub,
+                              int32_t nobj, const int32_t* obj_var, const int32_t* maximize,
+                              volatile int32_t* stop_flag, int32_t* best_lb, int32_t* best_ub,
+                              int32_t* has_solution, int32_t* exhaustive, int32_t* objective, tb_stats* stats);
+
 /* Intermediate solutions (-i / -a; the reference's consumer thread, gpu_dive_and_solve.hpp:100-132; its barebones
  * architecture cannot, barebones_dive_and_solve.hpp:465-467).  tb_stream_solutions (before tb_solve) makes every
  * improving solution also land in a ring of `slots` store images; tb_poll_solution, called from ANOTHER host thread

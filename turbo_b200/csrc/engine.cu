@@ -27,6 +27,7 @@
 #include <time.h>
 #include <algorithm>
 #include <mutex>
+#include <new>
 #include <string>
 #include <type_traits>
 #include <vector>
@@ -300,15 +301,22 @@ __device__ __forceinline__ int chunk_class(const DevParams& P, int ch) {
 }
 
 // Per-CTA state of the BATCH kernels only (a function-scope __shared__ object: the other kernels never reference it).
-// `group`: the group of the current task's root, set by thread 0 when the task starts.
-struct BatchCtl { int won; int group; };
+// Set by thread 0 when a task starts: `group`, the group of the task's root, its objective slot `obj` (-1 =
+// satisfaction) and sense `maximize`, and `image`, the root's box. `pick` / `key`: witness sharing (batch_share_witness).
+struct BatchCtl { int won; int group; int obj; int maximize; int image; int pick; int key; };
 __device__ __forceinline__ BatchCtl& batch_ctl() { __shared__ BatchCtl b; return b; }
+
+// The incumbent's key of a solution's objective domain [l, u]: l when minimising, ~u = -u - 1 when maximising. The
+// incumbent is the minimum key in both senses. The one's complement is a decreasing bijection of the int32 range that
+// swaps the sentinels (~TBD_PINF = TBD_NINF, the key of an unbounded objective; ~TBD_NINF = TBD_PINF, "none") and keeps
+// every finite bound finite: -u would turn u = INT32_MIN + 1 into TBD_PINF, a solution never recorded.
+__device__ __forceinline__ int objective_key(int l, int u, int maximize) { return maximize ? ~u : l; }
 
 // TMALL: every visit of every warp finds its propagator word in tensor memory (the table fits): the sweep is compiled
 // without the L2 path and without the test that chooses between the two.
-// BATCH: tb_solve_groups - subproblem g of depth D belongs to root g >> D, which has its own image and closed-weight
-// counter (BatchRoot); its group has the incumbent, the stop word and the best store (BatchGroup); every batch-only
-// branch is `if constexpr`.
+// BATCH: tb_solve_groups - subproblem g of depth D belongs to root g >> D, which has its image and closed-weight counter
+// (BatchRoot); its group has the objective, the incumbent, the stop word and the best store (BatchGroup); every
+// batch-only branch is `if constexpr`.
 template <int MEM, bool ACT = false, bool TMALL = false, bool BATCH = false>
 struct Ctx {
   const DevParams& P;
@@ -354,6 +362,16 @@ struct Ctx {
   __device__ __forceinline__ BatchGroup& batch_group() const { return P.batch_groups[batch_ctl().group]; }
   __device__ __forceinline__ bool batch_group_over() const { return *(volatile int*)&batch_group().stop != 0; }
   __device__ __forceinline__ void batch_cut() const { *(volatile int*)&batch_root().cut = 1; }
+  // the objective slot of the current task (-1 = satisfaction) and its sense: the problem's (minimise), or (BATCH) its
+  // group's; every BATCH read of the objective goes through these two
+  __device__ __forceinline__ int obj_slot() const {
+    if constexpr (BATCH) return batch_ctl().obj;
+    else return P.obj_var;
+  }
+  __device__ __forceinline__ bool maximizes() const {
+    if constexpr (BATCH) return batch_ctl().maximize != 0;
+    else return false;
+  }
   __device__ __forceinline__ unsigned long long* bound_cell() const {
     if constexpr (BATCH) return &batch_group().bound;
     else return P.cells + TB_CELL_BOUND;
@@ -946,15 +964,15 @@ struct Ctx {
     }
   }
 
-  // ---- tb_solve_groups: the best store of the task's group ------------------------------------------------------
-  // Optimisation: the block takes the group's lock and writes the image only if its bound still beats the image's; the
+  // ---- tb_solve_groups: the best store of group `grp` -----------------------------------------------------------
+  // Optimisation: the block takes the group's lock and writes the image only if its key still beats the image's; the
   // copy has landed before the lock is released, so two writers never interleave. Satisfaction: only the block that won
   // the group's stop word gets here, and writes without the lock.
-  __device__ __forceinline__ void batch_save_best(int bound) {
+  __device__ __forceinline__ void batch_save_best(int grp, int bound, bool optimise) {
     BatchCtl& b = batch_ctl();
     if (tid == 0) {
-      BatchGroup& g = batch_group();
-      if (P.obj_var >= 0) {
+      BatchGroup& g = P.batch_groups[grp];
+      if (optimise) {
         while (atomicCAS(&g.lock, 0, 1) != 0) __nanosleep(64);
         __threadfence();
         b.won = bound < *(volatile int*)&g.img_bound;
@@ -963,16 +981,56 @@ struct Ctx {
     sync();
     const bool won = b.won != 0;
     if (won) {
-      save_store(P.batch_best + (size_t)b.group * 2 * P.vpad, true);
+      save_store(P.batch_best + (size_t)grp * 2 * P.vpad, true);
       if (threadIdx.x == 0) bulk_wait_all();
       __threadfence();
       sync();
     }
     if (tid == 0) {
-      BatchGroup& g = batch_group();
+      BatchGroup& g = P.batch_groups[grp];
       if (won) { *(volatile int*)&g.img_bound = bound; *(volatile int*)&g.has = 1; }
       __threadfence();
-      if (P.obj_var >= 0) atomicExch(&g.lock, 0);
+      if (optimise) atomicExch(&g.lock, 0);
+    }
+  }
+
+  // ---- tb_solve_objectives: a solution is a witness for every group ----------------------------------------------
+  // The groups optimise over the same union of boxes, so a solution of one is a solution of every group whose objective
+  // variable is not empty in it (see below). The threads split the
+  // other groups (the task's own group went through propagate()): each computes the group's key from the store,
+  // publishes it where it beats the group's incumbent, and asks for the image where it beats the group's best image.
+  // The block then writes the image into those rows one group at a time, as batch_save_best does, so it holds one lock
+  // at a time. An unbounded key ends its group, as it ends the group that finds it.
+  __device__ __forceinline__ void batch_share_witness() {
+    BatchCtl& b = batch_ctl();
+    const int own = b.group, n = P.batch_share;
+    for (int base = 0; base < n; base += T) {
+      const int grp = base + tid;
+      int key = TBD_PINF;
+      bool want = false;
+      if (grp < n && grp != own) {
+        BatchGroup& g = P.batch_groups[grp];
+        int l, u; store.ld(g.obj, l, u);
+        // (an objective variable the propagators do not see can be empty in a box whose other variables have
+        // solutions: that group fails every node of the box, as its own search does, and the store is no witness for it)
+        if (l <= u) {
+          key = objective_key(l, u, g.maximize);
+          const unsigned long long w = bound_word(key);
+          if (w < *(volatile unsigned long long*)&g.bound) atomicMin(&g.bound, w);
+          if (key == TBD_NINF) *(volatile int*)&g.stop = 1;
+          want = key < *(volatile int*)&g.img_bound;
+        }
+      }
+      for (;;) {                                // one row per round: the lowest thread that still wants one
+        if (tid == 0) b.pick = T;
+        if (!__syncthreads_or(want)) break;
+        if (want) atomicMin(&b.pick, tid);
+        __syncthreads();
+        const int t = b.pick;
+        if (tid == t) { b.key = key; want = false; }
+        __syncthreads();
+        batch_save_best(base + t, b.key, true);
+      }
     }
   }
 
@@ -984,7 +1042,7 @@ struct Ctx {
     if (tid == 0) t0 = globaltimer_ns();
     int iters = 0, f;
     bool pre_failed = P.root_failed != 0;       // a referenced variable is already empty in the root store
-    if (P.obj_var >= 0) { int l, u; store.ld(P.obj_var, l, u); pre_failed |= l > u; }
+    if (obj_slot() >= 0) { int l, u; store.ld(obj_slot(), l, u); pre_failed |= l > u; }
     if (pre_failed) f = F_FAILED;
     else if constexpr (ACT) f = fixpoint_active(iters);
     else f = fixpoint(iters);
@@ -994,8 +1052,9 @@ struct Ctx {
     if (tid == 0) t1 = globaltimer_ns();
     bool improved = false;
     if (solution) {
-      if (P.obj_var >= 0) {
-        int l, u; store.ld(P.obj_var, l, u);
+      if (obj_slot() >= 0) {
+        int l, u; store.ld(obj_slot(), l, u);
+        if constexpr (BATCH) l = objective_key(l, u, maximizes());   // (the group's key)
         improved = c.best_bound > l;           // uniform: same smem word read by everybody
         sync();
         if (improved && tid == 0) {
@@ -1016,11 +1075,12 @@ struct Ctx {
         if (tid == 0) st->t_best = (long long)(globaltimer_ns() - P.t_start);
       }
       if (improved) {
-        if constexpr (BATCH) batch_save_best(P.obj_var >= 0 ? c.best_bound : 0);
+        if constexpr (BATCH) batch_save_best(batch_ctl().group, obj_slot() >= 0 ? c.best_bound : 0, obj_slot() >= 0);
         else save_store(g_best);
         if (tid == 0) { st->solutions++; st->has_best = 1; }
         if constexpr (!BATCH) { if (P.stream_slots) stream_solution(P.obj_var >= 0 ? c.best_bound : 0); }
       }
+      if constexpr (BATCH) { if (P.batch_share) batch_share_witness(); }
     }
     if (tid == 0) {
       c.leaf = failed || solution;
@@ -1030,7 +1090,7 @@ struct Ctx {
       st->fails += failed ? 1 : 0;
       if (c.depth > st->depth_max) st->depth_max = c.depth;
       st->t_fixpoint += (long long)(t1 - t0);
-      if (solution && P.obj_var < 0) {       // satisfaction: stop everybody after the first solution
+      if (solution && obj_slot() < 0) {      // satisfaction: stop everybody after the first solution
         st->exhaustive = 0;
         // (batch: the group's stop word is raised, the blocks of its roots move on; the root that found the group's
         // first solution is never exhaustive, whatever weight the task that found it closes, so neither is the group)
@@ -1201,7 +1261,9 @@ struct Ctx {
           if constexpr (BATCH) {
             c.best_bound = TBD_PINF;          // the incumbent of ANOTHER group must never prune this one
             const BatchRoot& r = batch_root();
-            batch_ctl().group = r.group;
+            const BatchGroup& g = P.batch_groups[r.group];
+            BatchCtl& b = batch_ctl();
+            b.group = r.group; b.image = r.image; b.obj = g.obj; b.maximize = g.maximize;
             c.abandon = r.skip || batch_group_over();   // (nothing left to do for a root that is over)
           }
         }
@@ -1209,7 +1271,7 @@ struct Ctx {
         if (BATCH && c.abandon) mode = M_NEXT;
         else {
           for (int i = tid; i < P.nsnap; i += T) g_snap_tag[i] = -1;       // snapshots belong to one subproblem
-          if constexpr (BATCH) load_store(P.batch_roots + (size_t)(idx >> c.task_depth) * 2 * P.vpad);
+          if constexpr (BATCH) load_store(P.batch_roots + (size_t)batch_ctl().image * 2 * P.vpad);
           else load_store(P.root_store);
           sync();
           mode = M_DIVE;
@@ -1261,12 +1323,19 @@ struct Ctx {
         if (c.stop) mode = M_SOLVE_END;
         else {
           // I. inject the incumbent bound (thread 0), detect an unconstrained objective
-          if (tid == 0 && P.obj_var >= 0) {
+          // (batch, a group that maximises: the incumbent is the key ~ub, so lb narrows to ~key + 1)
+          if (tid == 0 && obj_slot() >= 0) {
             int appx = read_bound();
             if (appx != TBD_PINF) {
-              bool moved = store.embed(P.obj_var, TBD_NINF, tbd::pred(appx));
-              moved |= store.embed(P.obj_var, TBD_NINF, tbd::pred(c.best_bound));
-              if (moved) mark_var(P.obj_var);
+              bool moved;
+              if (maximizes()) {
+                moved = store.embed(obj_slot(), tbd::succ(~appx), TBD_PINF);
+                moved |= store.embed(obj_slot(), tbd::succ(~c.best_bound), TBD_PINF);
+              } else {
+                moved = store.embed(obj_slot(), TBD_NINF, tbd::pred(appx));
+                moved |= store.embed(obj_slot(), TBD_NINF, tbd::pred(c.best_bound));
+              }
+              if (moved) mark_var(obj_slot());
             }
             if (appx == TBD_NINF) {
               if constexpr (BATCH) { *(volatile int*)&batch_group().stop = 1; batch_cut(); }   // this group only
@@ -1717,11 +1786,11 @@ struct tb_solver {
   // batch buffers (grown on demand)
   int *d_in_lb = nullptr, *d_in_ub = nullptr, *d_out_lb = nullptr, *d_out_ub = nullptr, *d_out_i0 = nullptr, *d_out_i1 = nullptr;
   size_t batch_cap = 0;
-  // tb_solve_groups buffers (grown on demand): root images and BatchRoot cells, best images and BatchGroup cells
+  // tb_solve_groups buffers (grown on demand): root images, BatchRoot cells, best images and BatchGroup cells
   int *d_batch_roots = nullptr, *d_batch_best = nullptr;
   BatchRoot* d_batch_state = nullptr;
   BatchGroup* d_batch_groups = nullptr;
-  size_t batch_roots_cap = 0, batch_groups_cap = 0;
+  size_t batch_images_cap = 0, batch_roots_cap = 0, batch_groups_cap = 0;
   int32_t* h_pinned_one = nullptr;
 };
 
@@ -2596,11 +2665,14 @@ extern "C" tb_status tb_solve(tb_solver* s, volatile int32_t* stop_flag, int32_t
   return rc;
 }
 
-static tb_status ensure_batch_buffers(tb_solver* s, size_t nroots, size_t ngroups) {
+static tb_status ensure_batch_buffers(tb_solver* s, size_t nimages, size_t nroots, size_t ngroups) {
   tb_status rc;
   const size_t img = (size_t)2 * s->P.vpad;
+  if (nimages > s->batch_images_cap) {
+    if ((rc = dev_alloc(s, &s->d_batch_roots, nimages * img))) return rc;
+    s->batch_images_cap = nimages;
+  }
   if (nroots > s->batch_roots_cap) {
-    if ((rc = dev_alloc(s, &s->d_batch_roots, nroots * img))) return rc;
     if ((rc = dev_alloc(s, &s->d_batch_state, nroots))) return rc;
     s->batch_roots_cap = nroots;
   }
@@ -2612,34 +2684,43 @@ static tb_status ensure_batch_buffers(tb_solver* s, size_t nroots, size_t ngroup
   return TB_OK;
 }
 
-// tb_solve_groups, and tb_solve_batch with group_of[r] = r; `fn` names the entry point in error messages.
-static tb_status solve_groups(tb_solver* s, const char* fn, int32_t nroots, const int32_t* root_lb, const int32_t* root_ub,
-                              const int32_t* group_of, int32_t ngroups, volatile int32_t* stop_flag, int32_t* best_lb,
-                              int32_t* best_ub, int32_t* has_solution, int32_t* exhaustive, int32_t* objective,
-                              tb_stats* stats) {
+// The one host path of the BATCH kernel: tb_solve_groups, tb_solve_batch and tb_solve_objectives. `nimages` boxes
+// (box_lb / box_ub [nimages][nvars]); root r searches box image_of[r] for group group_of[r] (nroots entries); group g
+// optimises variable obj_of[g] (-1 = satisfaction) in the sense maximize[g] (ngroups entries). `objectives`
+// (tb_solve_objectives): every solution is a witness for every group, each returned row has the group's objective
+// variable fixed to its value, and an unbounded objective is never exhaustive. `fn` names the entry point in errors.
+static tb_status solve_groups(tb_solver* s, const char* fn, int32_t nimages, const int32_t* box_lb, const int32_t* box_ub,
+                              long long nroots, const int32_t* image_of, const int32_t* group_of, int32_t ngroups,
+                              const int32_t* obj_of, const int32_t* maximize, bool objectives,
+                              volatile int32_t* stop_flag, int32_t* best_lb, int32_t* best_ub, int32_t* has_solution,
+                              int32_t* exhaustive, int32_t* objective, tb_stats* stats) {
   const std::string name(fn);
-  if (!s || nroots < 1 || ngroups < 1 || !group_of || (s->nvars && (!root_lb || !root_ub))) {
+  if (!s || nimages < 1 || nroots < 1 || ngroups < 1 || !group_of || (s->nvars && (!box_lb || !box_ub))) {
     set_error(name + ": needs nroots >= 1, ngroups >= 1, root_lb / root_ub and group_of"); return TB_ERR_INVALID;
   }
   if (!s->peer_cells.empty() || s->opt.gpu_world > 1) { set_error(name + ": a batch runs on one GPU (linked or sharded solvers are not supported)"); return TB_ERR_UNSUPPORTED; }
   if (s->mem_kind == TB_MEM_STORE_CLUSTER) { set_error(name + ": the STORE_CLUSTER placement is not supported"); return TB_ERR_UNSUPPORTED; }
   if (s->P.stream_slots) { set_error(name + ": intermediate solutions (tb_stream_solutions) are not supported"); return TB_ERR_UNSUPPORTED; }
-  std::vector<int> members((size_t)ngroups, 0);
-  for (int32_t r = 0; r < nroots; ++r) {
+  // the subproblem index (r << d) | local is counted by the dispenser's TB_K_BITS field
+  if ((unsigned long long)nroots > (1ull << TB_K_BITS)) {
+    set_error(name + ": " + std::to_string(nroots) + " roots do not fit the subproblem index (at most 2^40)"); return TB_ERR_INVALID;
+  }
+  std::vector<char> has_root((size_t)ngroups, 0);
+  for (long long r = 0; r < nroots; ++r) {
     if (group_of[r] < 0 || group_of[r] >= ngroups) {
       set_error(name + ": root " + std::to_string(r) + " names group " + std::to_string(group_of[r]) + ", outside [0, ngroups)");
       return TB_ERR_INVALID;
     }
-    ++members[(size_t)group_of[r]];
+    has_root[(size_t)group_of[r]] = 1;
   }
   for (int32_t g = 0; g < ngroups; ++g)
-    if (!members[(size_t)g]) { set_error(name + ": group " + std::to_string(g) + " has no root"); return TB_ERR_INVALID; }
-  // Every root narrows the solver's root: the layout pass chose each propagator's device class (folded constants, exact
+    if (!has_root[(size_t)g]) { set_error(name + ": group " + std::to_string(g) + " has no root"); return TB_ERR_INVALID; }
+  // Every box narrows the solver's root: the layout pass chose each propagator's device class (folded constants, exact
   // 32-bit arithmetic) from the root bounds, which stays valid under narrowing only.
   const size_t nv = (size_t)s->nvars;
-  for (size_t r = 0; r < (size_t)nroots; ++r)
+  for (size_t r = 0; r < (size_t)nimages; ++r)
     for (size_t v = 0; v < nv; ++v)
-      if (root_lb[r * nv + v] < s->root_lb[v] || root_ub[r * nv + v] > s->root_ub[v]) {
+      if (box_lb[r * nv + v] < s->root_lb[v] || box_ub[r * nv + v] > s->root_ub[v]) {
         set_error(name + ": root " + std::to_string(r) + " widens the solver's domain of variable " + std::to_string(v));
         return TB_ERR_INVALID;
       }
@@ -2657,35 +2738,44 @@ static tb_status solve_groups(tb_solver* s, const char* fn, int32_t nroots, cons
   int root_bits = 0;
   while ((1ull << root_bits) < (unsigned long long)nroots) ++root_bits;
   tb_status rc;
-  if ((rc = ensure_batch_buffers(s, (size_t)nroots, (size_t)ngroups))) return rc;
+  if ((rc = ensure_batch_buffers(s, (size_t)nimages, (size_t)nroots, (size_t)ngroups))) return rc;
   DevParams P = s->P;
   const size_t img = (size_t)2 * P.vpad;
-  // root images in the slot layout; a root with an empty referenced variable fails before any search, as tb_solve's
-  // does: its subproblems are skipped, and its group goes on with its other roots
-  std::vector<int> images((size_t)nroots * img, 0);
+  // box images in the slot layout; a box with an empty referenced variable fails before any search, as tb_solve's
+  // root does: the subproblems of its roots are skipped, and their groups go on with their other roots
+  std::vector<int> images((size_t)nimages * img, 0);
+  std::vector<char> empty((size_t)nimages, 0);
+  for (size_t r = 0; r < (size_t)nimages; ++r) {
+    int* im = images.data() + r * img;
+    for (size_t v = 0; v < nv; ++v) {
+      const int l = box_lb[r * nv + v], u = box_ub[r * nv + v];
+      im[img_lb(s, (int)v)] = l; im[img_ub(s, (int)v)] = u;
+      if (l > u && s->layout.referenced[v]) empty[r] = 1;
+    }
+  }
   std::vector<BatchRoot> state((size_t)nroots);
   for (size_t r = 0; r < (size_t)nroots; ++r) {
-    int* im = images.data() + r * img;
     BatchRoot& b = state[r];
     memset(&b, 0, sizeof(b));
     b.group = group_of[r];
-    for (size_t v = 0; v < nv; ++v) {
-      const int l = root_lb[r * nv + v], u = root_ub[r * nv + v];
-      im[img_lb(s, (int)v)] = l; im[img_ub(s, (int)v)] = u;
-      if (l > u && s->layout.referenced[v]) b.skip = 1;
-    }
+    b.image = image_of[r];
+    b.skip = empty[(size_t)b.image];
   }
   std::vector<BatchGroup> groups((size_t)ngroups);
-  for (BatchGroup& g : groups) {
-    memset(&g, 0, sizeof(g));
-    g.bound = ~0ull;                                   // epoch 0, no incumbent (as the cell at tb_create)
-    g.img_bound = TBD_PINF;
+  for (size_t g = 0; g < (size_t)ngroups; ++g) {
+    BatchGroup& G = groups[g];
+    memset(&G, 0, sizeof(G));
+    G.bound = ~0ull;                                   // epoch 0, no incumbent (as the cell at tb_create)
+    G.img_bound = TBD_PINF;
+    G.obj = obj_of[g] >= 0 ? s->layout.slot_of[obj_of[g]] : -1;
+    G.maximize = maximize[g];
   }
   CU(cudaMemcpyAsync(s->d_batch_roots, images.data(), images.size() * sizeof(int), cudaMemcpyHostToDevice, s->stream));
   CU(cudaMemcpyAsync(s->d_batch_state, state.data(), state.size() * sizeof(BatchRoot), cudaMemcpyHostToDevice, s->stream));
   CU(cudaMemcpyAsync(s->d_batch_groups, groups.data(), groups.size() * sizeof(BatchGroup), cudaMemcpyHostToDevice, s->stream));
   P.batch_roots = s->d_batch_roots; P.batch_best = s->d_batch_best; P.batch_state = s->d_batch_state;
   P.batch_groups = s->d_batch_groups;
+  P.batch_share = objectives && ngroups > 1 ? ngroups : 0;   // (one objective has nobody to share with)
   P.subproblems_power = d;
   P.num_subproblems = (unsigned long long)nroots << d;
   P.batch_max_depth = std::min(TB_BATCH_WEIGHT_BITS, 64 - root_bits);
@@ -2735,13 +2825,23 @@ static tb_status solve_groups(tb_solver* s, const char* fn, int32_t nroots, cons
   std::vector<int32_t> lb(std::max<size_t>(1, nv)), ub(std::max<size_t>(1, nv));
   for (size_t g = 0; g < (size_t)ngroups; ++g) {
     const bool has = groups[g].has != 0;
+    const int x = obj_of[g];
+    if (has) {
+      unpack_store(s, best.data() + g * img, lb.data(), ub.data());
+      // the value is lb(x) of the best store when minimising, ub(x) when maximising; tb_solve_objectives returns the
+      // point's side: x fixed to that value (a sub-box of an entailed box is entailed)
+      if (objectives) {
+        const int val = maximize[g] ? ub[(size_t)x] : lb[(size_t)x];
+        lb[(size_t)x] = ub[(size_t)x] = val;
+        if (val == (maximize[g] ? TB_POS_INF : TB_NEG_INF)) exh[g] = 0;     // unbounded: the objective ended there
+      }
+    }
     all_exhaustive &= exh[g];
     if (has_solution) has_solution[g] = has;
     if (exhaustive) exhaustive[g] = exh[g];
     if (objective) objective[g] = TB_POS_INF;
     if (!has) continue;
-    unpack_store(s, best.data() + g * img, lb.data(), ub.data());
-    if (objective && s->root_obj_var >= 0) objective[g] = lb[(size_t)s->root_obj_var];
+    if (objective && x >= 0) objective[g] = maximize[g] ? ub[(size_t)x] : lb[(size_t)x];
     if (best_lb && nv) memcpy(best_lb + g * nv, lb.data(), nv * 4);
     if (best_ub && nv) memcpy(best_ub + g * nv, ub.data(), nv * 4);
   }
@@ -2752,21 +2852,71 @@ static tb_status solve_groups(tb_solver* s, const char* fn, int32_t nroots, cons
   return rc;
 }
 
+// tb_solve_groups and tb_solve_batch: one root per box, every group optimises the problem's objective
+static tb_status solve_boxes(tb_solver* s, const char* fn, int32_t nroots, const int32_t* root_lb, const int32_t* root_ub,
+                             const int32_t* group_of, int32_t ngroups, volatile int32_t* stop_flag, int32_t* best_lb,
+                             int32_t* best_ub, int32_t* has_solution, int32_t* exhaustive, int32_t* objective,
+                             tb_stats* stats) try {
+  std::vector<int32_t> own((size_t)std::max(0, nroots));
+  for (size_t r = 0; r < own.size(); ++r) own[r] = (int32_t)r;
+  const int32_t obj = s ? s->root_obj_var : -1;
+  std::vector<int32_t> obj_of((size_t)std::max(0, ngroups), obj), minimize((size_t)std::max(0, ngroups), 0);
+  return solve_groups(s, fn, nroots, root_lb, root_ub, nroots, own.data(), group_of ? group_of : own.data(), ngroups,
+                      obj_of.data(), minimize.data(), false, stop_flag, best_lb, best_ub, has_solution, exhaustive,
+                      objective, stats);
+} catch (const std::bad_alloc&) {             // (the per-root host arrays: nothing may unwind through the C ABI)
+  set_error(std::string(fn) + ": out of host memory for the roots");
+  return TB_ERR_NOMEM;
+}
+
 extern "C" tb_status tb_solve_groups(tb_solver* s, int32_t nroots, const int32_t* root_lb, const int32_t* root_ub,
                                      const int32_t* group_of, int32_t ngroups, volatile int32_t* stop_flag,
                                      int32_t* best_lb, int32_t* best_ub, int32_t* has_solution, int32_t* exhaustive,
                                      int32_t* objective, tb_stats* stats) {
-  return solve_groups(s, "tb_solve_groups", nroots, root_lb, root_ub, group_of, ngroups, stop_flag, best_lb, best_ub,
-                      has_solution, exhaustive, objective, stats);
+  if (!group_of) { set_error("tb_solve_groups: needs nroots >= 1, ngroups >= 1, root_lb / root_ub and group_of"); return TB_ERR_INVALID; }
+  return solve_boxes(s, "tb_solve_groups", nroots, root_lb, root_ub, group_of, ngroups, stop_flag, best_lb, best_ub,
+                     has_solution, exhaustive, objective, stats);
 }
 
 extern "C" tb_status tb_solve_batch(tb_solver* s, int32_t nroots, const int32_t* root_lb, const int32_t* root_ub,
                                     volatile int32_t* stop_flag, int32_t* best_lb, int32_t* best_ub,
                                     int32_t* has_solution, int32_t* exhaustive, int32_t* objective, tb_stats* stats) {
-  std::vector<int32_t> own((size_t)std::max(0, nroots));
-  for (size_t r = 0; r < own.size(); ++r) own[r] = (int32_t)r;
-  return solve_groups(s, "tb_solve_batch", nroots, root_lb, root_ub, own.data(), nroots, stop_flag, best_lb, best_ub,
-                      has_solution, exhaustive, objective, stats);
+  return solve_boxes(s, "tb_solve_batch", nroots, root_lb, root_ub, nullptr, nroots, stop_flag, best_lb, best_ub,
+                     has_solution, exhaustive, objective, stats);
+}
+
+extern "C" tb_status tb_solve_objectives(tb_solver* s, int32_t nboxes, const int32_t* box_lb, const int32_t* box_ub,
+                                         int32_t nobj, const int32_t* obj_var, const int32_t* maximize,
+                                         volatile int32_t* stop_flag, int32_t* best_lb, int32_t* best_ub,
+                                         int32_t* has_solution, int32_t* exhaustive, int32_t* objective, tb_stats* stats) {
+  const std::string name("tb_solve_objectives");
+  if (!s || nboxes < 1 || nobj < 1 || !obj_var || !maximize) {
+    set_error(name + ": needs nboxes >= 1, nobj >= 1, obj_var and maximize"); return TB_ERR_INVALID;
+  }
+  for (int32_t m = 0; m < nobj; ++m) {
+    if (obj_var[m] < 0 || obj_var[m] >= s->nvars) {
+      set_error(name + ": objective " + std::to_string(m) + " names variable " + std::to_string(obj_var[m]) + ", outside [0, nvars)");
+      return TB_ERR_INVALID;
+    }
+    if (maximize[m] != 0 && maximize[m] != 1) {
+      set_error(name + ": maximize[" + std::to_string(m) + "] is neither 0 nor 1"); return TB_ERR_INVALID;
+    }
+  }
+  const long long nroots = (long long)nobj * nboxes;
+  if ((unsigned long long)nroots > (1ull << TB_K_BITS)) {     // (before the per-root arrays are allocated)
+    set_error(name + ": nobj * nboxes = " + std::to_string(nroots) + " roots do not fit the subproblem index (at most 2^40)");
+    return TB_ERR_INVALID;
+  }
+  // objective m is group m; its root m * nboxes + r searches box r
+  try {
+    std::vector<int32_t> image_of((size_t)nroots), group_of((size_t)nroots);
+    for (size_t i = 0; i < (size_t)nroots; ++i) { image_of[i] = (int32_t)(i % (size_t)nboxes); group_of[i] = (int32_t)(i / (size_t)nboxes); }
+    return solve_groups(s, "tb_solve_objectives", nboxes, box_lb, box_ub, nroots, image_of.data(), group_of.data(), nobj,
+                        obj_var, maximize, true, stop_flag, best_lb, best_ub, has_solution, exhaustive, objective, stats);
+  } catch (const std::bad_alloc&) {           // (the per-root host arrays: nothing may unwind through the C ABI)
+    set_error(name + ": out of host memory for " + std::to_string(nroots) + " roots");
+    return TB_ERR_NOMEM;
+  }
 }
 
 // ---- final gather across processes (SURVEY §8e; reduce_blocks, barebones :1033-1067, across GPUs) -------------------

@@ -71,27 +71,33 @@ struct SplitEntry {
 static_assert(sizeof(SplitEntry) == 32, "TB_CELL_BLOCK_BYTES counts 32 bytes per pool entry");
 #define TB_SPLIT_CAP 16384
 
-// tb_solve_groups / tb_solve_batch: what the grid shares about one root of the batch and about one group of roots
-// (both written by the host before each launch). Subproblem index g = (r << d) | local; a task of depth D belongs to
-// root g >> D, and root r to group BatchRoot::group. A group is solved over the union of its roots' boxes: the roots
-// share its incumbent, its stop word and its best store. tb_solve_batch puts every root in a group of its own.
+// tb_solve_groups / tb_solve_batch / tb_solve_objectives: what the grid shares about one root of the batch and about
+// one group of roots (both written by the host before each launch). Subproblem index g = (r << d) | local; a task of
+// depth D belongs to root g >> D, root r searches the box of image BatchRoot::image for group BatchRoot::group. A group
+// is solved over the union of its roots' boxes: the roots share its incumbent, its stop word and its best store.
+// tb_solve_batch puts every root in a group of its own; tb_solve_objectives makes objective m group m, with one root
+// per box (root m * nboxes + r reads image r).
 struct BatchRoot {
   unsigned long long closed;    // weight of the root's search space closed: 2^(56 - D) per task of depth D searched to
                                 // the end, 2^(56 - D + rem) per dive leaf at remaining depth rem; 2^56 = everything
   int cut;                      // a block was cut (stop, cutnodes, depth) while searching it, or stop was raised
   int skip;                     // a referenced domain is empty at the root: decided on the host, its subproblems skipped
   int group;                    // the group the root belongs to
-  int pad_;
+  int image;                    // the root's box: image `image` of batch_roots (several roots may share one)
 };
 static_assert(sizeof(BatchRoot) == 24, "host and device agree on BatchRoot");
+// The incumbent is an epoch-tagged MINIMUM of the group's key: lb(obj) when it minimises, ~ub(obj) = -ub(obj) - 1 when
+// it maximises (+oo maps to the -oo key, "unbounded", and -oo to the +oo key, "none").
 struct BatchGroup {
   unsigned long long bound;     // the group's incumbent, the TB_CELL_BOUND word (epoch-tagged, unsigned atomicMin)
   int stop;                     // the group is over (first solution of a satisfaction problem, unbounded objective)
   int lock;                     // one writer of the group's best image at a time
   int has;                      // the best image holds a solution
-  int img_bound;                // objective of the best image (TBD_PINF = none)
+  int img_bound;                // key of the best image (TBD_PINF = none)
+  int obj;                      // slot of the group's objective variable (-1 = satisfaction)
+  int maximize;                 // 1: the group maximises obj
 };
-static_assert(sizeof(BatchGroup) == 24, "host and device agree on BatchGroup");
+static_assert(sizeof(BatchGroup) == 32, "host and device agree on BatchGroup");
 #define TB_BATCH_WEIGHT_BITS 56
 
 // words of the split control block (unsigned), which lives in the cell block (TB_CELL_SPLIT) so that the peers see it
@@ -154,11 +160,12 @@ struct DevParams {
   int act_off;                           // byte offset of the active-set area in dynamic shared memory
   int act_fpw;                           // chunk flags per warp (multiple of 32): chunk ch is flag (ch / nwarps) of warp (ch % nwarps)
   // tb_solve_groups (read by the BATCH kernels only): num_subproblems = nroots << subproblems_power
-  const int* batch_roots;                // [nroots][2 * vpad] root images, layout of a block store
+  const int* batch_roots;                // [nimages][2 * vpad] root images, layout of a block store
   int* batch_best;                       // [ngroups][2 * vpad] best store of each group
   BatchRoot* batch_state;                // [nroots]
   int batch_max_depth;                   // deepest task: root bits + depth fit the 64-bit index, at most 56
-  int pad6_;
+  int batch_share;                       // tb_solve_objectives: ngroups, every solution is a witness for all of them;
+                                         // 0 = a solution counts for its own group only
   BatchGroup* batch_groups;              // [ngroups]
   unsigned long long pad8_;              // the size stays a multiple of 16: the kernel arguments behind DevParams keep
                                          // their alignment, so their loads keep their width

@@ -41,6 +41,8 @@ def lib():
         L.tb_solve_batch.argtypes = [vp, C.c_int32, i32p, i32p, i32p, i32p, i32p, i32p, i32p, i32p, C.POINTER(abi.TbStats)]
         L.tb_solve_groups.argtypes = [vp, C.c_int32, i32p, i32p, i32p, C.c_int32, i32p, i32p, i32p, i32p, i32p, i32p,
                                       C.POINTER(abi.TbStats)]
+        L.tb_solve_objectives.argtypes = [vp, C.c_int32, i32p, i32p, C.c_int32, i32p, i32p, i32p, i32p, i32p, i32p, i32p,
+                                          i32p, C.POINTER(abi.TbStats)]
         L.tb_link_peers.argtypes = [C.POINTER(vp), C.c_int32]
         L.tb_export_bound_handle.argtypes = [vp, vp]
         L.tb_import_peer_bounds.argtypes = [vp, vp, C.c_int32]
@@ -55,7 +57,7 @@ def lib():
         L.tb_version.restype = C.c_char_p
         L.tb_device_count.restype = C.c_int32
         for name in ("tb_create", "tb_propagate", "tb_propagate_batch", "tb_dive", "tb_dive_batch", "tb_solve",
-                     "tb_solve_batch", "tb_solve_groups", "tb_link_peers", "tb_export_bound_handle", "tb_import_peer_bounds", "tb_read_bound",
+                     "tb_solve_batch", "tb_solve_groups", "tb_solve_objectives", "tb_link_peers", "tb_export_bound_handle", "tb_import_peer_bounds", "tb_read_bound",
                      "tb_get_config"):
             getattr(L, name).restype = C.c_int
         _LIB = L
@@ -282,6 +284,54 @@ class Solver:
         g = max(0, ngroups)
         return dict(lb=olb[:g, :n], ub=oub[:g, :n], has_solution=has[:g].astype(bool), exhaustive=exh[:g].astype(bool),
                     objective=obj[:g].astype(np.int64), stats=st.as_dict())
+
+    def solve_objectives(self, lb, ub, obj_vars, maximize, stop_flag=None):
+        """tb_solve_objectives: this solver's network over the union of K boxes ([K, nvars] int32, each a narrowing of
+        the problem's), optimised for every objective m in one launch: variable obj_vars[m], maximised where
+        maximize[m] is true, minimised elsewhere. Every solution found is a witness for every objective. Returns arrays
+        of length nobj, shaped as solve_groups's: `objective` is the optimum in the objective's own sense (abi.POS_INF
+        without a solution), and row m of lb / ub is a solution with obj_vars[m] fixed to it. The problem's own
+        objective plays no part; narrow its upper bound in the boxes to keep to (near-)optimal solutions."""
+        n = self.problem.nvars
+        lb = np.ascontiguousarray(lb, dtype=np.int32).reshape(-1, n)
+        ub = np.ascontiguousarray(ub, dtype=np.int32).reshape(-1, n)
+        if lb.shape != ub.shape:
+            raise ValueError("lb and ub must have the same shape [K, nvars]")
+        obj_vars = np.ascontiguousarray(obj_vars, dtype=np.int32).reshape(-1)
+        maximize = np.ascontiguousarray(maximize, dtype=np.int32).reshape(-1)
+        if maximize.shape != obj_vars.shape:
+            raise ValueError("maximize must have one entry per objective")
+        m = obj_vars.shape[0]
+        olb = np.zeros((max(1, m), max(1, n)), np.int32)
+        oub = np.zeros((max(1, m), max(1, n)), np.int32)
+        has = np.zeros(max(1, m), np.int32)
+        exh = np.zeros(max(1, m), np.int32)
+        obj = np.zeros(max(1, m), np.int32)
+        st = abi.TbStats()
+        _check(lib().tb_solve_objectives(self._h, lb.shape[0], _p(lb), _p(ub), m, _p(obj_vars), _p(maximize), stop_flag,
+                                         _p(olb), _p(oub), _p(has), _p(exh), _p(obj), C.byref(st)))
+        return dict(lb=olb[:m, :n], ub=oub[:m, :n], has_solution=has[:m].astype(bool), exhaustive=exh[:m].astype(bool),
+                    objective=obj[:m].astype(np.int64), stats=st.as_dict())
+
+    def hull(self, vars=None, lb=None, ub=None, stop_flag=None):
+        """The solution hull: for each variable of `vars` (default: every variable), the smallest and the largest
+        value it takes in a solution of the network over the union of the boxes lb / ub ([K, nvars] or [nvars];
+        default: the problem's root), as one solve_objectives call of a minimisation and a maximisation per variable.
+        Returns `lb` / `ub` per variable, `exact_lb` / `exact_ub` (that side was proven: its objective was searched to
+        its end; otherwise the value is a witnessed one, inside the hull), `has_solution` and the stats. Without a
+        solution the hull is empty: lb = abi.POS_INF and ub = abi.NEG_INF."""
+        vs = np.arange(self.problem.nvars, dtype=np.int32) if vars is None else np.asarray(vars, np.int32).reshape(-1)
+        lb = self.problem.lb if lb is None else lb
+        ub = self.problem.ub if ub is None else ub
+        k = vs.shape[0]
+        r = self.solve_objectives(lb, ub, np.concatenate([vs, vs]),
+                                  np.concatenate([np.zeros(k, np.int32), np.ones(k, np.int32)]), stop_flag)
+        has = bool(r["has_solution"].any())
+        lo, hi = r["objective"][:k].copy(), r["objective"][k:].copy()
+        if not has:
+            lo[:], hi[:] = abi.POS_INF, abi.NEG_INF
+        return dict(vars=vs, lb=lo, ub=hi, exact_lb=r["exhaustive"][:k].copy(), exact_ub=r["exhaustive"][k:].copy(),
+                    has_solution=has, stats=r["stats"])
 
     def export_bound_handle(self):
         buf = C.create_string_buffer(64)
