@@ -228,6 +228,33 @@ tb_status tb_solve_objectives(tb_solver*, int32_t nboxes, const int32_t* box_lb,
                               volatile int32_t* stop_flag, int32_t* best_lb, int32_t* best_ub,
                               int32_t* has_solution, int32_t* exhaustive, int32_t* objective, tb_stats* stats);
 
+/* The solution domains of a model, in one launch: query i asks whether some solution of the network over the union of
+ * nboxes boxes (box_lb / box_ub laid out [nboxes][nvars], each a narrowing of the solver's root, as in
+ * tb_solve_objectives) has q_var[i] = q_val[i]. This is the set of supported values of a variable, which the hull
+ * cannot give: x in [1, 9] in the hull says nothing about x = 5. Every query is a satisfaction question; the problem's
+ * own obj_var plays no part (to ask about (near-)optimal solutions, narrow its upper bound in the boxes). All the
+ * queries share the union, so every solution found supports every query whose value it holds, and ends it.
+ * supported [nq]: 1 = a solution was found; 0 = proven that none exists (every (query, box) root was searched to its end
+ * and no block was cut while doing so, or was decided on the host); -1 = unknown (stop_flag, the timeout, cutnodes, a
+ * depth overflow, a node with nothing to branch on). Duplicate queries are legal and get the same answer. A query
+ * whose value lies outside a box's domain of q_var, or a box with an empty referenced domain, is decided on the host for
+ * that box (no solution, searched). Witnesses: solutions go to a pool of wit_cap rows, wit_lb / wit_ub
+ * [wit_cap][nvars], each a solution (entailed) store; *nwit (may be NULL) = rows written. witness [nq] (may be NULL):
+ * for a supported query the row w that holds q_val[i] in the domain of q_var[i] - fixing that variable to the value and
+ * taking the lower bounds gives a solution point, as for tb_solve_objectives's rows - or -1: no row (the pool was full,
+ * or the query is not supported). Rows of different queries may coincide. wit_cap = 0: answers only. Device memory
+ * grows with the pool, not with the queries: one store image per row, none per query.
+ * stop_flag, the timeout and the subproblems per root apply as in tb_solve_groups, with (distinct queries) * nboxes
+ * roots. TB_ERR_INVALID: nboxes < 1, nq < 1, a q_var outside [0, nvars), a q_val equal to TB_NEG_INF or TB_POS_INF, a
+ * widening box, nq * nboxes above 2^40 (the subproblem index), wit_cap < 0, wit_cap > 0 without wit_lb / wit_ub.
+ * TB_ERR_NOMEM: no host memory for the roots. TB_ERR_UNSUPPORTED: as tb_solve_batch. */
+tb_status tb_solve_supports(tb_solver*, int32_t nboxes, const int32_t* box_lb, const int32_t* box_ub,
+                            int32_t nq, const int32_t* q_var, const int32_t* q_val,
+                            volatile int32_t* stop_flag,
+                            int32_t* supported, int32_t* witness,
+                            int32_t wit_cap, int32_t* wit_lb, int32_t* wit_ub, int32_t* nwit,
+                            tb_stats* stats);
+
 /* Intermediate solutions (-i / -a; the reference's consumer thread, gpu_dive_and_solve.hpp:100-132; its barebones
  * architecture cannot, barebones_dive_and_solve.hpp:465-467).  tb_stream_solutions (before tb_solve) makes every
  * improving solution also land in a ring of `slots` store images; tb_poll_solution, called from ANOTHER host thread

@@ -302,8 +302,9 @@ __device__ __forceinline__ int chunk_class(const DevParams& P, int ch) {
 
 // Per-CTA state of the BATCH kernels only (a function-scope __shared__ object: the other kernels never reference it).
 // Set by thread 0 when a task starts: `group`, the group of the task's root, its objective slot `obj` (-1 =
-// satisfaction) and sense `maximize`, and `image`, the root's box. `pick` / `key`: witness sharing (batch_share_witness).
-struct BatchCtl { int won; int group; int obj; int maximize; int image; int pick; int key; };
+// satisfaction) and sense `maximize`, `image`, the root's box, and the group's fixing `fix` = `fix_val` (-1 = none).
+// `pick` / `key`: witness sharing (batch_share_witness, batch_support_witness).
+struct BatchCtl { int won; int group; int obj; int maximize; int image; int pick; int key; int fix; int fix_val; };
 __device__ __forceinline__ BatchCtl& batch_ctl() { __shared__ BatchCtl b; return b; }
 
 // The incumbent's key of a solution's objective domain [l, u]: l when minimising, ~u = -u - 1 when maximising. The
@@ -1034,6 +1035,60 @@ struct Ctx {
     }
   }
 
+  // ---- tb_solve_supports: a solution is a witness for every query value it holds ----------------------------------
+  // Every group asks whether some solution of the union has one slot at one value, so a solution store supports every
+  // query (slot, v) with v in the store's [l, u] of that slot (an entailed box: any value of it extends to a point). The
+  // threads split the queried slots; for each, a binary search finds the first value >= l and the walk goes up to u. A
+  // group that is still open is won with a CAS on its stop word: it is supported, and its blocks leave at their next
+  // node. A block that won something takes one row of the pool, writes its store there once and names that row as the
+  // witness of every group it won: the winner marks each won group with -2 - slot in the first walk and replaces the
+  // mark by the row (or -1, the pool being full) in the second. Nobody else writes a won group's `wit`, and the store
+  // does not change between the walks, so both walks meet the same groups. The task's own group is one of the queries.
+  // Returns (uniformly) whether the block won a group.
+  __device__ __forceinline__ bool batch_support_witness() {
+    BatchCtl& b = batch_ctl();
+    const int mark = -2 - slot;
+    if (!__syncthreads_or(support_walk(mark, 0, true))) return false;
+    if (tid == 0) {
+      const unsigned r = atomicAdd(P.batch_wit_n, 1u);
+      b.pick = r < (unsigned)P.batch_wit_cap ? (int)r : -1;
+    }
+    sync();
+    const int row = b.pick;
+    if (row >= 0) {
+      save_store(P.batch_wit + (size_t)row * 2 * P.vpad, true);
+      if (threadIdx.x == 0) bulk_wait_all();
+      __threadfence();
+      sync();
+    }
+    support_walk(mark, row, false);
+    __threadfence();
+    return true;
+  }
+  // One walk of batch_support_witness over this thread's query slots: claim the open groups (returns whether it won
+  // one), or give the groups marked `mark` their witness `row`.
+  __device__ __forceinline__ bool support_walk(int mark, int row, bool claim) {
+    bool mine = false;
+    for (int q = tid; q < P.batch_nqslots; q += T) {
+      int l, u; store.ld(__ldg(P.batch_qslot + q), l, u);
+      int lo = __ldg(P.batch_qoff + q), hi = __ldg(P.batch_qoff + q + 1);
+      const int end = hi;
+      while (lo < hi) {                         // the first value >= l
+        const int m = (lo + hi) >> 1;
+        if (__ldg(P.batch_qval + m) < l) lo = m + 1; else hi = m;
+      }
+      for (int k = lo; k < end && __ldg(P.batch_qval + k) <= u; ++k) {
+        BatchGroup& g = P.batch_groups[k];
+        if (claim) {
+          if (*(volatile int*)&g.stop == 0 && atomicCAS(&g.stop, 0, 1) == 0) { *(volatile int*)&g.wit = mark; mine = true; }
+        } else if (*(volatile int*)&g.wit == mark) {
+          *(volatile int*)&g.wit = row; *(volatile int*)&g.has = 1;
+        }
+      }
+    }
+    return mine;
+  }
+
   // ---- propagate() (barebones :903-1031) -----------------------------------------------------------
   // Runs the fixpoint, classifies the node, records solutions, updates counters and the stop flag.
   // Sets c.leaf / c.failed / c.stop uniformly (valid after return).
@@ -1065,9 +1120,13 @@ struct Ctx {
         }
       } else {
         if constexpr (BATCH) {                  // satisfaction: the first solution of the GROUP wins
-          if (tid == 0) batch_ctl().won = atomicCAS(&batch_group().stop, 0, 1) == 0;
-          sync();
-          improved = batch_ctl().won != 0;
+          if (P.batch_nqslots) {                // (supports: of every group it holds; no best row is written)
+            if (batch_support_witness() && tid == 0) { st->solutions++; st->has_best = 1; }
+          } else {
+            if (tid == 0) batch_ctl().won = atomicCAS(&batch_group().stop, 0, 1) == 0;
+            sync();
+            improved = batch_ctl().won != 0;
+          }
         } else {
           improved = st->solutions == 0;          // satisfaction: first solution wins
           sync();
@@ -1264,6 +1323,7 @@ struct Ctx {
             const BatchGroup& g = P.batch_groups[r.group];
             BatchCtl& b = batch_ctl();
             b.group = r.group; b.image = r.image; b.obj = g.obj; b.maximize = g.maximize;
+            b.fix = g.fix; b.fix_val = g.fix_val;
             c.abandon = r.skip || batch_group_over();   // (nothing left to do for a root that is over)
           }
         }
@@ -1271,8 +1331,16 @@ struct Ctx {
         if (BATCH && c.abandon) mode = M_NEXT;
         else {
           for (int i = tid; i < P.nsnap; i += T) g_snap_tag[i] = -1;       // snapshots belong to one subproblem
-          if constexpr (BATCH) load_store(P.batch_roots + (size_t)batch_ctl().image * 2 * P.vpad);
-          else load_store(P.root_store);
+          if constexpr (BATCH) {
+            load_store(P.batch_roots + (size_t)batch_ctl().image * 2 * P.vpad);
+            // The group's fixing (tb_solve_supports), marked for the active set before the first propagation. This is
+            // the only place a batch root store is built: the dive starts here, g_root and the snapshots are saved
+            // from stores below it, and a tail-split child is a task that starts here again, so all of them hold it.
+            if (tid == 0 && batch_ctl().fix >= 0) {
+              store.embed(batch_ctl().fix, batch_ctl().fix_val, batch_ctl().fix_val);
+              mark_var(batch_ctl().fix);
+            }
+          } else load_store(P.root_store);
           sync();
           mode = M_DIVE;
         }
@@ -1786,11 +1854,13 @@ struct tb_solver {
   // batch buffers (grown on demand)
   int *d_in_lb = nullptr, *d_in_ub = nullptr, *d_out_lb = nullptr, *d_out_ub = nullptr, *d_out_i0 = nullptr, *d_out_i1 = nullptr;
   size_t batch_cap = 0;
-  // tb_solve_groups buffers (grown on demand): root images, BatchRoot cells, best images and BatchGroup cells
-  int *d_batch_roots = nullptr, *d_batch_best = nullptr;
+  // tb_solve_groups buffers (grown on demand): root images, BatchRoot cells, best images and BatchGroup cells; for
+  // tb_solve_supports the query table (the pool's row counter, then the CSR) and the witness pool
+  int *d_batch_roots = nullptr, *d_batch_best = nullptr, *d_batch_query = nullptr, *d_batch_wit = nullptr;
   BatchRoot* d_batch_state = nullptr;
   BatchGroup* d_batch_groups = nullptr;
-  size_t batch_images_cap = 0, batch_roots_cap = 0, batch_groups_cap = 0;
+  size_t batch_images_cap = 0, batch_roots_cap = 0, batch_groups_cap = 0, batch_best_cap = 0, batch_query_cap = 0,
+         batch_wit_cap = 0;
   int32_t* h_pinned_one = nullptr;
 };
 
@@ -2665,7 +2735,8 @@ extern "C" tb_status tb_solve(tb_solver* s, volatile int32_t* stop_flag, int32_t
   return rc;
 }
 
-static tb_status ensure_batch_buffers(tb_solver* s, size_t nimages, size_t nroots, size_t ngroups) {
+static tb_status ensure_batch_buffers(tb_solver* s, size_t nimages, size_t nroots, size_t ngroups, size_t nbest,
+                                      size_t nquery, size_t nwit) {
   tb_status rc;
   const size_t img = (size_t)2 * s->P.vpad;
   if (nimages > s->batch_images_cap) {
@@ -2677,23 +2748,50 @@ static tb_status ensure_batch_buffers(tb_solver* s, size_t nimages, size_t nroot
     s->batch_roots_cap = nroots;
   }
   if (ngroups > s->batch_groups_cap) {
-    if ((rc = dev_alloc(s, &s->d_batch_best, ngroups * img))) return rc;
     if ((rc = dev_alloc(s, &s->d_batch_groups, ngroups))) return rc;
     s->batch_groups_cap = ngroups;
+  }
+  if (nbest > s->batch_best_cap) {
+    if ((rc = dev_alloc(s, &s->d_batch_best, nbest * img))) return rc;
+    s->batch_best_cap = nbest;
+  }
+  if (nquery > s->batch_query_cap) {
+    if ((rc = dev_alloc(s, &s->d_batch_query, nquery))) return rc;
+    s->batch_query_cap = nquery;
+  }
+  if (nwit > s->batch_wit_cap) {
+    if ((rc = dev_alloc(s, &s->d_batch_wit, nwit * img))) return rc;
+    s->batch_wit_cap = nwit;
   }
   return TB_OK;
 }
 
-// The one host path of the BATCH kernel: tb_solve_groups, tb_solve_batch and tb_solve_objectives. `nimages` boxes
-// (box_lb / box_ub [nimages][nvars]); root r searches box image_of[r] for group group_of[r] (nroots entries); group g
-// optimises variable obj_of[g] (-1 = satisfaction) in the sense maximize[g] (ngroups entries). `objectives`
-// (tb_solve_objectives): every solution is a witness for every group, each returned row has the group's objective
-// variable fixed to its value, and an unbounded objective is never exhaustive. `fn` names the entry point in errors.
+// tb_solve_supports's part of solve_groups. Group g fixes variable fix_var[g] to fix_val[g] in every root; the groups
+// are sorted by (slot, value), so fix_val is the value list of the CSR over the queried slots qslot / qoff. Solutions
+// go to a pool of wit_cap rows (*nwit of them written, wit_lb / wit_ub [wit_cap][nvars]); wit_of [ngroups] receives
+// each group's row (-1 = none).
+struct SupportQueries {
+  const int32_t* fix_var;
+  const int32_t* fix_val;
+  std::vector<int32_t> qslot, qoff;
+  int32_t wit_cap;
+  int32_t *wit_lb, *wit_ub, *nwit, *wit_of;
+};
+
+// The one host path of the BATCH kernel: tb_solve_groups, tb_solve_batch, tb_solve_objectives and tb_solve_supports.
+// `nimages` boxes (box_lb / box_ub [nimages][nvars]); root r searches box image_of[r] for group group_of[r] (nroots
+// entries); group g optimises variable obj_of[g] (-1 = satisfaction) in the sense maximize[g] (ngroups entries).
+// `objectives` (tb_solve_objectives): every solution is a witness for every group, each returned row has the group's
+// objective variable fixed to its value, and an unbounded objective is never exhaustive. `sup` (tb_solve_supports):
+// every group is a satisfaction group with one variable fixed, every solution is a witness for every group it holds,
+// and there are no best rows (best_lb / best_ub / objective are NULL), only the witness pool. `fn` names the entry
+// point in errors.
 static tb_status solve_groups(tb_solver* s, const char* fn, int32_t nimages, const int32_t* box_lb, const int32_t* box_ub,
                               long long nroots, const int32_t* image_of, const int32_t* group_of, int32_t ngroups,
                               const int32_t* obj_of, const int32_t* maximize, bool objectives,
-                              volatile int32_t* stop_flag, int32_t* best_lb, int32_t* best_ub, int32_t* has_solution,
-                              int32_t* exhaustive, int32_t* objective, tb_stats* stats) {
+                              const SupportQueries* sup, volatile int32_t* stop_flag, int32_t* best_lb,
+                              int32_t* best_ub, int32_t* has_solution, int32_t* exhaustive, int32_t* objective,
+                              tb_stats* stats) {
   const std::string name(fn);
   if (!s || nimages < 1 || nroots < 1 || ngroups < 1 || !group_of || (s->nvars && (!box_lb || !box_ub))) {
     set_error(name + ": needs nroots >= 1, ngroups >= 1, root_lb / root_ub and group_of"); return TB_ERR_INVALID;
@@ -2738,7 +2836,11 @@ static tb_status solve_groups(tb_solver* s, const char* fn, int32_t nimages, con
   int root_bits = 0;
   while ((1ull << root_bits) < (unsigned long long)nroots) ++root_bits;
   tb_status rc;
-  if ((rc = ensure_batch_buffers(s, (size_t)nimages, (size_t)nroots, (size_t)ngroups))) return rc;
+  // (tb_solve_supports: no best row per group - the groups may be many more than the solutions - only the pool)
+  const size_t nqslots = sup ? sup->qslot.size() : 0;
+  const size_t nquery = sup ? 1 + nqslots + (nqslots + 1) + (size_t)ngroups : 0;
+  if ((rc = ensure_batch_buffers(s, (size_t)nimages, (size_t)nroots, (size_t)ngroups, sup ? 0 : (size_t)ngroups, nquery,
+                                 sup ? (size_t)sup->wit_cap : 0))) return rc;
   DevParams P = s->P;
   const size_t img = (size_t)2 * P.vpad;
   // box images in the slot layout; a box with an empty referenced variable fails before any search, as tb_solve's
@@ -2760,6 +2862,11 @@ static tb_status solve_groups(tb_solver* s, const char* fn, int32_t nimages, con
     b.group = group_of[r];
     b.image = image_of[r];
     b.skip = empty[(size_t)b.image];
+    if (sup) {                                         // (a fixing outside the box: decided on the host, as empty)
+      const size_t at = (size_t)b.image * nv + (size_t)sup->fix_var[b.group];
+      const int v = sup->fix_val[b.group];
+      b.skip |= v < box_lb[at] || v > box_ub[at];
+    }
   }
   std::vector<BatchGroup> groups((size_t)ngroups);
   for (size_t g = 0; g < (size_t)ngroups; ++g) {
@@ -2769,6 +2876,9 @@ static tb_status solve_groups(tb_solver* s, const char* fn, int32_t nimages, con
     G.img_bound = TBD_PINF;
     G.obj = obj_of[g] >= 0 ? s->layout.slot_of[obj_of[g]] : -1;
     G.maximize = maximize[g];
+    G.fix = sup ? s->layout.slot_of[sup->fix_var[g]] : -1;
+    G.fix_val = sup ? sup->fix_val[g] : 0;
+    G.wit = -1;
   }
   CU(cudaMemcpyAsync(s->d_batch_roots, images.data(), images.size() * sizeof(int), cudaMemcpyHostToDevice, s->stream));
   CU(cudaMemcpyAsync(s->d_batch_state, state.data(), state.size() * sizeof(BatchRoot), cudaMemcpyHostToDevice, s->stream));
@@ -2776,6 +2886,22 @@ static tb_status solve_groups(tb_solver* s, const char* fn, int32_t nimages, con
   P.batch_roots = s->d_batch_roots; P.batch_best = s->d_batch_best; P.batch_state = s->d_batch_state;
   P.batch_groups = s->d_batch_groups;
   P.batch_share = objectives && ngroups > 1 ? ngroups : 0;   // (one objective has nobody to share with)
+  P.batch_nqslots = (int)nqslots;
+  if (sup) {
+    // the query table: the pool's row counter (0), then qslot, qoff and the values
+    std::vector<int32_t> q(nquery, 0);
+    std::copy(sup->qslot.begin(), sup->qslot.end(), q.begin() + 1);
+    std::copy(sup->qoff.begin(), sup->qoff.end(), q.begin() + 1 + nqslots);
+    std::copy(sup->fix_val, sup->fix_val + ngroups, q.begin() + 1 + 2 * nqslots + 1);
+    CU(cudaMemcpyAsync(s->d_batch_query, q.data(), q.size() * sizeof(int32_t), cudaMemcpyHostToDevice, s->stream));
+    P.batch_wit_n = (unsigned*)s->d_batch_query;
+    P.batch_qslot = s->d_batch_query + 1;
+    P.batch_qoff = P.batch_qslot + nqslots;
+    P.batch_qval = P.batch_qoff + nqslots + 1;
+    P.batch_wit = s->d_batch_wit;
+    P.batch_wit_cap = sup->wit_cap;
+    P.batch_best = nullptr;
+  }
   P.subproblems_power = d;
   P.num_subproblems = (unsigned long long)nroots << d;
   P.batch_max_depth = std::min(TB_BATCH_WEIGHT_BITS, 64 - root_bits);
@@ -2805,7 +2931,7 @@ static tb_status solve_groups(tb_solver* s, const char* fn, int32_t nimages, con
   CU(cudaMemcpy(state.data(), s->d_batch_state, state.size() * sizeof(BatchRoot), cudaMemcpyDeviceToHost));
   CU(cudaMemcpy(groups.data(), s->d_batch_groups, groups.size() * sizeof(BatchGroup), cudaMemcpyDeviceToHost));
   bool any = false;
-  for (auto& g : groups) any |= g.has != 0;
+  for (auto& g : groups) any |= g.has != 0 && !sup;
   std::vector<int> best(any ? (size_t)ngroups * img : 0);
   if (any) CU(cudaMemcpy(best.data(), s->d_batch_best, best.size() * sizeof(int), cudaMemcpyDeviceToHost));
   tb_stats st; memset(&st, 0, sizeof(st));
@@ -2826,7 +2952,7 @@ static tb_status solve_groups(tb_solver* s, const char* fn, int32_t nimages, con
   for (size_t g = 0; g < (size_t)ngroups; ++g) {
     const bool has = groups[g].has != 0;
     const int x = obj_of[g];
-    if (has) {
+    if (has && !sup) {
       unpack_store(s, best.data() + g * img, lb.data(), ub.data());
       // the value is lb(x) of the best store when minimising, ub(x) when maximising; tb_solve_objectives returns the
       // point's side: x fixed to that value (a sub-box of an entailed box is entailed)
@@ -2845,6 +2971,16 @@ static tb_status solve_groups(tb_solver* s, const char* fn, int32_t nimages, con
     if (best_lb && nv) memcpy(best_lb + g * nv, lb.data(), nv * 4);
     if (best_ub && nv) memcpy(best_ub + g * nv, ub.data(), nv * 4);
   }
+  if (sup) {
+    for (size_t g = 0; g < (size_t)ngroups; ++g) sup->wit_of[g] = groups[g].has && groups[g].wit >= 0 ? groups[g].wit : -1;
+    unsigned taken = 0;
+    CU(cudaMemcpy(&taken, s->d_batch_query, sizeof(unsigned), cudaMemcpyDeviceToHost));
+    const size_t rows = std::min<size_t>(taken, (size_t)sup->wit_cap);
+    std::vector<int> pool(rows * img);
+    if (rows) CU(cudaMemcpy(pool.data(), s->d_batch_wit, pool.size() * sizeof(int), cudaMemcpyDeviceToHost));
+    for (size_t w = 0; w < rows && nv; ++w) unpack_store(s, pool.data() + w * img, sup->wit_lb + w * nv, sup->wit_ub + w * nv);
+    if (sup->nwit) *sup->nwit = (int32_t)rows;
+  }
   st.exhaustive = all_exhaustive;
   st.kernel_ms = run.kernel_ms;
   st.timers_ns[TB_TIMER_OVERALL] = (int64_t)((now_ms() - t_begin) * 1e6);
@@ -2862,7 +2998,7 @@ static tb_status solve_boxes(tb_solver* s, const char* fn, int32_t nroots, const
   const int32_t obj = s ? s->root_obj_var : -1;
   std::vector<int32_t> obj_of((size_t)std::max(0, ngroups), obj), minimize((size_t)std::max(0, ngroups), 0);
   return solve_groups(s, fn, nroots, root_lb, root_ub, nroots, own.data(), group_of ? group_of : own.data(), ngroups,
-                      obj_of.data(), minimize.data(), false, stop_flag, best_lb, best_ub, has_solution, exhaustive,
+                      obj_of.data(), minimize.data(), false, nullptr, stop_flag, best_lb, best_ub, has_solution, exhaustive,
                       objective, stats);
 } catch (const std::bad_alloc&) {             // (the per-root host arrays: nothing may unwind through the C ABI)
   set_error(std::string(fn) + ": out of host memory for the roots");
@@ -2912,9 +3048,83 @@ extern "C" tb_status tb_solve_objectives(tb_solver* s, int32_t nboxes, const int
     std::vector<int32_t> image_of((size_t)nroots), group_of((size_t)nroots);
     for (size_t i = 0; i < (size_t)nroots; ++i) { image_of[i] = (int32_t)(i % (size_t)nboxes); group_of[i] = (int32_t)(i / (size_t)nboxes); }
     return solve_groups(s, "tb_solve_objectives", nboxes, box_lb, box_ub, nroots, image_of.data(), group_of.data(), nobj,
-                        obj_var, maximize, true, stop_flag, best_lb, best_ub, has_solution, exhaustive, objective, stats);
+                        obj_var, maximize, true, nullptr, stop_flag, best_lb, best_ub, has_solution, exhaustive, objective,
+                        stats);
   } catch (const std::bad_alloc&) {           // (the per-root host arrays: nothing may unwind through the C ABI)
     set_error(name + ": out of host memory for " + std::to_string(nroots) + " roots");
+    return TB_ERR_NOMEM;
+  }
+}
+
+extern "C" tb_status tb_solve_supports(tb_solver* s, int32_t nboxes, const int32_t* box_lb, const int32_t* box_ub,
+                                       int32_t nq, const int32_t* q_var, const int32_t* q_val,
+                                       volatile int32_t* stop_flag, int32_t* supported, int32_t* witness,
+                                       int32_t wit_cap, int32_t* wit_lb, int32_t* wit_ub, int32_t* nwit,
+                                       tb_stats* stats) {
+  const std::string name("tb_solve_supports");
+  if (!s || nboxes < 1 || nq < 1 || !q_var || !q_val || !supported) {
+    set_error(name + ": needs nboxes >= 1, nq >= 1, q_var, q_val and supported"); return TB_ERR_INVALID;
+  }
+  if (wit_cap < 0 || (wit_cap > 0 && (!wit_lb || !wit_ub))) {
+    set_error(name + ": needs wit_cap >= 0, and wit_lb / wit_ub when wit_cap > 0"); return TB_ERR_INVALID;
+  }
+  for (int32_t i = 0; i < nq; ++i) {
+    if (q_var[i] < 0 || q_var[i] >= s->nvars) {
+      set_error(name + ": query " + std::to_string(i) + " names variable " + std::to_string(q_var[i]) + ", outside [0, nvars)");
+      return TB_ERR_INVALID;
+    }
+    if (q_val[i] == TB_NEG_INF || q_val[i] == TB_POS_INF) {
+      set_error(name + ": query " + std::to_string(i) + " asks for an infinite value"); return TB_ERR_INVALID;
+    }
+  }
+  const long long nqroots = (long long)nq * nboxes;
+  if ((unsigned long long)nqroots > (1ull << TB_K_BITS)) {    // (before the per-root arrays are allocated)
+    set_error(name + ": nq * nboxes = " + std::to_string(nqroots) + " roots do not fit the subproblem index (at most 2^40)");
+    return TB_ERR_INVALID;
+  }
+  try {
+    // the distinct queries sorted by (slot, value): group g is the g-th of them, and its values are the CSR's
+    std::vector<int32_t> order((size_t)nq);
+    for (int32_t i = 0; i < nq; ++i) order[(size_t)i] = i;
+    auto key = [&](int32_t i) { return std::make_pair(s->layout.slot_of[q_var[i]], q_val[i]); };
+    std::sort(order.begin(), order.end(), [&](int32_t a, int32_t b) { return key(a) < key(b); });
+    std::vector<int32_t> group_of_query((size_t)nq), fix_var, fix_val;
+    SupportQueries sup;
+    for (int32_t i : order) {
+      if (fix_var.empty() || key(i) != std::make_pair(s->layout.slot_of[fix_var.back()], fix_val.back())) {
+        if (sup.qslot.empty() || sup.qslot.back() != key(i).first) {
+          sup.qslot.push_back(key(i).first);
+          sup.qoff.push_back((int32_t)fix_var.size());
+        }
+        fix_var.push_back(q_var[i]); fix_val.push_back(q_val[i]);
+      }
+      group_of_query[(size_t)i] = (int32_t)fix_var.size() - 1;
+    }
+    sup.qoff.push_back((int32_t)fix_var.size());
+    const int32_t ngroups = (int32_t)fix_var.size();
+    sup.fix_var = fix_var.data(); sup.fix_val = fix_val.data();
+    sup.wit_cap = wit_cap; sup.wit_lb = wit_lb; sup.wit_ub = wit_ub; sup.nwit = nwit;
+    std::vector<int32_t> wit_of((size_t)ngroups, -1);
+    sup.wit_of = wit_of.data();
+    // group g's root g * nboxes + r searches box r, as tb_solve_objectives's objectives do
+    const long long nroots = (long long)ngroups * nboxes;
+    std::vector<int32_t> image_of((size_t)nroots), group_of((size_t)nroots), obj_of((size_t)ngroups, -1),
+        maximize((size_t)ngroups, 0), has((size_t)ngroups), exh((size_t)ngroups);
+    for (size_t i = 0; i < (size_t)nroots; ++i) { image_of[i] = (int32_t)(i % (size_t)nboxes); group_of[i] = (int32_t)(i / (size_t)nboxes); }
+    if (nwit) *nwit = 0;
+    const tb_status rc = solve_groups(s, "tb_solve_supports", nboxes, box_lb, box_ub, nroots, image_of.data(),
+                                      group_of.data(), ngroups, obj_of.data(), maximize.data(), false, &sup, stop_flag,
+                                      nullptr, nullptr, has.data(), exh.data(), nullptr, stats);
+    if (rc != TB_OK && rc != TB_ERR_DEPTH) return rc;
+    // 1: a solution holds the value; 0: every root of the query was searched to its end uncut or decided on the host
+    for (int32_t i = 0; i < nq; ++i) {
+      const int32_t g = group_of_query[(size_t)i];
+      supported[i] = has[(size_t)g] ? 1 : exh[(size_t)g] ? 0 : -1;
+      if (witness) witness[i] = wit_of[(size_t)g];
+    }
+    return rc;
+  } catch (const std::bad_alloc&) {           // (the per-query and per-root host arrays)
+    set_error(name + ": out of host memory for " + std::to_string(nqroots) + " roots");
     return TB_ERR_NOMEM;
   }
 }

@@ -76,7 +76,8 @@ static_assert(sizeof(SplitEntry) == 32, "TB_CELL_BLOCK_BYTES counts 32 bytes per
 // depth D belongs to root g >> D, root r searches the box of image BatchRoot::image for group BatchRoot::group. A group
 // is solved over the union of its roots' boxes: the roots share its incumbent, its stop word and its best store.
 // tb_solve_batch puts every root in a group of its own; tb_solve_objectives makes objective m group m, with one root
-// per box (root m * nboxes + r reads image r).
+// per box (root m * nboxes + r reads image r); tb_solve_supports makes query g group g, a satisfaction group whose
+// roots g * nboxes + r read image r with one variable fixed (BatchGroup::fix).
 struct BatchRoot {
   unsigned long long closed;    // weight of the root's search space closed: 2^(56 - D) per task of depth D searched to
                                 // the end, 2^(56 - D + rem) per dive leaf at remaining depth rem; 2^56 = everything
@@ -96,8 +97,13 @@ struct BatchGroup {
   int img_bound;                // key of the best image (TBD_PINF = none)
   int obj;                      // slot of the group's objective variable (-1 = satisfaction)
   int maximize;                 // 1: the group maximises obj
+  int fix;                      // tb_solve_supports: slot fixed to fix_val in every root of the group (-1 = none)
+  int fix_val;
+  int wit;                      // tb_solve_supports: the witness row of the group (-1 = none; -2 - b while block b
+                                // that won the group takes its row)
+  int pad_;
 };
-static_assert(sizeof(BatchGroup) == 32, "host and device agree on BatchGroup");
+static_assert(sizeof(BatchGroup) == 48, "host and device agree on BatchGroup");
 #define TB_BATCH_WEIGHT_BITS 56
 
 // words of the split control block (unsigned), which lives in the cell block (TB_CELL_SPLIT) so that the peers see it
@@ -167,6 +173,14 @@ struct DevParams {
   int batch_share;                       // tb_solve_objectives: ngroups, every solution is a witness for all of them;
                                          // 0 = a solution counts for its own group only
   BatchGroup* batch_groups;              // [ngroups]
+  // tb_solve_supports: the queries as a CSR over the queried slots, values ascending per slot; the query at position k
+  // of batch_qval is group k. batch_nqslots = 0: every other batch call (a solution counts for the groups as above)
+  const int* batch_qslot;                // [nqslots] queried slots
+  const int* batch_qoff;                 // [nqslots + 1] their ranges in batch_qval
+  const int* batch_qval;                 // [ngroups]
+  int* batch_wit;                        // [wit_cap][2 * vpad] witness pool, one row per solution that won a query
+  unsigned* batch_wit_n;                 // rows taken (may run past wit_cap: those solutions keep no row)
+  int batch_nqslots, batch_wit_cap;
   unsigned long long pad8_;              // the size stays a multiple of 16: the kernel arguments behind DevParams keep
                                          // their alignment, so their loads keep their width
 };

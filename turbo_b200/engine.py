@@ -43,6 +43,8 @@ def lib():
                                       C.POINTER(abi.TbStats)]
         L.tb_solve_objectives.argtypes = [vp, C.c_int32, i32p, i32p, C.c_int32, i32p, i32p, i32p, i32p, i32p, i32p, i32p,
                                           i32p, C.POINTER(abi.TbStats)]
+        L.tb_solve_supports.argtypes = [vp, C.c_int32, i32p, i32p, C.c_int32, i32p, i32p, i32p, i32p, i32p, C.c_int32,
+                                        i32p, i32p, i32p, C.POINTER(abi.TbStats)]
         L.tb_link_peers.argtypes = [C.POINTER(vp), C.c_int32]
         L.tb_export_bound_handle.argtypes = [vp, vp]
         L.tb_import_peer_bounds.argtypes = [vp, vp, C.c_int32]
@@ -57,7 +59,7 @@ def lib():
         L.tb_version.restype = C.c_char_p
         L.tb_device_count.restype = C.c_int32
         for name in ("tb_create", "tb_propagate", "tb_propagate_batch", "tb_dive", "tb_dive_batch", "tb_solve",
-                     "tb_solve_batch", "tb_solve_groups", "tb_solve_objectives", "tb_link_peers", "tb_export_bound_handle", "tb_import_peer_bounds", "tb_read_bound",
+                     "tb_solve_batch", "tb_solve_groups", "tb_solve_objectives", "tb_solve_supports", "tb_link_peers", "tb_export_bound_handle", "tb_import_peer_bounds", "tb_read_bound",
                      "tb_get_config"):
             getattr(L, name).restype = C.c_int
         _LIB = L
@@ -332,6 +334,87 @@ class Solver:
             lo[:], hi[:] = abi.POS_INF, abi.NEG_INF
         return dict(vars=vs, lb=lo, ub=hi, exact_lb=r["exhaustive"][:k].copy(), exact_ub=r["exhaustive"][k:].copy(),
                     has_solution=has, stats=r["stats"])
+
+    def solve_supports(self, lb, ub, q_var, q_val, witnesses=0, stop_flag=None):
+        """tb_solve_supports: for every query i, is there a solution of this solver's network over the union of K boxes
+        ([K, nvars] int32, each a narrowing of the problem's) with q_var[i] = q_val[i]? Returns `supported` (int8 [nq]:
+        1 = yes, 0 = proven no, -1 = unknown), `witness` (int32 [nq]: the row of wit_lb / wit_ub that holds the value,
+        -1 = none), `wit_lb` / `wit_ub` ([nwit, nvars] solution stores; at most `witnesses` rows) and the stats. The
+        problem's own objective plays no part; narrow its upper bound in the boxes to ask about (near-)optimal
+        solutions."""
+        n = self.problem.nvars
+        lb = np.ascontiguousarray(lb, dtype=np.int32).reshape(-1, n)
+        ub = np.ascontiguousarray(ub, dtype=np.int32).reshape(-1, n)
+        if lb.shape != ub.shape:
+            raise ValueError("lb and ub must have the same shape [K, nvars]")
+        q_var = np.ascontiguousarray(q_var, dtype=np.int32).reshape(-1)
+        q_val = np.ascontiguousarray(q_val, dtype=np.int32).reshape(-1)
+        if q_val.shape != q_var.shape:
+            raise ValueError("q_val must have one entry per query")
+        m, w = q_var.shape[0], int(witnesses)
+        sup = np.zeros(max(1, m), np.int32)
+        wit = np.full(max(1, m), -1, np.int32)
+        wlb = np.zeros((max(1, w), max(1, n)), np.int32) if w >= 0 else None
+        wub = np.zeros((max(1, w), max(1, n)), np.int32) if w >= 0 else None
+        nwit = np.zeros(1, np.int32)
+        st = abi.TbStats()
+        _check(lib().tb_solve_supports(self._h, lb.shape[0], _p(lb), _p(ub), m, _p(q_var), _p(q_val), stop_flag, _p(sup),
+                                       _p(wit), w, _p(wlb), _p(wub), _p(nwit), C.byref(st)))
+        k = int(nwit[0])
+        return dict(supported=sup[:m].astype(np.int8), witness=wit[:m].copy(), wit_lb=wlb[:k, :n], wit_ub=wub[:k, :n],
+                    stats=st.as_dict())
+
+    # Input guard of solution_domains: one query per value, each a group of the launch with a root per box.
+    MAX_DOMAIN_VALUES = 1 << 22
+
+    def solution_domains(self, vars=None, lb=None, ub=None, witnesses=0, stop_flag=None):
+        """The solution domains: for each variable of `vars` (default: every variable), the values it takes in some
+        solution of the network over the union of the boxes lb / ub ([K, nvars] or [nvars]; default: the problem's
+        root), as one solve_supports call with a query per value of the variable's range over the boxes. Returns, per
+        variable, `supported` (the values with a solution) and `unknown` (the values neither supported nor proven
+        unsupported), `exact` (every value of the variable was decided), `has_solution` (some value is supported), and
+        the stats; with `witnesses` > 0 also `witness` (per variable, the pool row of each supported value, -1 = none)
+        and the pool `wit_lb` / `wit_ub`. Raises ValueError on an infinite bound of a queried variable or when the
+        values number more than MAX_DOMAIN_VALUES."""
+        n = self.problem.nvars
+        vs = np.arange(n, dtype=np.int32) if vars is None else np.asarray(vars, np.int32).reshape(-1)
+        lb = np.asarray(self.problem.lb if lb is None else lb, np.int64).reshape(-1, n)
+        ub = np.asarray(self.problem.ub if ub is None else ub, np.int64).reshape(-1, n)
+        ranges = []
+        for v in vs:
+            live = lb[:, v] <= ub[:, v]
+            if not live.any():
+                ranges.append((0, -1))
+                continue
+            a, b = int(lb[live, v].min()), int(ub[live, v].max())
+            if a == abi.NEG_INF or b == abi.POS_INF:
+                raise ValueError(f"variable {int(v)} has an infinite bound: its solution domain cannot be enumerated")
+            ranges.append((a, b))
+        total = sum(b - a + 1 for a, b in ranges)
+        if total > self.MAX_DOMAIN_VALUES:
+            raise ValueError(f"{total} values to query, more than MAX_DOMAIN_VALUES = {self.MAX_DOMAIN_VALUES}")
+        q_var = np.concatenate([np.full(b - a + 1, v, np.int32) for v, (a, b) in zip(vs, ranges)] + [np.zeros(0, np.int32)])
+        q_val = np.concatenate([np.arange(a, b + 1, dtype=np.int64) for a, b in ranges] + [np.zeros(0, np.int64)])
+        if total:
+            r = self.solve_supports(lb, ub, q_var, q_val, witnesses, stop_flag)
+        else:                                   # (every queried variable is empty in every box)
+            r = dict(supported=np.zeros(0, np.int8), witness=np.zeros(0, np.int32), wit_lb=np.zeros((0, n), np.int32),
+                     wit_ub=np.zeros((0, n), np.int32), stats=None)
+        out = dict(vars=vs, supported=[], unknown=[], exact=np.zeros(len(vs), bool),
+                   has_solution=bool((r["supported"] == 1).any()), stats=r["stats"])
+        if witnesses > 0:
+            out.update(witness=[], wit_lb=r["wit_lb"], wit_ub=r["wit_ub"])
+        at = 0
+        for i, (a, b) in enumerate(ranges):
+            k = b - a + 1
+            ans, vals = r["supported"][at:at + k], q_val[at:at + k]
+            out["supported"].append(vals[ans == 1])
+            out["unknown"].append(vals[ans == -1])
+            out["exact"][i] = not (ans == -1).any()
+            if witnesses > 0:
+                out["witness"].append(r["witness"][at:at + k][ans == 1])
+            at += k
+        return out
 
     def export_bound_handle(self):
         buf = C.create_string_buffer(64)
