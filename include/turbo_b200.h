@@ -255,6 +255,34 @@ tb_status tb_solve_supports(tb_solver*, int32_t nboxes, const int32_t* box_lb, c
                             int32_t wit_cap, int32_t* wit_lb, int32_t* wit_ub, int32_t* nwit,
                             tb_stats* stats);
 
+/* The Pareto front of two objectives, in one launch. level [nlev] is strictly ascending and finite; level i answers:
+ * the best y_var, in its own sense (maximize_y), over the solutions of the network on the union of nboxes boxes
+ * (box_lb / box_ub laid out [nboxes][nvars], each a narrowing of the solver's root, as in tb_solve_objectives) with
+ * x_var <= level[i] (x_var >= level[i] when maximize_x = 1). The problem's own obj_var plays no part. The front is the
+ * set of levels whose value strictly improves on the previous level in x's preferred order (ascending levels when x
+ * is minimised, descending when maximised); with one level per value of x's range it is the exact Pareto front
+ * whenever every level is exhaustive. The levels search disjoint slices of x's range - (level[i-1], level[i]] when x is
+ * minimised, [level[i], level[i+1]) when maximised, the outermost slice open - and every solution is a witness for
+ * every level on its side, so each part of the space is searched once. Outputs per level [nlev], shaped as in
+ * tb_solve_objectives: has_solution; objective = the value (TB_POS_INF without a solution; an unbounded y reports its
+ * infinity and ends that level, not exhaustive); exhaustive = the value is proven: every slice on the level's side
+ * (levels 0..i when x is minimised, i..nlev-1 when maximised) was searched to its end with no block cut, or decided on
+ * the host; best_lb / best_ub [nlev][nvars] (may be NULL) = a solution store with y fixed to the value and x fixed to
+ * the best value the row allows on the level's side, so the row's lower bounds are the point (x*, y*) (rows of levels
+ * without a solution are left as they are). A root whose box's range of x misses its slice, or whose box has an empty
+ * referenced domain, is decided on the host. Device memory: the nboxes box images, 24 bytes per root (nlev * nboxes
+ * roots), 48 bytes per level, and one best row of 2 * vpad int32 per level (vpad: the padded variable count).
+ * stop_flag, the timeout and the subproblems per root apply as in tb_solve_groups. TB_ERR_INVALID: nboxes < 1,
+ * nlev < 1, x_var or y_var outside [0, nvars), x_var == y_var, a maximize_* other than 0 / 1, levels not strictly
+ * ascending, a level equal to TB_NEG_INF or TB_POS_INF, a widening box, nlev * nboxes above 2^40 (the subproblem
+ * index), has_solution / exhaustive / objective NULL. TB_ERR_NOMEM: no host memory for the roots.
+ * TB_ERR_UNSUPPORTED: as tb_solve_batch. */
+tb_status tb_solve_front(tb_solver*, int32_t nboxes, const int32_t* box_lb, const int32_t* box_ub,
+                         int32_t x_var, int32_t maximize_x, int32_t y_var, int32_t maximize_y,
+                         int32_t nlev, const int32_t* level,
+                         volatile int32_t* stop_flag, int32_t* best_lb, int32_t* best_ub,
+                         int32_t* has_solution, int32_t* exhaustive, int32_t* objective, tb_stats* stats);
+
 /* Intermediate solutions (-i / -a; the reference's consumer thread, gpu_dive_and_solve.hpp:100-132; its barebones
  * architecture cannot, barebones_dive_and_solve.hpp:465-467).  tb_stream_solutions (before tb_solve) makes every
  * improving solution also land in a ring of `slots` store images; tb_poll_solution, called from ANOTHER host thread

@@ -302,9 +302,9 @@ __device__ __forceinline__ int chunk_class(const DevParams& P, int ch) {
 
 // Per-CTA state of the BATCH kernels only (a function-scope __shared__ object: the other kernels never reference it).
 // Set by thread 0 when a task starts: `group`, the group of the task's root, its objective slot `obj` (-1 =
-// satisfaction) and sense `maximize`, `image`, the root's box, and the group's fixing `fix` = `fix_val` (-1 = none).
-// `pick` / `key`: witness sharing (batch_share_witness, batch_support_witness).
-struct BatchCtl { int won; int group; int obj; int maximize; int image; int pick; int key; int fix; int fix_val; };
+// satisfaction) and sense `maximize`, `image`, the root's box, and the group's fixing `fix` in [fix_lo, fix_hi] (-1 =
+// none). `pick` / `key`: witness sharing (batch_share_witness, batch_support_witness).
+struct BatchCtl { int won; int group; int obj; int maximize; int image; int pick; int key; int fix; int fix_lo; int fix_hi; };
 __device__ __forceinline__ BatchCtl& batch_ctl() { __shared__ BatchCtl b; return b; }
 
 // The incumbent's key of a solution's objective domain [l, u]: l when minimising, ~u = -u - 1 when maximising. The
@@ -1002,10 +1002,26 @@ struct Ctx {
   // publishes it where it beats the group's incumbent, and asks for the image where it beats the group's best image.
   // The block then writes the image into those rows one group at a time, as batch_save_best does, so it holds one lock
   // at a time. An unbounded key ends its group, as it ends the group that finds it.
+  // tb_solve_front: group i asks for the best y with x <= level[i] (x >= level[i] when maximising x), and level[i] is
+  // its fix_hi (fix_lo). A store with x in [l, u] is a witness for group i iff l <= level[i] (u >= level[i]): the levels
+  // ascend, so those groups are a suffix (a prefix) of the groups, found by a binary search. This is the dominance cut:
+  // a solution of a low slice is the incumbent of every level above it.
   __device__ __forceinline__ void batch_share_witness() {
     BatchCtl& b = batch_ctl();
-    const int own = b.group, n = P.batch_share;
-    for (int base = 0; base < n; base += T) {
+    const int own = b.group;
+    int first = 0, n = P.batch_share;
+    if (P.batch_front) {
+      int l, u; store.ld(P.batch_front_x, l, u);
+      const bool min_x = P.batch_front == 1;
+      int lo = 0, hi = n;                       // the first group whose level the store does not reach from below
+      while (lo < hi) {                         // (min x) / reaches (max x)
+        const int m = (lo + hi) >> 1;
+        const BatchGroup& g = P.batch_groups[m];
+        if (min_x ? g.fix_hi < l : g.fix_lo <= u) lo = m + 1; else hi = m;
+      }
+      if (min_x) first = lo; else n = lo;
+    }
+    for (int base = first; base < n; base += T) {
       const int grp = base + tid;
       int key = TBD_PINF;
       bool want = false;
@@ -1323,7 +1339,7 @@ struct Ctx {
             const BatchGroup& g = P.batch_groups[r.group];
             BatchCtl& b = batch_ctl();
             b.group = r.group; b.image = r.image; b.obj = g.obj; b.maximize = g.maximize;
-            b.fix = g.fix; b.fix_val = g.fix_val;
+            b.fix = g.fix; b.fix_lo = g.fix_lo; b.fix_hi = g.fix_hi;
             c.abandon = r.skip || batch_group_over();   // (nothing left to do for a root that is over)
           }
         }
@@ -1333,11 +1349,12 @@ struct Ctx {
           for (int i = tid; i < P.nsnap; i += T) g_snap_tag[i] = -1;       // snapshots belong to one subproblem
           if constexpr (BATCH) {
             load_store(P.batch_roots + (size_t)batch_ctl().image * 2 * P.vpad);
-            // The group's fixing (tb_solve_supports), marked for the active set before the first propagation. This is
-            // the only place a batch root store is built: the dive starts here, g_root and the snapshots are saved
-            // from stores below it, and a tail-split child is a task that starts here again, so all of them hold it.
+            // The group's fixing (tb_solve_supports, tb_solve_front), marked for the active set before the first
+            // propagation. This is the only place a batch root store is built: the dive starts here, g_root and the
+            // snapshots are saved from stores below it, and a tail-split child is a task that starts here again, so
+            // all of them hold it.
             if (tid == 0 && batch_ctl().fix >= 0) {
-              store.embed(batch_ctl().fix, batch_ctl().fix_val, batch_ctl().fix_val);
+              store.embed(batch_ctl().fix, batch_ctl().fix_lo, batch_ctl().fix_hi);
               mark_var(batch_ctl().fix);
             }
           } else load_store(P.root_store);
@@ -2766,29 +2783,38 @@ static tb_status ensure_batch_buffers(tb_solver* s, size_t nimages, size_t nroot
   return TB_OK;
 }
 
-// tb_solve_supports's part of solve_groups. Group g fixes variable fix_var[g] to fix_val[g] in every root; the groups
-// are sorted by (slot, value), so fix_val is the value list of the CSR over the queried slots qslot / qoff. Solutions
-// go to a pool of wit_cap rows (*nwit of them written, wit_lb / wit_ub [wit_cap][nvars]); wit_of [ngroups] receives
-// each group's row (-1 = none).
+// The fixing of tb_solve_supports and tb_solve_front: group g narrows variable var[g] to [lo[g], hi[g]] in every root
+// (a query's value; a level's slice of x). A root whose box's range of that variable misses the interval is decided on
+// the host, as an empty box is. `front` (tb_solve_front: 1 = the front minimises x, 2 = it maximises x; 0 = none):
+// every group narrows x, its level is hi[g] (lo[g]), a solution is a witness for every level it reaches, and each
+// returned row also has x fixed to the best value the row allows on the level's side.
+struct GroupFixing {
+  const int32_t *var, *lo, *hi;
+  int front;
+};
+
+// tb_solve_supports's part of solve_groups. The groups fix one variable each (GroupFixing, lo = hi = the value) and are
+// sorted by (slot, value), so their values are the value list of the CSR over the queried slots qslot / qoff.
+// Solutions go to a pool of wit_cap rows (*nwit of them written, wit_lb / wit_ub [wit_cap][nvars]); wit_of [ngroups]
+// receives each group's row (-1 = none).
 struct SupportQueries {
-  const int32_t* fix_var;
-  const int32_t* fix_val;
   std::vector<int32_t> qslot, qoff;
   int32_t wit_cap;
   int32_t *wit_lb, *wit_ub, *nwit, *wit_of;
 };
 
-// The one host path of the BATCH kernel: tb_solve_groups, tb_solve_batch, tb_solve_objectives and tb_solve_supports.
-// `nimages` boxes (box_lb / box_ub [nimages][nvars]); root r searches box image_of[r] for group group_of[r] (nroots
-// entries); group g optimises variable obj_of[g] (-1 = satisfaction) in the sense maximize[g] (ngroups entries).
-// `objectives` (tb_solve_objectives): every solution is a witness for every group, each returned row has the group's
-// objective variable fixed to its value, and an unbounded objective is never exhaustive. `sup` (tb_solve_supports):
-// every group is a satisfaction group with one variable fixed, every solution is a witness for every group it holds,
-// and there are no best rows (best_lb / best_ub / objective are NULL), only the witness pool. `fn` names the entry
-// point in errors.
+// The one host path of the BATCH kernel: tb_solve_groups, tb_solve_batch, tb_solve_objectives, tb_solve_supports and
+// tb_solve_front. `nimages` boxes (box_lb / box_ub [nimages][nvars]); root r searches box image_of[r] for group
+// group_of[r] (nroots entries); group g optimises variable obj_of[g] (-1 = satisfaction) in the sense maximize[g]
+// (ngroups entries). `objectives` (tb_solve_objectives, tb_solve_front): every solution is a witness for every group
+// (for the groups whose level it reaches, with a front `fix`), each returned row has the group's objective variable
+// fixed to its value, and an unbounded objective is never exhaustive. `fix`: each group's fixing (GroupFixing).
+// `sup` (tb_solve_supports, with `fix`): every group is a satisfaction group with one variable fixed, every solution is
+// a witness for every group it holds, and there are no best rows (best_lb / best_ub / objective are NULL), only the
+// witness pool. `fn` names the entry point in errors.
 static tb_status solve_groups(tb_solver* s, const char* fn, int32_t nimages, const int32_t* box_lb, const int32_t* box_ub,
                               long long nroots, const int32_t* image_of, const int32_t* group_of, int32_t ngroups,
-                              const int32_t* obj_of, const int32_t* maximize, bool objectives,
+                              const int32_t* obj_of, const int32_t* maximize, bool objectives, const GroupFixing* fix,
                               const SupportQueries* sup, volatile int32_t* stop_flag, int32_t* best_lb,
                               int32_t* best_ub, int32_t* has_solution, int32_t* exhaustive, int32_t* objective,
                               tb_stats* stats) {
@@ -2862,10 +2888,9 @@ static tb_status solve_groups(tb_solver* s, const char* fn, int32_t nimages, con
     b.group = group_of[r];
     b.image = image_of[r];
     b.skip = empty[(size_t)b.image];
-    if (sup) {                                         // (a fixing outside the box: decided on the host, as empty)
-      const size_t at = (size_t)b.image * nv + (size_t)sup->fix_var[b.group];
-      const int v = sup->fix_val[b.group];
-      b.skip |= v < box_lb[at] || v > box_ub[at];
+    if (fix) {                                         // (a fixing that misses the box: decided on the host, as empty)
+      const size_t at = (size_t)b.image * nv + (size_t)fix->var[b.group];
+      b.skip |= std::max(fix->lo[b.group], box_lb[at]) > std::min(fix->hi[b.group], box_ub[at]);
     }
   }
   std::vector<BatchGroup> groups((size_t)ngroups);
@@ -2876,8 +2901,9 @@ static tb_status solve_groups(tb_solver* s, const char* fn, int32_t nimages, con
     G.img_bound = TBD_PINF;
     G.obj = obj_of[g] >= 0 ? s->layout.slot_of[obj_of[g]] : -1;
     G.maximize = maximize[g];
-    G.fix = sup ? s->layout.slot_of[sup->fix_var[g]] : -1;
-    G.fix_val = sup ? sup->fix_val[g] : 0;
+    G.fix = fix ? s->layout.slot_of[fix->var[g]] : -1;
+    G.fix_lo = fix ? fix->lo[g] : 0;
+    G.fix_hi = fix ? fix->hi[g] : 0;
     G.wit = -1;
   }
   CU(cudaMemcpyAsync(s->d_batch_roots, images.data(), images.size() * sizeof(int), cudaMemcpyHostToDevice, s->stream));
@@ -2887,12 +2913,14 @@ static tb_status solve_groups(tb_solver* s, const char* fn, int32_t nimages, con
   P.batch_groups = s->d_batch_groups;
   P.batch_share = objectives && ngroups > 1 ? ngroups : 0;   // (one objective has nobody to share with)
   P.batch_nqslots = (int)nqslots;
+  P.batch_front = fix ? fix->front : 0;
+  P.batch_front_x = fix && fix->front ? s->layout.slot_of[fix->var[0]] : 0;
   if (sup) {
     // the query table: the pool's row counter (0), then qslot, qoff and the values
     std::vector<int32_t> q(nquery, 0);
     std::copy(sup->qslot.begin(), sup->qslot.end(), q.begin() + 1);
     std::copy(sup->qoff.begin(), sup->qoff.end(), q.begin() + 1 + nqslots);
-    std::copy(sup->fix_val, sup->fix_val + ngroups, q.begin() + 1 + 2 * nqslots + 1);
+    std::copy(fix->lo, fix->lo + ngroups, q.begin() + 1 + 2 * nqslots + 1);
     CU(cudaMemcpyAsync(s->d_batch_query, q.data(), q.size() * sizeof(int32_t), cudaMemcpyHostToDevice, s->stream));
     P.batch_wit_n = (unsigned*)s->d_batch_query;
     P.batch_qslot = s->d_batch_query + 1;
@@ -2961,6 +2989,12 @@ static tb_status solve_groups(tb_solver* s, const char* fn, int32_t nimages, con
         lb[(size_t)x] = ub[(size_t)x] = val;
         if (val == (maximize[g] ? TB_POS_INF : TB_NEG_INF)) exh[g] = 0;     // unbounded: the objective ended there
       }
+      // tb_solve_front: x at the best value of the row, which is on the level's side: the row is the group's own
+      // solution, inside its slice, or a witness, whose x reaches the level (batch_share_witness)
+      if (fix && fix->front) {
+        const size_t xv = (size_t)fix->var[g];
+        if (fix->front == 1) ub[xv] = lb[xv]; else lb[xv] = ub[xv];
+      }
     }
     all_exhaustive &= exh[g];
     if (has_solution) has_solution[g] = has;
@@ -2988,6 +3022,13 @@ static tb_status solve_groups(tb_solver* s, const char* fn, int32_t nimages, con
   return rc;
 }
 
+// tb_solve_objectives, tb_solve_supports and tb_solve_front: group g's root g * nboxes + r searches box r
+static void roots_per_box(int32_t nboxes, long long nroots, std::vector<int32_t>& image_of, std::vector<int32_t>& group_of) {
+  image_of.resize((size_t)nroots);
+  group_of.resize((size_t)nroots);
+  for (size_t i = 0; i < (size_t)nroots; ++i) { image_of[i] = (int32_t)(i % (size_t)nboxes); group_of[i] = (int32_t)(i / (size_t)nboxes); }
+}
+
 // tb_solve_groups and tb_solve_batch: one root per box, every group optimises the problem's objective
 static tb_status solve_boxes(tb_solver* s, const char* fn, int32_t nroots, const int32_t* root_lb, const int32_t* root_ub,
                              const int32_t* group_of, int32_t ngroups, volatile int32_t* stop_flag, int32_t* best_lb,
@@ -2998,7 +3039,7 @@ static tb_status solve_boxes(tb_solver* s, const char* fn, int32_t nroots, const
   const int32_t obj = s ? s->root_obj_var : -1;
   std::vector<int32_t> obj_of((size_t)std::max(0, ngroups), obj), minimize((size_t)std::max(0, ngroups), 0);
   return solve_groups(s, fn, nroots, root_lb, root_ub, nroots, own.data(), group_of ? group_of : own.data(), ngroups,
-                      obj_of.data(), minimize.data(), false, nullptr, stop_flag, best_lb, best_ub, has_solution, exhaustive,
+                      obj_of.data(), minimize.data(), false, nullptr, nullptr, stop_flag, best_lb, best_ub, has_solution, exhaustive,
                       objective, stats);
 } catch (const std::bad_alloc&) {             // (the per-root host arrays: nothing may unwind through the C ABI)
   set_error(std::string(fn) + ": out of host memory for the roots");
@@ -3043,13 +3084,13 @@ extern "C" tb_status tb_solve_objectives(tb_solver* s, int32_t nboxes, const int
     set_error(name + ": nobj * nboxes = " + std::to_string(nroots) + " roots do not fit the subproblem index (at most 2^40)");
     return TB_ERR_INVALID;
   }
-  // objective m is group m; its root m * nboxes + r searches box r
+  // objective m is group m
   try {
-    std::vector<int32_t> image_of((size_t)nroots), group_of((size_t)nroots);
-    for (size_t i = 0; i < (size_t)nroots; ++i) { image_of[i] = (int32_t)(i % (size_t)nboxes); group_of[i] = (int32_t)(i / (size_t)nboxes); }
+    std::vector<int32_t> image_of, group_of;
+    roots_per_box(nboxes, nroots, image_of, group_of);
     return solve_groups(s, "tb_solve_objectives", nboxes, box_lb, box_ub, nroots, image_of.data(), group_of.data(), nobj,
-                        obj_var, maximize, true, nullptr, stop_flag, best_lb, best_ub, has_solution, exhaustive, objective,
-                        stats);
+                        obj_var, maximize, true, nullptr, nullptr, stop_flag, best_lb, best_ub, has_solution, exhaustive,
+                        objective, stats);
   } catch (const std::bad_alloc&) {           // (the per-root host arrays: nothing may unwind through the C ABI)
     set_error(name + ": out of host memory for " + std::to_string(nroots) + " roots");
     return TB_ERR_NOMEM;
@@ -3102,19 +3143,18 @@ extern "C" tb_status tb_solve_supports(tb_solver* s, int32_t nboxes, const int32
     }
     sup.qoff.push_back((int32_t)fix_var.size());
     const int32_t ngroups = (int32_t)fix_var.size();
-    sup.fix_var = fix_var.data(); sup.fix_val = fix_val.data();
+    const GroupFixing fix{fix_var.data(), fix_val.data(), fix_val.data(), 0};
     sup.wit_cap = wit_cap; sup.wit_lb = wit_lb; sup.wit_ub = wit_ub; sup.nwit = nwit;
     std::vector<int32_t> wit_of((size_t)ngroups, -1);
     sup.wit_of = wit_of.data();
-    // group g's root g * nboxes + r searches box r, as tb_solve_objectives's objectives do
     const long long nroots = (long long)ngroups * nboxes;
-    std::vector<int32_t> image_of((size_t)nroots), group_of((size_t)nroots), obj_of((size_t)ngroups, -1),
-        maximize((size_t)ngroups, 0), has((size_t)ngroups), exh((size_t)ngroups);
-    for (size_t i = 0; i < (size_t)nroots; ++i) { image_of[i] = (int32_t)(i % (size_t)nboxes); group_of[i] = (int32_t)(i / (size_t)nboxes); }
+    std::vector<int32_t> image_of, group_of, obj_of((size_t)ngroups, -1), maximize((size_t)ngroups, 0),
+        has((size_t)ngroups), exh((size_t)ngroups);
+    roots_per_box(nboxes, nroots, image_of, group_of);
     if (nwit) *nwit = 0;
     const tb_status rc = solve_groups(s, "tb_solve_supports", nboxes, box_lb, box_ub, nroots, image_of.data(),
-                                      group_of.data(), ngroups, obj_of.data(), maximize.data(), false, &sup, stop_flag,
-                                      nullptr, nullptr, has.data(), exh.data(), nullptr, stats);
+                                      group_of.data(), ngroups, obj_of.data(), maximize.data(), false, &fix, &sup,
+                                      stop_flag, nullptr, nullptr, has.data(), exh.data(), nullptr, stats);
     if (rc != TB_OK && rc != TB_ERR_DEPTH) return rc;
     // 1: a solution holds the value; 0: every root of the query was searched to its end uncut or decided on the host
     for (int32_t i = 0; i < nq; ++i) {
@@ -3125,6 +3165,64 @@ extern "C" tb_status tb_solve_supports(tb_solver* s, int32_t nboxes, const int32
     return rc;
   } catch (const std::bad_alloc&) {           // (the per-query and per-root host arrays)
     set_error(name + ": out of host memory for " + std::to_string(nqroots) + " roots");
+    return TB_ERR_NOMEM;
+  }
+}
+
+extern "C" tb_status tb_solve_front(tb_solver* s, int32_t nboxes, const int32_t* box_lb, const int32_t* box_ub,
+                                    int32_t x_var, int32_t maximize_x, int32_t y_var, int32_t maximize_y,
+                                    int32_t nlev, const int32_t* level, volatile int32_t* stop_flag, int32_t* best_lb,
+                                    int32_t* best_ub, int32_t* has_solution, int32_t* exhaustive, int32_t* objective,
+                                    tb_stats* stats) {
+  const std::string name("tb_solve_front");
+  if (!s || nboxes < 1 || nlev < 1 || !level || !has_solution || !exhaustive || !objective) {
+    set_error(name + ": needs nboxes >= 1, nlev >= 1, level, has_solution, exhaustive and objective"); return TB_ERR_INVALID;
+  }
+  if (x_var < 0 || x_var >= s->nvars || y_var < 0 || y_var >= s->nvars || x_var == y_var) {
+    set_error(name + ": x_var = " + std::to_string(x_var) + " and y_var = " + std::to_string(y_var) +
+              " must be two different variables of [0, nvars)");
+    return TB_ERR_INVALID;
+  }
+  if ((maximize_x != 0 && maximize_x != 1) || (maximize_y != 0 && maximize_y != 1)) {
+    set_error(name + ": maximize_x and maximize_y must be 0 or 1"); return TB_ERR_INVALID;
+  }
+  for (int32_t i = 0; i < nlev; ++i) {
+    if (level[i] == TB_NEG_INF || level[i] == TB_POS_INF) {
+      set_error(name + ": level " + std::to_string(i) + " is infinite"); return TB_ERR_INVALID;
+    }
+    if (i && level[i] <= level[i - 1]) {
+      set_error(name + ": the levels are not strictly ascending at level " + std::to_string(i)); return TB_ERR_INVALID;
+    }
+  }
+  const long long nroots = (long long)nlev * nboxes;
+  if ((unsigned long long)nroots > (1ull << TB_K_BITS)) {     // (before the per-root arrays are allocated)
+    set_error(name + ": nlev * nboxes = " + std::to_string(nroots) + " roots do not fit the subproblem index (at most 2^40)");
+    return TB_ERR_INVALID;
+  }
+  try {
+    // Level i is group i, optimising y over its slice of x: (level[i-1], level[i]] when the front minimises x, the
+    // first slice open below; [level[i], level[i+1]) when it maximises x, the last open above. The slices partition x's
+    // range, so every part of the space is searched once, and a solution of a slice is a witness for every level on
+    // its side (batch_share_witness).
+    std::vector<int32_t> var((size_t)nlev, x_var), lo((size_t)nlev), hi((size_t)nlev), obj_of((size_t)nlev, y_var),
+        maximize((size_t)nlev, maximize_y), image_of, group_of;
+    for (int32_t i = 0; i < nlev; ++i) {
+      if (maximize_x) { lo[(size_t)i] = level[i]; hi[(size_t)i] = i + 1 < nlev ? level[i + 1] - 1 : TB_POS_INF; }
+      else { lo[(size_t)i] = i ? level[i - 1] + 1 : TB_NEG_INF; hi[(size_t)i] = level[i]; }
+    }
+    const GroupFixing fix{var.data(), lo.data(), hi.data(), maximize_x ? 2 : 1};
+    roots_per_box(nboxes, nroots, image_of, group_of);
+    const tb_status rc = solve_groups(s, "tb_solve_front", nboxes, box_lb, box_ub, nroots, image_of.data(), group_of.data(),
+                                      nlev, obj_of.data(), maximize.data(), true, &fix, nullptr, stop_flag, best_lb,
+                                      best_ub, has_solution, exhaustive, objective, stats);
+    if (rc != TB_OK && rc != TB_ERR_DEPTH) return rc;
+    // A level's value is the best over its own slice and every witness on its side, so it is proven when every slice on
+    // its side was searched to its end (or decided on the host): groups 0..i when minimising x, i..last when maximising.
+    if (maximize_x) for (int32_t i = nlev - 2; i >= 0; --i) exhaustive[i] &= exhaustive[i + 1];
+    else for (int32_t i = 1; i < nlev; ++i) exhaustive[i] &= exhaustive[i - 1];
+    return rc;
+  } catch (const std::bad_alloc&) {           // (the per-level and per-root host arrays)
+    set_error(name + ": out of host memory for " + std::to_string(nroots) + " roots");
     return TB_ERR_NOMEM;
   }
 }

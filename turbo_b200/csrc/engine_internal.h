@@ -77,7 +77,8 @@ static_assert(sizeof(SplitEntry) == 32, "TB_CELL_BLOCK_BYTES counts 32 bytes per
 // is solved over the union of its roots' boxes: the roots share its incumbent, its stop word and its best store.
 // tb_solve_batch puts every root in a group of its own; tb_solve_objectives makes objective m group m, with one root
 // per box (root m * nboxes + r reads image r); tb_solve_supports makes query g group g, a satisfaction group whose
-// roots g * nboxes + r read image r with one variable fixed (BatchGroup::fix).
+// roots g * nboxes + r read image r with one variable fixed (BatchGroup::fix); tb_solve_front makes level i group i,
+// whose roots i * nboxes + r read image r with x narrowed to the level's slice.
 struct BatchRoot {
   unsigned long long closed;    // weight of the root's search space closed: 2^(56 - D) per task of depth D searched to
                                 // the end, 2^(56 - D + rem) per dive leaf at remaining depth rem; 2^56 = everything
@@ -97,11 +98,11 @@ struct BatchGroup {
   int img_bound;                // key of the best image (TBD_PINF = none)
   int obj;                      // slot of the group's objective variable (-1 = satisfaction)
   int maximize;                 // 1: the group maximises obj
-  int fix;                      // tb_solve_supports: slot fixed to fix_val in every root of the group (-1 = none)
-  int fix_val;
+  int fix;                      // slot narrowed to [fix_lo, fix_hi] in every root of the group (-1 = none):
+  int fix_lo;                   // tb_solve_supports fixes it to one value, tb_solve_front to the level's slice
   int wit;                      // tb_solve_supports: the witness row of the group (-1 = none; -2 - b while block b
                                 // that won the group takes its row)
-  int pad_;
+  int fix_hi;
 };
 static_assert(sizeof(BatchGroup) == 48, "host and device agree on BatchGroup");
 #define TB_BATCH_WEIGHT_BITS 56
@@ -181,6 +182,8 @@ struct DevParams {
   int* batch_wit;                        // [wit_cap][2 * vpad] witness pool, one row per solution that won a query
   unsigned* batch_wit_n;                 // rows taken (may run past wit_cap: those solutions keep no row)
   int batch_nqslots, batch_wit_cap;
-  unsigned long long pad8_;              // the size stays a multiple of 16: the kernel arguments behind DevParams keep
-                                         // their alignment, so their loads keep their width
+  // tb_solve_front: 0 = off (every other call), 1 = the front minimises x, 2 = it maximises x; batch_front_x = x's
+  // slot. The two words keep the size a multiple of 16: the kernel arguments behind DevParams keep their alignment, so
+  // their loads keep their width
+  int batch_front, batch_front_x;
 };

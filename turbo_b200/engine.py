@@ -45,6 +45,8 @@ def lib():
                                           i32p, C.POINTER(abi.TbStats)]
         L.tb_solve_supports.argtypes = [vp, C.c_int32, i32p, i32p, C.c_int32, i32p, i32p, i32p, i32p, i32p, C.c_int32,
                                         i32p, i32p, i32p, C.POINTER(abi.TbStats)]
+        L.tb_solve_front.argtypes = [vp, C.c_int32, i32p, i32p, C.c_int32, C.c_int32, C.c_int32, C.c_int32, C.c_int32,
+                                     i32p, i32p, i32p, i32p, i32p, i32p, i32p, C.POINTER(abi.TbStats)]
         L.tb_link_peers.argtypes = [C.POINTER(vp), C.c_int32]
         L.tb_export_bound_handle.argtypes = [vp, vp]
         L.tb_import_peer_bounds.argtypes = [vp, vp, C.c_int32]
@@ -59,7 +61,7 @@ def lib():
         L.tb_version.restype = C.c_char_p
         L.tb_device_count.restype = C.c_int32
         for name in ("tb_create", "tb_propagate", "tb_propagate_batch", "tb_dive", "tb_dive_batch", "tb_solve",
-                     "tb_solve_batch", "tb_solve_groups", "tb_solve_objectives", "tb_solve_supports", "tb_link_peers", "tb_export_bound_handle", "tb_import_peer_bounds", "tb_read_bound",
+                     "tb_solve_batch", "tb_solve_groups", "tb_solve_objectives", "tb_solve_supports", "tb_solve_front", "tb_link_peers", "tb_export_bound_handle", "tb_import_peer_bounds", "tb_read_bound",
                      "tb_get_config"):
             getattr(L, name).restype = C.c_int
         _LIB = L
@@ -101,6 +103,25 @@ def layout_watch_lists(problem, nbanks=16):
     chunk_of = np.zeros(max(1, problem.nprops), np.int32)
     _check(L.tb_layout_watch_lists(C.byref(problem.c), nbanks, C.byref(ns), C.byref(ne), _p(off), _p(lst), _p(slot_of), _p(chunk_of)))
     return off, lst[:ne.value], slot_of[:problem.nvars], chunk_of[:problem.nprops]
+
+
+def front_points(r, x, maximize_x=False, maximize_y=False):
+    """The Pareto front in per-level answers of Solver.solve_front (`r`, levels ascending): walking the levels in x's
+    preferred order (ascending when x is minimised), the levels whose value strictly improves on every level before
+    them. Returns `points` [(x*, y*)] in that order, with x* read from the level's row, the rows `lb` / `ub`, `proven`
+    (that level is exhaustive) and `level` (the index of each point's level)."""
+    k = len(r["objective"])
+    best, idx = None, []
+    for i in (range(k - 1, -1, -1) if maximize_x else range(k)):
+        if not r["has_solution"][i]:
+            continue
+        key = -int(r["objective"][i]) if maximize_y else int(r["objective"][i])
+        if best is None or key < best:
+            best = key
+            idx.append(i)
+    idx = np.array(idx, np.int64)
+    return dict(points=[(int(r["lb"][i][x]), int(r["objective"][i])) for i in idx], lb=r["lb"][idx], ub=r["ub"][idx],
+                proven=np.asarray(r["exhaustive"], bool)[idx], level=idx)
 
 
 def device_count():
@@ -415,6 +436,68 @@ class Solver:
                 out["witness"].append(r["witness"][at:at + k][ans == 1])
             at += k
         return out
+
+    def solve_front(self, lb, ub, x, y, levels, maximize_x=False, maximize_y=False, stop_flag=None):
+        """tb_solve_front: for every level t of `levels` (strictly ascending, finite), the best value of variable y
+        (maximised when maximize_y, minimised elsewhere) over the solutions of this solver's network on the union of K
+        boxes ([K, nvars] int32, each a narrowing of the problem's) with x <= t (x >= t when maximize_x), in one launch.
+        Returns arrays of length nlev, shaped as solve_objectives's: row i of lb / ub is a solution with y fixed to
+        the value and x fixed to the best value the row allows on the level's side; `exhaustive` says the value is
+        proven. The problem's own objective plays no part."""
+        n = self.problem.nvars
+        lb = np.ascontiguousarray(lb, dtype=np.int32).reshape(-1, n)
+        ub = np.ascontiguousarray(ub, dtype=np.int32).reshape(-1, n)
+        if lb.shape != ub.shape:
+            raise ValueError("lb and ub must have the same shape [K, nvars]")
+        lv = np.asarray(levels, np.int64).reshape(-1)
+        if ((lv < abi.NEG_INF) | (lv > abi.POS_INF)).any():
+            raise ValueError("a level is outside the int32 range")
+        lv = np.ascontiguousarray(lv, dtype=np.int32)
+        m = lv.shape[0]
+        olb = np.zeros((max(1, m), max(1, n)), np.int32)
+        oub = np.zeros((max(1, m), max(1, n)), np.int32)
+        has = np.zeros(max(1, m), np.int32)
+        exh = np.zeros(max(1, m), np.int32)
+        obj = np.zeros(max(1, m), np.int32)
+        st = abi.TbStats()
+        _check(lib().tb_solve_front(self._h, lb.shape[0], _p(lb), _p(ub), int(x), int(maximize_x), int(y),
+                                    int(maximize_y), m, _p(lv), stop_flag, _p(olb), _p(oub), _p(has), _p(exh), _p(obj),
+                                    C.byref(st)))
+        return dict(lb=olb[:m, :n], ub=oub[:m, :n], has_solution=has[:m].astype(bool), exhaustive=exh[:m].astype(bool),
+                    objective=obj[:m].astype(np.int64), stats=st.as_dict())
+
+    # Input guard of pareto_front: every level is a group of the launch with a best row of the store's size.
+    MAX_FRONT_LEVELS = 1 << 16
+
+    def pareto_front(self, x, y, lb=None, ub=None, maximize_x=False, maximize_y=False, levels=None, stop_flag=None):
+        """The Pareto front of objectives x and y (each minimised, or maximised where maximize_* is true) over the union
+        of the boxes lb / ub ([K, nvars] or [nvars]; default: the problem's root), as one solve_front call. `levels`
+        defaults to one level per value of x's range over the boxes, which makes the front exact when every level is
+        exhaustive. Returns `points` [(x*, y*)] in x's preferred order, with their rows `lb` / `ub` and `proven` per
+        point (its level is exhaustive), `exact` (every level is), `levels` and the stats. Raises ValueError on an
+        infinite bound of x when `levels` is None, and on more than MAX_FRONT_LEVELS levels, before any launch."""
+        n = self.problem.nvars
+        lb = np.asarray(self.problem.lb if lb is None else lb, np.int64).reshape(-1, n)
+        ub = np.asarray(self.problem.ub if ub is None else ub, np.int64).reshape(-1, n)
+        if levels is None:
+            live = lb[:, x] <= ub[:, x]
+            a, b = (int(lb[live, x].min()), int(ub[live, x].max())) if live.any() else (0, -1)
+            if a == abi.NEG_INF or b == abi.POS_INF:
+                raise ValueError(f"variable {int(x)} has an infinite bound: give the levels of the front")
+            if b - a + 1 > self.MAX_FRONT_LEVELS:
+                raise ValueError(f"{b - a + 1} levels, more than MAX_FRONT_LEVELS = {self.MAX_FRONT_LEVELS}")
+            levels = np.arange(a, b + 1, dtype=np.int64)
+        levels = np.asarray(levels, np.int64).reshape(-1)
+        if len(levels) > self.MAX_FRONT_LEVELS:
+            raise ValueError(f"{len(levels)} levels, more than MAX_FRONT_LEVELS = {self.MAX_FRONT_LEVELS}")
+        if len(levels):
+            r = self.solve_front(lb, ub, x, y, levels, maximize_x, maximize_y, stop_flag)
+        else:                                   # (x is empty in every box: no solution, nothing to search)
+            r = dict(lb=np.zeros((0, n), np.int32), ub=np.zeros((0, n), np.int32), has_solution=np.zeros(0, bool),
+                     exhaustive=np.zeros(0, bool), objective=np.zeros(0, np.int64), stats=None)
+        f = front_points(r, x, maximize_x, maximize_y)
+        return dict(points=f["points"], lb=f["lb"], ub=f["ub"], proven=f["proven"], exact=bool(r["exhaustive"].all()),
+                    levels=levels, stats=r["stats"])
 
     def export_bound_handle(self):
         buf = C.create_string_buffer(64)
